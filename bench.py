@@ -433,6 +433,17 @@ def io_throughput(L, capi, fh):
     return out
 
 
+def dump_features(L, dev, n, out_dir):
+    """The resident features as a caller of KLTB200ResidentEnd would receive them, written as
+    out_dir/x.npy, y.npy (float32) and val.npy (the int32 status / eigenvalue, exact in float64), so
+    that two builds can be compared output for output.  Synchronises; changes no device state."""
+    x, y, val = np.empty(n, np.float32), np.empty(n, np.float32), np.empty(n, np.int32)
+    L.dev_check(dev, L.klt_dev_features_download(dev, n, x, y, val))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("x", x), ("y", y), ("val", val.astype(np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------- B200 arm
 def run_b200(args, rank, local_rank, world):
     import torch
@@ -524,6 +535,8 @@ def run_b200(args, rank, local_rank, world):
     launches = int(L.klt_dev_launch_count(dev) - launches0)
     L.klt_dev_live_total(dev, C.byref(live), 1)
     dev_ms, dev_feats = float(ms.value), int(live.value)
+    if args.dump_outputs and rank == 0:
+        dump_features(L, dev, nfeat, args.dump_outputs)
     # ---- (1b) the same loop for max(K, 2000) more steps: a timed region of >= 0.1 s (K = 20 is 1.5 ms)
     KS = max(K, 2000)
     barrier()
@@ -944,7 +957,12 @@ def main():
     ap.add_argument("--c5-segment", type=int, default=128, help="config 5: frames per KLTTrackFeaturesSequence call")
     ap.add_argument("--c5-segments", type=int, default=8, help="config 5: calls per sequence")
     ap.add_argument("--c5-inflight", type=int, default=4, help="config 5: sequences in flight per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the features the timed loop of `value` holds after its last step (rank 0) "
+                         "to DIR/x.npy, y.npy, val.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

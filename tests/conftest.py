@@ -45,23 +45,6 @@ def oracle_mod():
 
 
 @pytest.fixture(scope="session")
-def ref(capi, oracle_mod):
-    """The unmodified reference CPU sources compiled in place (oracle/_ref)."""
-    if not os.path.exists(oracle_mod.REF_PATH):
-        pytest.skip("oracle/_ref/libklt_ref.so not built (needs /root/reference)")
-    from tests import refbind
-    return refbind.RefLib(capi, oracle_mod.REF_PATH)
-
-
-@pytest.fixture(scope="session")
-def ref_qsort(capi, oracle_mod):
-    if not os.path.exists(oracle_mod.REF_QSORT_PATH):
-        pytest.skip("oracle/_ref/libklt_ref_qsort.so not built")
-    from tests import refbind
-    return refbind.RefLib(capi, oracle_mod.REF_QSORT_PATH)
-
-
-@pytest.fixture(scope="session")
 def provided(capi):
     """The 10 frames of data/images_provided (config 1), copied to tests/golden."""
     return [capi.read_pgm_numpy(os.path.join(GOLDEN, "images_provided", "img%d.pgm" % i))
