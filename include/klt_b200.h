@@ -12,6 +12,9 @@
 extern "C" {
 #endif
 
+/* val of a feature the forward-backward check rejected (KLTB200SetForwardBackward) */
+#define KLT_B200_FB_INCONSISTENT  -6
+
 /* CUDA device the context's work runs on.  Default: environment variable
  * KLT_B200_DEVICE, else the calling thread's current device.  Must be called
  * before the first Select/Track call on tc. */
@@ -24,6 +27,25 @@ void KLTB200SetDevice(KLT_TrackingContext tc, int device);
  * ranking keys are truncated integers. */
 void KLTB200SetExact(KLT_TrackingContext tc, int exact);
 int  KLTB200GetExact(KLT_TrackingContext tc);
+
+/* Forward-backward check of every tracking call on tc (KLTTrackFeatures, KLTTrackFeaturesDevice,
+ * KLTB200Resident*, KLTTrackFeaturesSequence).  Each feature the translation tracker keeps is
+ * tracked back from frame 2 into frame 1 with the same parameters; it stays KLT_TRACKED, at the
+ * position it has with the check off, when the backward leg tracks and ends no more than max_error
+ * pixels from where the feature started.  Otherwise it is lost as x = y = -1,
+ * val = KLT_B200_FB_INCONSISTENT, before the affine consistency check, so that
+ * KLTReplaceLostFeatures refills the slot.  max_error <= 0 switches the check off; INFINITY drops
+ * only the features whose backward leg fails.  Default: environment variable KLT_B200_FB_MAX_ERROR
+ * when tc's state is created, else off.  NaN ends in KLTError. */
+void  KLTB200SetForwardBackward(KLT_TrackingContext tc, float max_error);
+float KLTB200GetForwardBackward(KLT_TrackingContext tc);
+/* Per feature of the last tracking call on tc (the last frame of a sequence or resident step), into
+ * the non-NULL arrays: where the backward leg ended (xb, yb), its distance from the start position
+ * (err) and its status (back_val); -1 in xb, yb and err when the backward leg lost the feature, and
+ * xb = yb = err = -1, back_val = 1 for a feature the check did not run on.  Synchronises.  KLTError
+ * when that call did not run the check or had a number of features other than n. */
+void KLTB200ForwardBackwardResult(KLT_TrackingContext tc, int n, float *xb, float *yb, float *err,
+                                  int *back_val);
 
 /* the device context behind tc (created on demand) */
 klt_dev *KLTB200Device(KLT_TrackingContext tc);

@@ -71,6 +71,8 @@ typedef struct {
   int   exact;
   int   lighting_insensitive;  /* tc->lighting_insensitive: gain / bias normalised windows
                                   (reference src/V1/trackFeatures.c:125-220, :433-437, :466-468) */
+  float fb_max_error;          /* > 0: forward-backward check in the same launch (klt_dev_fb_results);
+                                  0: off */
 } klt_dev_track_params;
 
 /* replaces the scalar arguments of _KLTSelectGoodFeatures /
@@ -126,6 +128,15 @@ int klt_dev_features_upload(klt_dev *d, int n, const float *x, const float *y, c
 int klt_dev_track_resident(klt_dev *d, int slot_prev, int slot_cur,
                            const klt_dev_track_params *p);
 int klt_dev_features_download(klt_dev *d, int n, float *x, float *y, int *val);   /* synchronises */
+/* Forward-backward check (fb_max_error > 0): after the forward leg of a feature the same warp tracks
+ * the result back from frame 2 into frame 1; the feature is kept when that leg ends KLT_TRACKED within
+ * fb_max_error pixels of the start, else it is recorded as (-1, -1, KLT_B200_FB_INCONSISTENT).
+ * klt_dev_fb_results copies the per-feature records of the last klt_dev_track* call into the non-NULL
+ * arrays: where the backward leg ended (xb, yb; -1 when it lost the feature), the distance from the
+ * start (err; -1 when the backward leg lost it) and its status (back_val); xb = yb = err = -1,
+ * back_val = 1 for a feature the check did not run on.  Fails unless that call ran the check on
+ * exactly n features.  Synchronises. */
+int klt_dev_fb_results(klt_dev *d, int n, float *xb, float *yb, float *err, int *back_val);
 /* Ring of pinned snapshots of the resident features for pipelined drivers
  * (KLTTrackFeaturesSequence): klt_dev_snapshot_ring sizes it (depth <= 64 slots),
  * klt_dev_snapshot_push queues a copy of the current x | y | val into a slot behind the work

@@ -19,6 +19,7 @@ KLT_SMALL_DET = -2
 KLT_MAX_ITERATIONS = -3
 KLT_OOB = -4
 KLT_LARGE_RESIDUE = -5
+KLT_B200_FB_INCONSISTENT = -6      # include/klt_b200.h: rejected by the forward-backward check
 
 STATUS_NAMES = {
     0: "TRACKED", -1: "NOT_FOUND", -2: "SMALL_DET", -3: "MAX_ITERATIONS",

@@ -57,6 +57,12 @@ klt_tc_state *klt_state_get(KLT_TrackingContext tc)
   s->last_slot = -1;
   e = getenv("KLT_B200_EXACT");
   s->exact = (e && atoi(e) != 0) ? 1 : 0;
+  e = getenv("KLT_B200_FB_MAX_ERROR");
+  s->fb_max_error = e ? strtof(e, NULL) : 0.0f;
+  if (isnan(s->fb_max_error)) {
+    free(s);
+    KLTError("(KLT/B200) KLT_B200_FB_MAX_ERROR = %s is not a number of pixels", e);
+  }
   pthread_mutex_lock(&g_lock);
   s->next = g_states;
   g_states = s;
@@ -118,6 +124,25 @@ void KLTB200SetExact(KLT_TrackingContext tc, int exact)
 }
 
 int KLTB200GetExact(KLT_TrackingContext tc) { return klt_state_get(tc)->exact; }
+
+/* a setting of the tracker's launch only: the pyramids stay valid */
+void KLTB200SetForwardBackward(KLT_TrackingContext tc, float max_error)
+{
+  if (isnan(max_error)) KLTError("(KLTB200SetForwardBackward) max_error is NaN");
+  klt_state_get(tc)->fb_max_error = max_error;
+}
+
+float KLTB200GetForwardBackward(KLT_TrackingContext tc) { return klt_state_get(tc)->fb_max_error; }
+
+void KLTB200ForwardBackwardResult(KLT_TrackingContext tc, int n, float *xb, float *yb, float *err,
+                                  int *back_val)
+{
+  klt_tc_state *s = klt_state_find(tc);
+  if (s == NULL || s->dev == NULL)
+    KLTError("(KLTB200ForwardBackwardResult) no tracking call on this context ran the check");
+  if (klt_dev_fb_results(s->dev, n, xb, yb, err, back_val) != 0)
+    KLTError("(KLTB200ForwardBackwardResult) %s", klt_dev_error(s->dev));
+}
 klt_dev *KLTB200Device(KLT_TrackingContext tc) { return klt_state_device(klt_state_get(tc)); }
 int KLTB200LastSlot(KLT_TrackingContext tc)
 {

@@ -38,6 +38,7 @@
 #define KLT_MAX_ITERATIONS -3
 #define KLT_OOB            -4
 #define KLT_LARGE_RESIDUE  -5
+#define KLT_B200_FB_INCONSISTENT -6   // include/klt_b200.h
 
 // ---------------------------------------------------------------------------
 // arithmetic helpers
@@ -817,6 +818,43 @@ struct FeatIO {
   float* ox; float* oy; int* oval; int ostride;
 };
 
+// Forward-backward check, one record per feature of the last tracking call (klt_dev_fb_results):
+// where the backward leg from frame 2 into frame 1 ended, its distance from the start position and
+// its status; (-1, -1, -1, 1) for a feature the check did not run on.
+struct __align__(16) FbRec { float xb, yb, err; int back_val; };
+// The check's kernel argument, the trackers' last: the records and the largest round-trip distance
+// kept.  (Last, and not in TrackArgs, so that the parameter layout of the FB = false kernels is the
+// one they have without the check.)
+struct FbArgs { FbRec* rec; float max_error; };
+
+// value and position the tracker records for a feature (:1383-1437): the final border test
+__device__ __forceinline__ int track_outcome(const TrackArgs& a, int status, float x, float y) {
+  const bool outside = (x < (float)a.borderx || x > (float)(a.ncols - 1 - a.borderx) ||
+                        y < (float)a.bordery || y > (float)(a.nrows - 1 - a.bordery));
+  return (status == KLT_OOB || outside) ? KLT_OOB : status;
+}
+__device__ __forceinline__ void record_feature(const FeatIO& io, int f, int v, float x, float y) {
+  const size_t o = (size_t)f * io.ostride;
+  if (v != KLT_TRACKED) { io.ox[o] = -1.0f; io.oy[o] = -1.0f; io.oval[o] = v; }
+  else { io.ox[o] = x; io.oy[o] = y; io.oval[o] = KLT_TRACKED; }
+}
+// The decision of the check, in separately rounded float32 in both arithmetic modes: the feature is
+// kept when the backward leg tracked and !(d2 > max_error^2).  Fills the feature's record.
+__device__ __forceinline__ bool fb_keep(float max_error, float x0, float y0, float xb, float yb, int back_val,
+                                        FbRec& r) {
+  r.back_val = back_val;
+  if (back_val != KLT_TRACKED) { r.xb = -1.0f; r.yb = -1.0f; r.err = -1.0f; return false; }
+  const float dx = __fsub_rn(xb, x0), dy = __fsub_rn(yb, y0);
+  const float d2 = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
+  r.xb = xb; r.yb = yb; r.err = __fsqrt_rn(d2);
+  return !(d2 > __fmul_rn(max_error, max_error));
+}
+__device__ __forceinline__ FbRec fb_unchecked() {
+  FbRec r;
+  r.xb = -1.0f; r.yb = -1.0f; r.err = -1.0f; r.back_val = 1;
+  return r;
+}
+
 // bilinear weights of _interpolate (trackFeatures.c:31-57): the four products
 // (1-ax)(1-ay), ax(1-ay), (1-ax)ay, ax*ay are rounded first, then multiplied by
 // the pixels and summed left to right.
@@ -909,37 +947,18 @@ __device__ __forceinline__ LiGain li_gain(const float (&g1)[PPL], const float (&
 // PPL = window pixels per lane (ceil(ww*wh / 32)); the frame-1 samples of the
 // window are constant while a level iterates, so they are sampled once per
 // level and kept in registers.
+// The pyramid descent of one feature from (x, y) in p1's frame into p2's frame (:1343-1378): the
+// status of the finest level reached and the end position (xend, yend), before the border test.
 template <bool EXACT, int PPL>
-__global__ void __launch_bounds__(128)
-track_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
-             unsigned long long* __restrict__ live_total) {
-  extern __shared__ float s_win[];     // EXACT only: [warps][3][npix]
-  const int lane = threadIdx.x & 31;
-  const int wib = threadIdx.x >> 5;
-  const int f = blockIdx.x * (blockDim.x >> 5) + wib;
-  if (f >= n) return;
-  if (io.val[(size_t)f * io.istride] < 0) return;             // only features that are not lost (:1346)
-  if (lane == 0) atomicAdd(live_total, 1ULL);
-
+__device__ __forceinline__ int track_descent(const PyrView& p1, const PyrView& p2, const TrackArgs& a, int lane,
+                                             const float (&offi)[PPL], const float (&offj)[PPL],
+                                             float* swx, float* swy, float* swd,
+                                             float x, float y, float& xend, float& yend) {
   const int ww = a.ww, wh = a.wh, hw = ww / 2, hh = wh / 2, npix = ww * wh;
-  float* swx = s_win + (size_t)wib * 3 * npix;
-  float* swy = swx + npix;
-  float* swd = swy + npix;
-
-  float xloc = io.x[(size_t)f * io.istride], yloc = io.y[(size_t)f * io.istride];
+  float xloc = x, yloc = y;
   for (int r = a.nlevels - 1; r >= 0; --r) { xloc = __fdiv_rn(xloc, a.ss); yloc = __fdiv_rn(yloc, a.ss); }
   float xout = xloc, yout = yloc;
   int status = KLT_TRACKED;
-
-  // per-lane window offsets (raster order: pixel p -> (i,j) = (p % ww - hw, p / ww - hh))
-  float offi[PPL], offj[PPL];
-#pragma unroll
-  for (int k = 0; k < PPL; ++k) {
-    const int p = lane + 32 * k;
-    const int pp = p < npix ? p : 0;
-    offi[k] = (float)(pp % ww - hw);
-    offj[k] = (float)(pp / ww - hh);
-  }
 
   for (int r = a.nlevels - 1; r >= 0; --r) {
     xloc = __fmul_rn(xloc, a.ss); yloc = __fmul_rn(yloc, a.ss);
@@ -1127,20 +1146,56 @@ track_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
     xout = x2; yout = y2;
     if (v == KLT_SMALL_DET || v == KLT_OOB) break;      // :1378
   }
+  xend = xout; yend = yout;
+  return status;
+}
 
-  // record (:1383-1437)
-  if (lane == 0) {
-    const bool outside = (xout < (float)a.borderx || xout > (float)(a.ncols - 1 - a.borderx) ||
-                          yout < (float)a.bordery || yout > (float)(a.nrows - 1 - a.bordery));
-    const size_t o = (size_t)f * io.ostride;
-    if (status == KLT_OOB || outside) {
-      io.ox[o] = -1.0f; io.oy[o] = -1.0f; io.oval[o] = KLT_OOB;
-    } else if (status != KLT_TRACKED) {
-      io.ox[o] = -1.0f; io.oy[o] = -1.0f; io.oval[o] = status;
-    } else {
-      io.ox[o] = xout; io.oy[o] = yout; io.oval[o] = KLT_TRACKED;
-    }
+// FB: the forward-backward check runs in the same warp after the forward leg (klt_dev_fb_results)
+template <bool EXACT, int PPL, bool FB>
+__global__ void __launch_bounds__(128)
+track_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
+             unsigned long long* __restrict__ live_total, FbArgs fb) {
+  extern __shared__ float s_win[];     // EXACT only: [warps][3][npix]
+  const int lane = threadIdx.x & 31;
+  const int wib = threadIdx.x >> 5;
+  const int f = blockIdx.x * (blockDim.x >> 5) + wib;
+  if (f >= n) return;
+  if (io.val[(size_t)f * io.istride] < 0) {                   // only features that are not lost (:1346)
+    if (FB && lane == 0) fb.rec[f] = fb_unchecked();
+    return;
   }
+  if (lane == 0) atomicAdd(live_total, 1ULL);
+
+  const int ww = a.ww, wh = a.wh, hw = ww / 2, hh = wh / 2, npix = ww * wh;
+  float* swx = s_win + (size_t)wib * 3 * npix;
+  float* swy = swx + npix;
+  float* swd = swy + npix;
+
+  // per-lane window offsets (raster order: pixel p -> (i,j) = (p % ww - hw, p / ww - hh))
+  float offi[PPL], offj[PPL];
+#pragma unroll
+  for (int k = 0; k < PPL; ++k) {
+    const int p = lane + 32 * k;
+    const int pp = p < npix ? p : 0;
+    offi[k] = (float)(pp % ww - hw);
+    offj[k] = (float)(pp / ww - hh);
+  }
+
+  const float x0 = io.x[(size_t)f * io.istride], y0 = io.y[(size_t)f * io.istride];
+  float xout, yout;
+  int v = track_outcome(a, track_descent<EXACT, PPL>(p1, p2, a, lane, offi, offj, swx, swy, swd, x0, y0, xout, yout),
+                        xout, yout);
+  if (FB) {
+    FbRec r = fb_unchecked();
+    if (v == KLT_TRACKED) {                                   // the backward leg: frame 2 into frame 1
+      float xb, yb;
+      const int vb = track_outcome(a, track_descent<EXACT, PPL>(p2, p1, a, lane, offi, offj, swx, swy, swd,
+                                                                xout, yout, xb, yb), xb, yb);
+      if (!fb_keep(fb.max_error, x0, y0, xb, yb, vb, r)) v = KLT_B200_FB_INCONSISTENT;
+    }
+    if (lane == 0) fb.rec[f] = r;
+  }
+  if (lane == 0) record_feature(io, f, v, xout, yout);     // record (:1383-1437)
 }
 
 #include "klt_track_fast.cuh"
@@ -1255,6 +1310,8 @@ struct klt_dev {
   int trace_n; int* trace_kid; float* trace_t0; float* trace_t1;
   // features entering klt_dev_track* with val >= 0, accumulated on the device
   unsigned long long* d_live;
+  // forward-backward check: one FbRec per feature of the last tracking call that ran it (fb_n >= 0)
+  FbRec* d_fb; int fb_cap, fb_n; float fb_max_error;   // (fb_max_error: of the tracker being launched)
 };
 
 // RAII around one kernel launch: counts it and, in profiling mode, brackets it
@@ -1411,6 +1468,7 @@ extern "C" int klt_dev_create(int device, klt_dev** out) {
   c->reg_frames = getenv("KLT_B200_REGISTER_FRAMES") ? atoi(getenv("KLT_B200_REGISTER_FRAMES")) : 0;   // opt-in: see klt_cuda.h
   if (e != cudaSuccess) { free(c); return fail(nullptr, "cudaStreamCreate: %s", cudaGetErrorString(e)); }
   c->tstream = c->stream;
+  c->fb_n = -1;
   c->overlap_l0_ctas = getenv("KLT_B200_OVERLAP_L0_CTAS") ? atoi(getenv("KLT_B200_OVERLAP_L0_CTAS")) : 0;
   e = cudaMalloc(&c->d_live, sizeof(unsigned long long));
   if (e == cudaSuccess) e = cudaMemsetAsync(c->d_live, 0, sizeof(unsigned long long), c->stream);
@@ -1478,6 +1536,7 @@ extern "C" void klt_dev_destroy(klt_dev* d) {
   free_geometry(d);
   cudaFree(d->frame_buf[0]); cudaFree(d->frame_buf[1]);
   guarded_free(d, d->d_x);
+  guarded_free(d, d->d_fb);
   cudaFreeHost(d->h_x);
   for (int i = 0; i < 2; ++i) { guarded_free(d, d->c_val[i]); guarded_free(d, d->c_idx[i]); }
   cudaFree(d->cub_tmp); guarded_free(d, d->fmap); guarded_free(d, d->open_slots); guarded_free(d, d->rank_list); guarded_free(d, d->sel_state);
@@ -2591,42 +2650,56 @@ static FeatIO feat_io(klt_dev* d) {
   return io;
 }
 
-template <bool EXACT, int PPL>
+static FbArgs fb_args(const klt_dev* d) {
+  FbArgs f;
+  f.rec = d->d_fb; f.max_error = d->fb_max_error;
+  return f;
+}
+
+template <bool EXACT, int PPL, bool FB>
 static int launch_track(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n) {
   const int warps = 4;
   const size_t smem = EXACT ? (size_t)warps * 3 * a.ww * a.wh * sizeof(float) : 0;
-  if (set_smem(d, track_kernel<EXACT, PPL>, smem)) return 1;
+  if (set_smem(d, track_kernel<EXACT, PPL, FB>, smem)) return 1;
   { Launch l(d, KID_TRACK, d->tstream);
-    track_kernel<EXACT, PPL><<<(n + warps - 1) / warps, warps * 32, smem, d->tstream>>>(
-        v1, v2, a, n, feat_io(d), d->d_live); }
+    track_kernel<EXACT, PPL, FB><<<(n + warps - 1) / warps, warps * 32, smem, d->tstream>>>(
+        v1, v2, a, n, feat_io(d), d->d_live, fb_args(d)); }
   return 0;
+}
+template <bool EXACT, int PPL>
+static int launch_track(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb) {
+  return fb ? launch_track<EXACT, PPL, true>(d, v1, v2, a, n) : launch_track<EXACT, PPL, false>(d, v1, v2, a, n);
 }
 
 template <int WW, int RPL>
-static void launch_track_fast_t(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n) {
+static void launch_track_fast_t(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb) {
   Launch l(d, KID_TRACK_FAST, d->tstream);
-  track_fast_kernel<WW, RPL><<<(8 * n + 127) / 128, 128, 0, d->tstream>>>(
-      v1, v2, a, n, feat_io(d), d->d_live);
+  if (fb)
+    track_fast_kernel<WW, RPL, true><<<(8 * n + 127) / 128, 128, 0, d->tstream>>>(
+        v1, v2, a, n, feat_io(d), d->d_live, fb_args(d));
+  else
+    track_fast_kernel<WW, RPL, false><<<(8 * n + 127) / 128, 128, 0, d->tstream>>>(
+        v1, v2, a, n, feat_io(d), d->d_live, fb_args(d));
 }
 // square odd windows up to 15x15; returns false if this window has no instantiation
-static bool launch_track_fast(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n) {
+static bool launch_track_fast(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb) {
   switch (a.ww) {
-    case 3: launch_track_fast_t<3, 1>(d, v1, v2, a, n); return true;
-    case 5: launch_track_fast_t<5, 1>(d, v1, v2, a, n); return true;
+    case 3: launch_track_fast_t<3, 1>(d, v1, v2, a, n, fb); return true;
+    case 5: launch_track_fast_t<5, 1>(d, v1, v2, a, n, fb); return true;
     case 7:
-      if (d->track7_off) { launch_track_fast_t<7, 1>(d, v1, v2, a, n); return true; }
+      if (d->track7_off) { launch_track_fast_t<7, 1>(d, v1, v2, a, n, fb); return true; }
       if (!d->no_track7w) {                                  // one warp per feature, scalar loads
         Launch l(d, KID_TRACK7W, d->tstream);
-        launch_k(track7w_kernel, dim3((n + 3) / 4), dim3(128), 0, d->tstream, d->pdl != 0 && !d->overlap, v1, v2, a, n,
-                 feat_io(d), d->d_live);
+        launch_k(fb ? track7w_kernel<true> : track7w_kernel<false>, dim3((n + 3) / 4), dim3(128), 0, d->tstream,
+                 d->pdl != 0 && !d->overlap, v1, v2, a, n, feat_io(d), d->d_live, fb_args(d));
         return true;
       }
-      launch_track_fast_t<7, 1>(d, v1, v2, a, n);
+      launch_track_fast_t<7, 1>(d, v1, v2, a, n, fb);
       return true;
-    case 9: launch_track_fast_t<9, 2>(d, v1, v2, a, n); return true;
-    case 11: launch_track_fast_t<11, 2>(d, v1, v2, a, n); return true;
-    case 13: launch_track_fast_t<13, 2>(d, v1, v2, a, n); return true;
-    case 15: launch_track_fast_t<15, 2>(d, v1, v2, a, n); return true;
+    case 9: launch_track_fast_t<9, 2>(d, v1, v2, a, n, fb); return true;
+    case 11: launch_track_fast_t<11, 2>(d, v1, v2, a, n, fb); return true;
+    case 13: launch_track_fast_t<13, 2>(d, v1, v2, a, n, fb); return true;
+    case 15: launch_track_fast_t<15, 2>(d, v1, v2, a, n, fb); return true;
     default: return false;
   }
 }
@@ -2650,7 +2723,17 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
   if (p->window_width < 3 || p->window_height < 3 || !(p->window_width & 1) || !(p->window_height & 1))
     return fail(d, "tracking window %d x %d must be odd and >= 3", p->window_width, p->window_height);
   const int n = d->feat_n;
+  const bool fb = p->fb_max_error > 0.0f;
+  d->fb_n = fb ? n : -1;
+  d->fb_max_error = p->fb_max_error;
   if (n == 0) return 0;
+  if (fb && d->fb_cap < n) {                         // the check's result records (klt_dev_fb_results)
+    if (sync_all(d)) return fail(d, "stream synchronisation failed");
+    guarded_free(d, d->d_fb); d->d_fb = nullptr; d->fb_cap = 0;
+    const int cap = (n + 1023) / 1024 * 1024;
+    CU(guarded_malloc(d, &d->d_fb, (size_t)cap * sizeof(FbRec)));
+    d->fb_cap = cap;
+  }
   if (feat_flush(d)) return 1;
   if (d->feat_pending) {                             // features uploaded on the copy stream
     CU(cudaStreamWaitEvent(d->tstream, d->ev_feat, 0));
@@ -2673,18 +2756,18 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
   const int ppl = (npix + 31) / 32;
   int rc;
   if (p->exact) {
-    if (ppl <= 2) rc = launch_track<true, 2>(d, v1, v2, a, n);
-    else if (ppl <= 4) rc = launch_track<true, 4>(d, v1, v2, a, n);
-    else if (ppl <= 8) rc = launch_track<true, 8>(d, v1, v2, a, n);
-    else if (ppl <= 16) rc = launch_track<true, 16>(d, v1, v2, a, n);
+    if (ppl <= 2) rc = launch_track<true, 2>(d, v1, v2, a, n, fb);
+    else if (ppl <= 4) rc = launch_track<true, 4>(d, v1, v2, a, n, fb);
+    else if (ppl <= 8) rc = launch_track<true, 8>(d, v1, v2, a, n, fb);
+    else if (ppl <= 16) rc = launch_track<true, 16>(d, v1, v2, a, n, fb);
     else return fail(d, "tracking window %d x %d too large (max 512 pixels)", a.ww, a.wh);
-  } else if (!d->force_generic && !a.lighting && a.ww == a.wh && a.ww <= 15 && launch_track_fast(d, v1, v2, a, n)) {
+  } else if (!d->force_generic && !a.lighting && a.ww == a.wh && a.ww <= 15 && launch_track_fast(d, v1, v2, a, n, fb)) {
     rc = 0;
   } else {
-    if (ppl <= 2) rc = launch_track<false, 2>(d, v1, v2, a, n);
-    else if (ppl <= 4) rc = launch_track<false, 4>(d, v1, v2, a, n);
-    else if (ppl <= 8) rc = launch_track<false, 8>(d, v1, v2, a, n);
-    else if (ppl <= 16) rc = launch_track<false, 16>(d, v1, v2, a, n);
+    if (ppl <= 2) rc = launch_track<false, 2>(d, v1, v2, a, n, fb);
+    else if (ppl <= 4) rc = launch_track<false, 4>(d, v1, v2, a, n, fb);
+    else if (ppl <= 8) rc = launch_track<false, 8>(d, v1, v2, a, n, fb);
+    else if (ppl <= 16) rc = launch_track<false, 16>(d, v1, v2, a, n, fb);
     else return fail(d, "tracking window %d x %d too large (max 512 pixels)", a.ww, a.wh);
   }
   if (rc) return rc;
@@ -2694,6 +2777,26 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
     CU(cudaEventRecord(d->ev_read[slot_cur], d->tstream));
     d->read_pending[slot_prev] = d->read_pending[slot_cur] = 1;
   }
+  return 0;
+}
+
+extern "C" int klt_dev_fb_results(klt_dev* d, int n, float* xb, float* yb, float* err, int* back_val) {
+  CU(cudaSetDevice(d->device));
+  if (d->fb_n < 0) return fail(d, "fb_results: the last tracking call did not run the forward-backward check");
+  if (n != d->fb_n) return fail(d, "fb_results: %d features requested, the last tracking call had %d", n, d->fb_n);
+  if (n == 0) return 0;
+  FbRec* h = (FbRec*)malloc((size_t)n * sizeof(FbRec));
+  if (!h) return fail(d, "out of host memory");
+  cudaError_t e = cudaMemcpyAsync(h, d->d_fb, (size_t)n * sizeof(FbRec), cudaMemcpyDeviceToHost, d->tstream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(d->tstream);
+  if (e != cudaSuccess) { free(h); return fail(d, "fb_results: %s", cudaGetErrorString(e)); }
+  for (int i = 0; i < n; ++i) {
+    if (xb) xb[i] = h[i].xb;
+    if (yb) yb[i] = h[i].yb;
+    if (err) err[i] = h[i].err;
+    if (back_val) back_val[i] = h[i].back_val;
+  }
+  free(h);
   return 0;
 }
 

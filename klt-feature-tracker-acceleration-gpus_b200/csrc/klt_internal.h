@@ -14,6 +14,7 @@ typedef struct klt_tc_state {
   klt_dev *dev;          /* created on first use of the hot path            */
   int device;            /* CUDA device ordinal, -1 = KLT_B200_DEVICE / current */
   int exact;             /* arithmetic mode for tracking pyramids            */
+  float fb_max_error;    /* forward-backward check, > 0: on (KLTB200SetForwardBackward) */
   int last_slot;         /* slot holding the previous frame's pyramids       */
   /* affine consistency check: which host template (aff_img pointer) the device's template
    * slot i mirrors; valid for list aff_list while klt_aff_epoch == aff_epoch */

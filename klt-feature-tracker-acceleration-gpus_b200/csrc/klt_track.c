@@ -36,7 +36,7 @@ static int timing_on(void)
   return on;
 }
 
-static void fill_track_params(KLT_TrackingContext tc, int exact, klt_dev_track_params *p)
+static void fill_track_params(KLT_TrackingContext tc, const klt_tc_state *s, klt_dev_track_params *p)
 {
   p->window_width = tc->window_width;
   p->window_height = tc->window_height;
@@ -47,8 +47,9 @@ static void fill_track_params(KLT_TrackingContext tc, int exact, klt_dev_track_p
   p->max_residue = tc->max_residue;
   p->borderx = tc->borderx;
   p->bordery = tc->bordery;
-  p->exact = exact;
+  p->exact = s->exact;
   p->lighting_insensitive = tc->lighting_insensitive ? 1 : 0;
+  p->fb_max_error = s->fb_max_error > 0.0f ? s->fb_max_error : 0.0f;
 }
 
 static void check_supported(KLT_TrackingContext tc, int pipelined)
@@ -282,7 +283,7 @@ static void track_common(KLT_TrackingContext tc, const KLT_PixelType *img1,
     klt_list_to_arrays(fl, x, y, v);
     DEVCALL(s, klt_dev_features_commit(dev, n));
   }
-  fill_track_params(tc, s->exact, &tp);
+  fill_track_params(tc, s, &tp);
   if (affine) {
     fill_affine_params(tc, &ap);
     DEVCALL(s, klt_dev_affine_begin(dev, n, &ap, &ast));
@@ -295,7 +296,7 @@ static void track_common(KLT_TrackingContext tc, const KLT_PixelType *img1,
   DEVCALL(s, klt_dev_build(dev, slot_cur, img2, on_device, pitch, &q));
   if (timing) t1 = now_us();
 
-  fill_track_params(tc, s->exact, &tp);
+  fill_track_params(tc, s, &tp);
   DEVCALL(s, klt_dev_track_resident(dev, slot_prev, slot_cur, &tp));
   if (affine) DEVCALL(s, klt_dev_affine_check(dev, slot_prev, slot_cur, &tp, &ap));
   if (timing) t2 = now_us();
@@ -390,7 +391,7 @@ void KLTB200ResidentStep(KLT_TrackingContext tc, const KLT_PixelType *img2, int 
   slot_cur = (slot_prev + 1) % KLT_DEV_SLOTS;      /* third slot: build(k+1) may overlap track(k) */
   klt_fill_build_desc(tc, ncols, nrows, tc->nPyramidLevels, 1, s->exact, &q);
   DEVCALL(s, klt_dev_build(s->dev, slot_cur, img2, on_device, pitch ? pitch : (size_t)ncols, &q));
-  fill_track_params(tc, s->exact, &tp);
+  fill_track_params(tc, s, &tp);
   DEVCALL(s, klt_dev_track_resident(s->dev, slot_prev, slot_cur, &tp));
   hand_over(tc, s, slot_cur);
 }
@@ -494,7 +495,7 @@ void KLTTrackFeaturesSequence(KLT_TrackingContext tc, KLT_PixelType *const *fram
   if (replace) klt_fill_select_params(tc, 1, &sp);
   if (affine) {                 /* the per-feature state goes up once and stays on the device */
     fill_affine_params(tc, &ap);
-    fill_track_params(tc, s->exact, &tp);
+    fill_track_params(tc, s, &tp);
     DEVCALL(s, klt_dev_affine_begin(s->dev, n, &ap, &ast));
     affine_stage(tc, s, fl, ast);
     DEVCALL(s, klt_dev_affine_upload_states(s->dev, n));

@@ -42,31 +42,15 @@ __device__ __forceinline__ void sample_row(const float* __restrict__ img, int pi
     out[i] = fmaf(w11, b[i + 1], fmaf(w10, b[i], fmaf(w01, a[i + 1], w00 * a[i])));
 }
 
+// The pyramid descent of the feature of this lane's group from (x, y) in p1's frame into p2's frame:
+// the status of the finest level reached and the end position, before the border test.  Called by
+// all lanes of the warp; groups with alive == false only take part in the shuffles.
 // WW: window width (odd, <= 15); RPL: window rows per lane (window height <= 8 * RPL)
 template <int WW, int RPL>
-__global__ void __launch_bounds__(128)
-track_fast_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
-                  unsigned long long* __restrict__ live_total) {
-  const int lane = threadIdx.x & 31;
-  const int r8 = lane & 7;                                   // lane within the feature group
-  const int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 3;   // feature of this group
+__device__ __forceinline__ int track_fast_descent(const PyrView& p1, const PyrView& p2, const TrackArgs& a,
+                                                  int r8, bool alive, float x, float y, float& xend, float& yend) {
   const int wh = a.wh, hw = WW / 2, hh = wh / 2;
-  const float inv_npix = 0.0f;                               // (unused; residue uses division below)
-  (void)inv_npix;
-
-  bool alive = false;                                        // feature still being tracked
-  float xloc = 0.0f, yloc = 0.0f;
-  if (f < n) {
-    const int v0 = io.val[(size_t)f * io.istride];
-    alive = v0 >= 0;                                         // only features that are not lost (:1346)
-    if (alive) { xloc = io.x[(size_t)f * io.istride]; yloc = io.y[(size_t)f * io.istride]; }
-  }
-  {
-    const unsigned bal = __ballot_sync(0xffffffffu, alive && r8 == 0);
-    if (lane == 0 && bal) atomicAdd(live_total, (unsigned long long)__popc(bal));
-  }
-  if (!__any_sync(0xffffffffu, alive)) return;
-
+  float xloc = x, yloc = y;
   for (int r = a.nlevels - 1; r >= 0; --r) { xloc = xloc / a.ss; yloc = yloc / a.ss; }
   float xout = xloc, yout = yloc;
   int status = KLT_TRACKED;
@@ -210,14 +194,52 @@ track_fast_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
     if (!__any_sync(0xffffffffu, running)) break;
   }
 
-  if (alive && r8 == 0) {                                   // record (:1383-1437)
-    const bool outside = (xout < (float)a.borderx || xout > (float)(a.ncols - 1 - a.borderx) ||
-                          yout < (float)a.bordery || yout > (float)(a.nrows - 1 - a.bordery));
-    const size_t o = (size_t)f * io.ostride;
-    if (status == KLT_OOB || outside) { io.ox[o] = -1.0f; io.oy[o] = -1.0f; io.oval[o] = KLT_OOB; }
-    else if (status != KLT_TRACKED) { io.ox[o] = -1.0f; io.oy[o] = -1.0f; io.oval[o] = status; }
-    else { io.ox[o] = xout; io.oy[o] = yout; io.oval[o] = KLT_TRACKED; }
+  xend = xout; yend = yout;
+  return status;
+}
+
+// FB: the forward-backward check runs in the same group after the forward leg (klt_dev_fb_results)
+template <int WW, int RPL, bool FB>
+__global__ void __launch_bounds__(128)
+track_fast_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
+                  unsigned long long* __restrict__ live_total, FbArgs fb) {
+  const int lane = threadIdx.x & 31;
+  const int r8 = lane & 7;                                   // lane within the feature group
+  const int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 3;   // feature of this group
+
+  bool alive = false;                                        // feature still being tracked
+  float x0 = 0.0f, y0 = 0.0f;
+  if (f < n) {
+    const int v0 = io.val[(size_t)f * io.istride];
+    alive = v0 >= 0;                                         // only features that are not lost (:1346)
+    if (alive) { x0 = io.x[(size_t)f * io.istride]; y0 = io.y[(size_t)f * io.istride]; }
   }
+  {
+    const unsigned bal = __ballot_sync(0xffffffffu, alive && r8 == 0);
+    if (lane == 0 && bal) atomicAdd(live_total, (unsigned long long)__popc(bal));
+  }
+  if (!__any_sync(0xffffffffu, alive)) {
+    if (FB && f < n && r8 == 0) fb.rec[f] = fb_unchecked();
+    return;
+  }
+
+  float xout, yout;
+  int v = track_fast_descent<WW, RPL>(p1, p2, a, r8, alive, x0, y0, xout, yout);
+  if (alive) v = track_outcome(a, v, xout, yout);
+  if (FB) {
+    FbRec r = fb_unchecked();
+    const bool back = alive && v == KLT_TRACKED;             // the backward leg: frame 2 into frame 1
+    if (__any_sync(0xffffffffu, back)) {
+      float xb, yb;
+      int vb = track_fast_descent<WW, RPL>(p2, p1, a, r8, back, xout, yout, xb, yb);
+      if (back) {
+        vb = track_outcome(a, vb, xb, yb);
+        if (!fb_keep(fb.max_error, x0, y0, xb, yb, vb, r)) v = KLT_B200_FB_INCONSISTENT;
+      }
+    }
+    if (f < n && r8 == 0) fb.rec[f] = r;
+  }
+  if (alive && r8 == 0) record_feature(io, f, v, xout, yout);   // record (:1383-1437)
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -303,23 +325,16 @@ __device__ __forceinline__ void warp_sum4x(float& g0, float& g1, float& g2, floa
   g2 = __shfl_sync(0xffffffffu, k, 16); g3 = __shfl_sync(0xffffffffu, k, 24);
 }
 
-__global__ void __launch_bounds__(128)
-track7w_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
-               unsigned long long* __restrict__ live_total) {
+// The pyramid descent of the warp's feature from (x, y) in p1's frame (gathers with L2 policy pol1)
+// into p2's frame (pol2): the status of the finest level reached and the end position, before the
+// border test.
+__device__ __forceinline__ int track7w_descent(const PyrView& p1, const PyrView& p2, const TrackArgs& a, int lane,
+                                               unsigned long long pol1, unsigned long long pol2,
+                                               float x, float y, float& xend, float& yend) {
   constexpr int hw = 3, hh = 3;
-  const int lane = threadIdx.x & 31;
   const int r = lane >> 2, c = lane & 3;                     // footprint row, column pair
   const bool v0 = r < 7, v1 = r < 7 && c < 3;                // window samples (2c, r) and (2c + 1, r)
-  const int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const unsigned long long pol1 = l2_policy(a.l2_keep ? 2 : 0), pol2 = l2_policy(a.l2_keep ? 1 : 0);
-  pdl_wait();                                                 // pyramids and features come from earlier kernels
-  // the whole grid is resident at once (a warp per feature, no shared memory): whatever follows in
-  // the stream -- the next frame's level-0 kernel -- may move into the SMs as these warps retire
-  pdl_launch_dependents();
-  if (f >= n) return;
-  if (io.val[(size_t)f * io.istride] < 0) return;             // only features that are not lost (:1346)
-  if (lane == 0) atomicAdd(live_total, 1ULL);
-  float xloc = io.x[(size_t)f * io.istride], yloc = io.y[(size_t)f * io.istride];
+  float xloc = x, yloc = y;
   for (int l = a.nlevels - 1; l >= 0; --l) { xloc = xloc / a.ss; yloc = yloc / a.ss; }
   float xout = xloc, yout = yloc;
   int status = KLT_TRACKED;
@@ -414,13 +429,42 @@ track7w_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
     if (v == KLT_SMALL_DET || v == KLT_OOB) break;           // :1378
   }
 
-  if (lane == 0) {                                           // record (:1383-1437)
-    const bool outside = (xout < (float)a.borderx || xout > (float)(a.ncols - 1 - a.borderx) ||
-                          yout < (float)a.bordery || yout > (float)(a.nrows - 1 - a.bordery));
-    const size_t o = (size_t)f * io.ostride;
-    if (status == KLT_OOB || outside) { io.ox[o] = -1.0f; io.oy[o] = -1.0f; io.oval[o] = KLT_OOB; }
-    else if (status != KLT_TRACKED) { io.ox[o] = -1.0f; io.oy[o] = -1.0f; io.oval[o] = status; }
-    else { io.ox[o] = xout; io.oy[o] = yout; io.oval[o] = KLT_TRACKED; }
+  xend = xout; yend = yout;
+  return status;
+}
+
+// FB: the forward-backward check runs in the same warp after the forward leg (klt_dev_fb_results).
+// Its backward leg reads the new frame with the new frame's policy (evict_last) and the old frame
+// with the old frame's (evict_first), as the forward leg does.
+template <bool FB>
+__global__ void __launch_bounds__(128)
+track7w_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
+               unsigned long long* __restrict__ live_total, FbArgs fb) {
+  const int lane = threadIdx.x & 31;
+  const int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const unsigned long long pol1 = l2_policy(a.l2_keep ? 2 : 0), pol2 = l2_policy(a.l2_keep ? 1 : 0);
+  pdl_wait();                                                 // pyramids and features come from earlier kernels
+  // the whole grid is resident at once (a warp per feature, no shared memory): whatever follows in
+  // the stream -- the next frame's level-0 kernel -- may move into the SMs as these warps retire
+  pdl_launch_dependents();
+  if (f >= n) return;
+  if (io.val[(size_t)f * io.istride] < 0) {                   // only features that are not lost (:1346)
+    if (FB && lane == 0) fb.rec[f] = fb_unchecked();
+    return;
   }
+  if (lane == 0) atomicAdd(live_total, 1ULL);
+  const float x0 = io.x[(size_t)f * io.istride], y0 = io.y[(size_t)f * io.istride];
+  float xout, yout;
+  int v = track_outcome(a, track7w_descent(p1, p2, a, lane, pol1, pol2, x0, y0, xout, yout), xout, yout);
+  if (FB) {
+    FbRec r = fb_unchecked();
+    if (v == KLT_TRACKED) {                                   // the backward leg: frame 2 into frame 1
+      float xb, yb;
+      const int vb = track_outcome(a, track7w_descent(p2, p1, a, lane, pol2, pol1, xout, yout, xb, yb), xb, yb);
+      if (!fb_keep(fb.max_error, x0, y0, xb, yb, vb, r)) v = KLT_B200_FB_INCONSISTENT;
+    }
+    if (lane == 0) fb.rec[f] = r;
+  }
+  if (lane == 0) record_feature(io, f, v, xout, yout);     // record (:1383-1437)
 }
 

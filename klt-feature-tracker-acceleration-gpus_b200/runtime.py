@@ -35,7 +35,7 @@ class TrackParams(C.Structure):       # klt_dev_track_params
                 ("step_factor", C.c_float), ("max_iterations", C.c_int),
                 ("min_determinant", C.c_float), ("min_displacement", C.c_float),
                 ("max_residue", C.c_float), ("borderx", C.c_int), ("bordery", C.c_int),
-                ("exact", C.c_int), ("lighting_insensitive", C.c_int)]
+                ("exact", C.c_int), ("lighting_insensitive", C.c_int), ("fb_max_error", C.c_float)]
 
 
 class SelectParams(C.Structure):      # klt_dev_select_params
@@ -109,10 +109,14 @@ DEV_API = {
     "klt_dev_trace_count": (C.c_int, [C.c_void_p]),
     "klt_dev_trace_get": (C.c_char_p, [C.c_void_p, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "klt_dev_live_total": (C.c_int, [C.c_void_p, C.POINTER(C.c_ulonglong), C.c_int]),
+    "klt_dev_fb_results": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     # include/klt_b200.h
     "KLTB200SetDevice": (None, [_TC, C.c_int]),
     "KLTB200SetExact": (None, [_TC, C.c_int]),
     "KLTB200GetExact": (C.c_int, [_TC]),
+    "KLTB200SetForwardBackward": (None, [_TC, C.c_float]),
+    "KLTB200GetForwardBackward": (C.c_float, [_TC]),
+    "KLTB200ForwardBackwardResult": (None, [_TC, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "KLTB200Device": (C.c_void_p, [_TC]),
     "KLTB200LastSlot": (C.c_int, [_TC]),
     "KLTTrackFeaturesDevice": (None, [_TC, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, _FL]),
@@ -205,11 +209,26 @@ class B200Library(capi.KLTLibrary):
         self.dev_check(dev, self.lib.klt_dev_read_level(dev, slot, which, level, out))
         return out
 
-    def track_params(self, tc, exact=0) -> TrackParams:
+    def track_params(self, tc, exact=0, fb_max_error=0.0) -> TrackParams:
         t = tc.contents
         return TrackParams(t.window_width, t.window_height, t.step_factor, t.max_iterations,
                            t.min_determinant, t.min_displacement, t.max_residue,
-                           t.borderx, t.bordery, exact, t.lighting_insensitive)
+                           t.borderx, t.bordery, exact, t.lighting_insensitive, fb_max_error)
+
+    def forward_backward(self, tc, n):
+        """KLTB200ForwardBackwardResult: (xb, yb, err, back_val) of the last tracking call on tc"""
+        xb, yb, err = np.empty(n, np.float32), np.empty(n, np.float32), np.empty(n, np.float32)
+        bv = np.empty(n, np.int32)
+        self.lib.KLTB200ForwardBackwardResult(tc, n, xb.ctypes.data, yb.ctypes.data, err.ctypes.data, bv.ctypes.data)
+        return xb, yb, err, bv
+
+    def dev_forward_backward(self, dev, n):
+        """klt_dev_fb_results: (xb, yb, err, back_val) of the last klt_dev_track* call on dev"""
+        xb, yb, err = np.empty(n, np.float32), np.empty(n, np.float32), np.empty(n, np.float32)
+        bv = np.empty(n, np.int32)
+        self.dev_check(dev, self.lib.klt_dev_fb_results(dev, n, xb.ctypes.data, yb.ctypes.data, err.ctypes.data,
+                                                        bv.ctypes.data))
+        return xb, yb, err, bv
 
     def select_params(self, tc, overwrite_all=1) -> SelectParams:
         t = tc.contents
