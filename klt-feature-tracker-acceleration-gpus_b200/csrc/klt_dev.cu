@@ -1838,6 +1838,8 @@ struct FusedPlan {
   int TX[KLT_DEV_MAX_LEVELS], TY[KLT_DEV_MAX_LEVELS], tiles_x[KLT_DEV_MAX_LEVELS], tiles_y[KLT_DEV_MAX_LEVELS];
   int SS, R;                                    // pyramid step geometry of the fused level kernels
   bool l0_march;                                // level 0 on l0_march_kernel (strips x segments) instead of tiles
+  bool chain;                                   // level 0 on L0GeoC (also makes L1), levels >= 1 on
+                                                // level_chain_kernel (map[l]: L_l itself)
 };
 
 static int level_shape_for(int ss, int r, int w, int h, int num_sms) {
@@ -1857,6 +1859,11 @@ static int level_shape_for(int ss, int r, int w, int h, int num_sms) {
   if (ss == 4 && r == 10) return SHAPE_4_10_32_16;
   return SHAPE_NONE;
 }
+template <int TX, int TY>
+static bool chain_map(CUtensorMap* m, const Level& a) {
+  using G = ChGeo<TX, TY>;
+  return make_tensor_map(m, a.img, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.w, a.h, (size_t)a.pitch * 4, G::SW, G::SH);
+}
 template <int SS, int R, int TX, int TY>
 static bool level_map(CUtensorMap* m, const Level& a) {
   using G = LvGeo<SS, R, TX, TY>;
@@ -1864,6 +1871,10 @@ static bool level_map(CUtensorMap* m, const Level& a) {
 }
 
 using L0GeoB = L0GeoT<48, 6, 6, 4>;      // 48-row tiles: 2 even passes in stages A / C, 54 KB of shared memory, 4 CTAs / SM
+// Level 0 of a chained pyramid (subsampling 2, radius 5, more than one level): the tile also makes its
+// 32 x 20 block of L1.  With the L1 halo and the horizontal L1 buffer a 48-row tile needs 63.6 KB, which
+// leaves 3 CTAs per SM; 40-row tiles need 55.7 KB and keep 4 (32 warps).
+using L0GeoC = L0GeoT<40, 7, 5, 4, true>;
 // 0: 64-row tiles, 3 CTAs / SM; 1 (default): 48-row tiles, 4 CTAs / SM; 2: l0_march_kernel (klt_march.cuh: the
 // barrier-free strip formulation, bit-identical, measured slower: 32.5 vs 28.7 us per 4K frame)
 static int g_l0_variant = -1;
@@ -1903,12 +1914,43 @@ static void fused_plan(klt_dev* d, const PyrSet& S, const unsigned char* src, in
     P->TX[0] = L0Geo::TX; P->TY[0] = l0_ty;
     P->tiles_x[0] = (W + L0Geo::TX - 1) / L0Geo::TX; P->tiles_y[0] = (H + l0_ty - 1) / l0_ty;
   }
+  // Chained pyramid: level 0 makes L1, level l makes L_{l+1}, so every level >= 1 reads only its own
+  // plane.  The default level-0 variant with subsampling 2 / radius 5 and every level fused; builds of
+  // one level keep L0GeoB.
+  if (P->l0_ok && !P->l0_march && l0_variant() == 1 && q->nlevels_built > 1 && q->subsampling == 2 &&
+      tp.w == 2 * NEXT_R + 1) {
+    bool all = true;
+    for (int l = 1; l < q->nlevels_built; ++l)
+      all = all && level_shape_for(2, NEXT_R, S.lv[l].w, S.lv[l].h, d->num_sms) != SHAPE_NONE;
+    CUtensorMap m0;
+    if (all && make_tensor_map(&m0, src, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, W, H, (size_t)spitch, L0GeoC::U8_W,
+                               L0GeoC::U8_H)) {
+      P->chain = true;
+      P->map[0] = m0;
+      P->TY[0] = L0GeoC::TY;
+      P->tiles_y[0] = (H + L0GeoC::TY - 1) / L0GeoC::TY;
+    }
+  }
   P->SS = q->subsampling; P->R = tp.w / 2;
   for (int l = 1; l < q->nlevels_built; ++l) {
     const Level& a = S.lv[l - 1];
     const Level& b = S.lv[l];
     int shape = force_shape != SHAPE_NONE ? force_shape : level_shape_for(q->subsampling, tp.w / 2, b.w, b.h, d->num_sms);
     bool ok = false;
+    if (P->chain) {
+      switch (shape) {
+        case SHAPE_2_5_64_32: ok = chain_map<64, 32>(&P->map[l], b); P->TX[l] = 64; P->TY[l] = 32; break;
+        case SHAPE_2_5_64_24: ok = chain_map<64, 24>(&P->map[l], b); P->TX[l] = 64; P->TY[l] = 24; break;
+        case SHAPE_2_5_64_16: ok = chain_map<64, 16>(&P->map[l], b); P->TX[l] = 64; P->TY[l] = 16; break;
+        case SHAPE_2_5_32_16: ok = chain_map<32, 16>(&P->map[l], b); P->TX[l] = 32; P->TY[l] = 16; break;
+        default: break;
+      }
+      if (!ok) { memset(P, 0, sizeof(*P)); return; }   // tensor map refused: nothing runs fused
+      P->shape[l] = shape;
+      P->tiles_x[l] = (b.w + P->TX[l] - 1) / P->TX[l];
+      P->tiles_y[l] = (b.h + P->TY[l] - 1) / P->TY[l];
+      continue;
+    }
     switch (shape) {
       case SHAPE_2_5_64_32: ok = level_map<2, 5, 64, 32>(&P->map[l], a); P->TX[l] = 64; P->TY[l] = 32; break;
       case SHAPE_2_5_64_24: ok = level_map<2, 5, 64, 24>(&P->map[l], a); P->TX[l] = 64; P->TY[l] = 24; break;
@@ -1924,10 +1966,10 @@ static void fused_plan(klt_dev* d, const PyrSet& S, const unsigned char* src, in
   }
 }
 
-// fused level 0 (u8 -> L0, gx0, gy0), tile rows [jr0, jr1)
+// fused level 0 (u8 -> L0, gx0, gy0 (+ L1 with G::NX)), tile rows [jr0, jr1)
 template <class G, bool EXACT>
 static int l0_fused_launch_t(klt_dev* d, const FusedPlan& P, int W, int H, const TapsR& ts, const TapsR& tg,
-                             const TapsR& td, const Level& lv, int jr0, int jr1) {
+                             const TapsR& td, const TapsR& tp, const Level& lv, const Level* l1, int jr0, int jr1) {
   static bool attr_dev[64] = {};                 // function attributes are per device
   bool& attr_set = attr_dev[d->device & 63];
   static int cps = 0;
@@ -1944,7 +1986,8 @@ static int l0_fused_launch_t(klt_dev* d, const FusedPlan& P, int W, int H, const
   { Launch l(d, KID_L0_FUSED);
     CU(launch_k(l0_fused_kernel<G, EXACT>, dim3(grid), dim3(256), G::SMEM, d->stream, d->pdl != 0, P.map[0], W, H,
                 tiles_x, tile0, tile1, d->d_tile_ctr, d->tile_base[0], to_fused(ts), to_fused(tg), to_fused(td), lv.img,
-                lv.gx, lv.gy, lv.pitch));
+                lv.gx, lv.gy, lv.pitch, to_fused(tp), l1 ? l1->img : nullptr, l1 ? l1->pitch : 0, l1 ? l1->w : 0,
+                l1 ? l1->h : 0));
     d->tile_base[0] += (unsigned)(n + grid); }
   return 0;
 }
@@ -1971,14 +2014,16 @@ static int l0_march_launch(klt_dev* d, const FusedPlan& P, int W, int H, const T
                 nstrips, P.TY[0], task0, task1, to_fused(ts), to_fused(tg), to_fused(td), lv.img, lv.gx, lv.gy, lv.pitch)); }
   return 0;
 }
+// l1: level 1, made by the same kernel when the plan is chained (else unused)
 template <bool EXACT>
 static int l0_fused_launch(klt_dev* d, const FusedPlan& P, int W, int H, const TapsR& ts, const TapsR& tg,
-                           const TapsR& td, const Level& lv, int jr0, int jr1) {
+                           const TapsR& td, const TapsR& tp, const Level& lv, const Level& l1, int jr0, int jr1) {
   if (jr1 <= jr0) return 0;
   if (P.l0_march) return l0_march_launch<EXACT>(d, P, W, H, ts, tg, td, lv, jr0, jr1);
+  if (P.chain) return l0_fused_launch_t<L0GeoC, EXACT>(d, P, W, H, ts, tg, td, tp, lv, &l1, jr0, jr1);
   switch (P.TY[0]) {
-    case L0GeoB::TY: return l0_fused_launch_t<L0GeoB, EXACT>(d, P, W, H, ts, tg, td, lv, jr0, jr1);
-    default: return l0_fused_launch_t<L0Geo, EXACT>(d, P, W, H, ts, tg, td, lv, jr0, jr1);
+    case L0GeoB::TY: return l0_fused_launch_t<L0GeoB, EXACT>(d, P, W, H, ts, tg, td, tp, lv, nullptr, jr0, jr1);
+    default: return l0_fused_launch_t<L0Geo, EXACT>(d, P, W, H, ts, tg, td, tp, lv, nullptr, jr0, jr1);
   }
 }
 
@@ -2020,6 +2065,51 @@ static int level_fused_launch(klt_dev* d, const FusedPlan& P, int level, const L
     case SHAPE_2_5_32_16: return level_fused_launch_t<2, 5, 32, 16, EXACT>(d, P, level, a, b, tp, tg, td, jr0, jr1);
     case SHAPE_4_10_32_16: return level_fused_launch_t<4, 10, 32, 16, EXACT>(d, P, level, a, b, tp, tg, td, jr0, jr1);
     default: return fail(d, "level %d has no fused kernel", level);
+  }
+}
+
+// chained level l >= 1 (L_l -> gx_l, gy_l (+ L_{l+1} when nx)), tile rows [jr0, jr1)
+template <int TX, int TY, bool NX, bool EXACT>
+static int level_chain_launch_t(klt_dev* d, const FusedPlan& P, int level, const Level& a, const Level* nx,
+                                const TapsR& tp, const TapsR& tg, const TapsR& td, int jr0, int jr1) {
+  using G = ChGeo<TX, TY>;
+  static bool attr_dev[64] = {};                 // function attributes are per device
+  bool& attr_set = attr_dev[d->device & 63];
+  static int cps = 0;                                                       // resident CTAs per SM
+  if (!attr_set) {
+    CU(cudaFuncSetAttribute(level_chain_kernel<TX, TY, NX, EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cps, level_chain_kernel<TX, TY, NX, EXACT>, 256, G::SMEM));
+    if (cps < 1) cps = 1;
+    attr_set = true;
+  }
+  const int tiles_x = P.tiles_x[level];
+  const int tile0 = jr0 * tiles_x, tile1 = jr1 * tiles_x, n = tile1 - tile0;
+  const int grid = n < cps * d->num_sms ? n : cps * d->num_sms;             // persistent
+  { Launch l(d, level <= 1 ? KID_LEVEL_FUSED : level == 2 ? KID_LEVEL_FUSED_L2 : KID_LEVEL_FUSED_L3);
+    CU(launch_k(level_chain_kernel<TX, TY, NX, EXACT>, dim3(grid), dim3(256), G::SMEM, d->stream, d->pdl != 0,
+                P.map[level], a.w, a.h, nx ? nx->w : 0, nx ? nx->h : 0, tiles_x, tile0, tile1,
+                d->d_tile_ctr + (level & 15), d->tile_base[level & 15], to_fused(tp), to_fused(tg), to_fused(td),
+                a.gx, a.gy, a.pitch, nx ? nx->img : nullptr, nx ? nx->pitch : 0));
+    d->tile_base[level & 15] += (unsigned)(n + grid); }
+  return 0;
+}
+template <int TX, int TY, bool EXACT>
+static int level_chain_launch_s(klt_dev* d, const FusedPlan& P, int level, const Level& a, const Level* nx,
+                                const TapsR& tp, const TapsR& tg, const TapsR& td, int jr0, int jr1) {
+  return nx ? level_chain_launch_t<TX, TY, true, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1)
+            : level_chain_launch_t<TX, TY, false, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
+}
+// nx: level l+1, null for the coarsest level
+template <bool EXACT>
+static int level_chain_launch(klt_dev* d, const FusedPlan& P, int level, const Level& a, const Level* nx,
+                              const TapsR& tp, const TapsR& tg, const TapsR& td, int jr0, int jr1) {
+  if (jr1 <= jr0) return 0;
+  switch (P.shape[level]) {
+    case SHAPE_2_5_64_32: return level_chain_launch_s<64, 32, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
+    case SHAPE_2_5_64_24: return level_chain_launch_s<64, 24, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
+    case SHAPE_2_5_64_16: return level_chain_launch_s<64, 16, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
+    case SHAPE_2_5_32_16: return level_chain_launch_s<32, 16, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
+    default: return fail(d, "level %d has no chained kernel", level);
   }
 }
 
@@ -2262,20 +2352,42 @@ static int build_impl(klt_dev* d, PyrSet& S, const unsigned char* src, int spitc
     // exist -- all at once for a resident frame, band by band behind the upload of a host frame
     int rows_done[KLT_DEV_MAX_LEVELS] = {0}, valid[KLT_DEV_MAX_LEVELS] = {0};
     const int SS = P.SS, R = P.R, RG = FUSED_RG;
+    // u8 rows a level-0 tile row reads below its last output row
+    const int l0_reach = P.chain ? L0GeoC::U8_H - L0GeoC::TY - (L0GeoC::RS + L0GeoC::RG + L0GeoC::XR)
+                                 : L0Geo::RS + L0Geo::RG;
     int u8_rows = feed ? 0 : H;
     if (feed && feed_enqueue_copies(d, feed)) return 1;
     do {
       if (feed && feed_wait(d, feed, false, &u8_rows)) return 1;
       int j = rows_done[0];
       while (j < P.tiles_y[0]) {
-        int need = P.TY[0] * (j + 1) + L0Geo::RS + L0Geo::RG;
+        int need = P.TY[0] * (j + 1) + l0_reach;
         if (need > H) need = H;
         if (need > u8_rows) break;
         ++j;
       }
-      if (l0_fused_launch<EXACT>(d, P, W, H, ts, tg, td, S.lv[0], rows_done[0], j)) return 1;
+      if (l0_fused_launch<EXACT>(d, P, W, H, ts, tg, td, tp, S.lv[0], S.lv[nb > 1 ? 1 : 0], rows_done[0], j)) return 1;
       rows_done[0] = j;
       valid[0] = P.TY[0] * j < H ? P.TY[0] * j : H;
+      if (P.chain) {
+        // tile row j of level l makes rows TY_l/2 * j .. of L_{l+1} and reads L_l rows up to TY_l*(j+1)+4
+        valid[1] = P.TY[0] / 2 * rows_done[0] < S.lv[1].h ? P.TY[0] / 2 * rows_done[0] : S.lv[1].h;
+        for (int l = 1; l < nb; ++l) {
+          const Level& a = S.lv[l];
+          j = rows_done[l];
+          while (j < P.tiles_y[l]) {
+            int need = P.TY[l] * (j + 1) + NEXT_R;
+            if (need > a.h) need = a.h;
+            if (need > valid[l]) break;
+            ++j;
+          }
+          if (level_chain_launch<EXACT>(d, P, l, a, l + 1 < nb ? &S.lv[l + 1] : nullptr, tp, tg, td, rows_done[l], j))
+            return 1;
+          rows_done[l] = j;
+          if (l + 1 < nb) valid[l + 1] = P.TY[l] / 2 * j < S.lv[l + 1].h ? P.TY[l] / 2 * j : S.lv[l + 1].h;
+        }
+        continue;
+      }
       for (int l = 1; l < nb; ++l) {
         const Level& a = S.lv[l - 1];
         const Level& b = S.lv[l];
@@ -2312,7 +2424,7 @@ static int build_impl(klt_dev* d, PyrSet& S, const unsigned char* src, int spitc
   }
   int grad_from = 0;                 // first level whose gradients are still to be computed
   if (P.l0_ok) {
-    if (l0_fused_launch<EXACT>(d, P, W, H, ts, tg, td, S.lv[0], 0, P.tiles_y[0])) return 1;
+    if (l0_fused_launch<EXACT>(d, P, W, H, ts, tg, td, tp, S.lv[0], S.lv[0], 0, P.tiles_y[0])) return 1;
     grad_from = 1;
   }
   d->last_fused = grad_from;

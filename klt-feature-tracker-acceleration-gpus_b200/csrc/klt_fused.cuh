@@ -1,7 +1,10 @@
 // klt_fused.cuh -- TMA-staged, fused frame kernels (included by klt_dev.cu).
 //
 // l0_fused_kernel   : u8 frame          -> L0, gx0, gy0      (1 B read + 12 B written per pixel)
-// level_fused_kernel: L_{l-1} (float)   -> L_l, gx_l, gy_l   (one pyramid step + its gradients)
+//                     (+ L1 with the NX geometry: the pyramid step from the L0 tile already on chip)
+// level_chain_kernel: L_l (float)       -> gx_l, gy_l (+ L_{l+1})
+// level_fused_kernel: L_{l-1} (float)   -> L_l, gx_l, gy_l   (one pyramid step + its gradients;
+//                     subsampling 4, other radii and the non-chained level-0 variants)
 //
 // Replaces, per level, _KLTToFloatImage + _KLTComputeSmoothedImage (+ the smooth/subsample
 // step of _KLTComputePyramid) + _KLTComputeGradients (reference src/V1/convolve.c:37-53,
@@ -201,6 +204,78 @@ __device__ __forceinline__ void stage_hgrad(const float* sL, float* sHd, float* 
   }
 }
 
+// ---- the next pyramid level (subsampling 2, radius 5) from a level tile on chip ----------------
+// L_{l+1}(X, Y) = S(2X+1, 2Y+1), S the separable Gaussian of L_l; a tile with origin (x0, y0) (both
+// even) makes the block X = x0/2 .. x0/2+TX/2-1, Y = y0/2 .. y0/2+TY/2-1, from L_l rows y0-4 ..
+// y0+TY+4 and columns x0-4 .. x0+TX+4.  Same operation sequence as lv_p1_item / P2 of
+// level_fused_kernel: taps in increasing order, horizontal before vertical, zero bands on the
+// source coordinate.
+static constexpr int NEXT_R = 5;
+// horizontal pass at the kept columns, every source row.  sL [NR][SP]: col c <-> x0-4+c, row r <->
+// y0-4+r.  sN [NR][NP]: col c <-> x0/2+c.  Lane mapping of stage_hgrad (a quarter warp is 4 groups x
+// 2 rows, conflict free on the loads because SP/4 is odd); the row units go to the warps in reverse
+// order, because the last warps are the ones stage_hgrad leaves idle in its last pass.
+template <bool EXACT, bool BORDER, int TX, int NR, int SP, int NP, int NTH = 256>
+__device__ __forceinline__ void stage_hnext(const float* sL, float* sN, const TapsF& tp, int x0, int Wsrc) {
+  constexpr int R = NEXT_R;
+  constexpr int NG = TX / 8;                        // groups of 4 kept columns: 8 or 4
+  constexpr int RPW = 32 / NG, NW = NTH / 32, NU = (NR + RPW - 1) / RPW;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int sub = lane & 3, rpar = (lane >> 2) & 1, rem = lane >> 3;
+  const int g = NG == 8 ? 4 * (rem & 1) + sub : sub;
+  const int rl = NG == 8 ? 2 * (rem >> 1) + rpar : 2 * rem + rpar;
+  for (int u = NW - 1 - warp; u < NU; u += NW) {
+    const int r = u * RPW + rl;
+    if (r < NR) {
+      float win[20];
+      const float* p = sL + r * SP + 8 * g;
+#pragma unroll
+      for (int v = 0; v < 5; ++v) {
+        const float4 t = lds128(p + 4 * v);
+        win[4 * v] = t.x; win[4 * v + 1] = t.y; win[4 * v + 2] = t.z; win[4 * v + 3] = t.w;
+      }
+      float o[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        float acc = 0.0f;
+#pragma unroll
+        for (int m = 0; m < 2 * R + 1; ++m) acc = mac<EXACT>(acc, win[2 * q + m], tp.k[m]);
+        if (BORDER) {
+          const int xs = x0 + 8 * g + 2 * q + 1;
+          if (xs < R || xs >= Wsrc - R) acc = 0.0f;
+        }
+        o[q] = acc;
+      }
+      *reinterpret_cast<float4*>(sN + r * NP + 4 * g) = make_float4(o[0], o[1], o[2], o[3]);
+    }
+  }
+}
+// vertical pass at the kept rows, stored to L_{l+1}: items of 4 columns x 1 row, handed out from the
+// last thread down (the gy half of stage_vgrad_both, whose derivative pass skips its centre tap, or
+// its idle threads, comes first).
+template <bool EXACT, bool BORDER, int TX, int TY, int NP, int NTH = 256>
+__device__ __forceinline__ void stage_vnext(const float* sN, const TapsF& tp, float* __restrict__ out, int npitch,
+                                            int x0, int y0, int Hsrc, int Wn, int Hn) {
+  constexpr int R = NEXT_R;
+  constexpr int NG = TX / 8, ITEMS = NG * (TY / 2);
+  const unsigned long long pol = store_policy(true);        // read back by the next kernel of the chain
+  for (int i = NTH - 1 - (int)threadIdx.x; i < ITEMS; i += NTH) {
+    const int yl = i / NG, g = i - yl * NG;
+    const float* src = sN + (2 * yl) * NP + 4 * g;
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+    for (int m = 0; m < 2 * R + 1; ++m) fma4(acc, lds128(src + m * NP), tp, m, EXACT);
+    const int X = x0 / 2 + 4 * g, Y = y0 / 2 + yl;
+    if (BORDER) {
+      const int ys = 2 * Y + 1;
+      if (ys < R || ys >= Hsrc - R) acc = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (X < Wn && Y < Hn) stg128(out + (size_t)Y * npitch + X, acc, pol);
+    } else {
+      stg128(out + (size_t)Y * npitch + X, acc, pol);
+    }
+  }
+}
+
 // ---- stage D: vertical 7-tap pass, 4 columns x PY rows per thread, straight to HBM ------------
 // scatter form: every loaded row feeds the outputs it belongs to, taps in increasing order
 // (== the reference's summation order for each output).
@@ -259,28 +334,38 @@ __device__ __forceinline__ void stage_vgrad_both(const float* sHd, const float* 
 // level 0
 // ============================================================================================
 // TY_: tile height; PYB_ / PYD_: output rows per thread of the two vertical stages; CPS_: resident
-// CTAs per SM the kernel is compiled for (register budget).
-template <int TY_, int PYB_, int PYD_, int CPS_>
+// CTAs per SM the kernel is compiled for (register budget).  NX_: the tile also makes its block of
+// L1 (subsampling 2, radius 5): L0 is computed XR rows above, XH - XR rows below and one column
+// right of what the gradients need, and the horizontal L1 pass gets a buffer of its own.
+template <int TY_, int PYB_, int PYD_, int CPS_, bool NX_ = false>
 struct L0GeoT {
   static constexpr int TX = 64, TY = TY_, PYB = PYB_, PYD = PYD_, CPS = CPS_;
+  static constexpr bool NX = NX_;
   static constexpr int RS = 2, RG = FUSED_RG;                          // smoothing / gradient radii
-  static constexpr int U8_W = 96, U8_H = TY + 2 * (RS + RG);           // 96 x 74 bytes, col c <-> x0-16+c
-  static constexpr int HS_P = 76, HS_H = U8_H;                         // col c <-> x0-4+c, row r <-> y0-5+r
-  static constexpr int L0_P = 76, L0_H = TY + 2 * RG;                  // row r <-> y0-3+r
-  static constexpr int HG_P = 68, HG_H = L0_H;                         // col c <-> x0+c
+  static constexpr int XR = NX ? NEXT_R - 1 - RG : 0, XH = NX ? 2 * (NEXT_R - 1 - RG) + 1 : 0;
+  static constexpr int U8_W = 96, U8_H = TY + 2 * (RS + RG) + XH;      // col c <-> x0-16+c
+  static constexpr int HS_P = 76, HS_H = U8_H;                         // col c <-> x0-4+c, row r <-> y0-5-XR+r
+  static constexpr int L0_P = 76, L0_H = TY + 2 * RG + XH;             // row r <-> y0-3-XR+r
+  static constexpr int HG_P = 68, HG_H = TY + 2 * RG;                  // col c <-> x0+c, row r <-> y0-3+r
+  static constexpr int NGB = NX ? 19 : 18;                             // stage B column groups of 4
+  static constexpr int N1_P = TX / 2 + 4;                              // horizontal L1 pass, col c <-> x0/2+c
   static constexpr int OFF_U8 = 0;
-  static constexpr int OFF_HS = U8_W * U8_H;                           // 7104
+  static constexpr int OFF_HS = U8_W * U8_H;
   static constexpr int OFF_L0 = OFF_HS + HS_H * HS_P * 4;
   static constexpr int OFF_HD = OFF_HS;                                // Hd reuses Hs
   static constexpr int OFF_HG = OFF_L0 + L0_H * L0_P * 4;
-  static constexpr int OFF_BAR = OFF_HG + HG_H * HG_P * 4;
+  static constexpr int OFF_N1 = OFF_HG + HG_H * HG_P * 4;
+  static constexpr int OFF_BAR = OFF_N1 + (NX ? L0_H * N1_P * 4 : 0);
   static constexpr int SMEM = OFF_BAR + 16;
-  static_assert(L0_H % PYB == 0 && TY % PYD == 0 && (TX / 4) * (TY / PYD) <= 128 && (L0_H / PYB) * 18 <= 256, "stage B / D mapping");
+  static_assert(L0_H % PYB == 0 && TY % PYD == 0 && (TX / 4) * (TY / PYD) <= 128 && (L0_H / PYB) * NGB <= 256, "stage B / D mapping");
+  static_assert(HG_H * HG_P <= HS_H * HS_P && 4 * NGB <= L0_P && 8 * 9 + (NX ? 4 : 0) <= HS_P, "buffer shapes");
+  static_assert(CPS * (SMEM + 1024) <= 228 * 1024, "CPS resident CTAs must fit into the SM's shared memory");
 };
 using L0Geo = L0GeoT<64, 5, 8, 3>;       // (tile width, halo and radii are the same for every variant)
 
-// stage A item: 8 outputs (Hs cols 8g..8g+7 <-> global x0-4+8g+q) of row r from 12 u8 pixels
-template <class G, bool EXACT, bool BORDER>
+// stage A item: NOUT (8, or 4 for the last column group of the NX geometry) outputs (Hs cols
+// 8g..8g+NOUT-1 <-> global x0-4+8g+q) of row r from 12 u8 pixels
+template <class G, bool EXACT, bool BORDER, int NOUT = 8>
 __device__ __forceinline__ void l0_stage_a_item(const unsigned char* sU8, float* sHs, const TapsF& ts,
                                                 int r, int g, int x0, int W) {
   constexpr int RS = G::RS;
@@ -295,7 +380,7 @@ __device__ __forceinline__ void l0_stage_a_item(const unsigned char* sU8, float*
   px[10] = u8_to_float(wb.y, 0); px[11] = u8_to_float(wb.y, 1);
   float o[8];
 #pragma unroll
-  for (int q = 0; q < 8; ++q) {
+  for (int q = 0; q < NOUT; ++q) {
     float acc = 0.0f;
 #pragma unroll
     for (int m = 0; m < 2 * RS + 1; ++m) acc = mac<EXACT>(acc, px[q + m], ts.k[m]);
@@ -307,7 +392,7 @@ __device__ __forceinline__ void l0_stage_a_item(const unsigned char* sU8, float*
   }
   float4* dst = reinterpret_cast<float4*>(sHs + r * G::HS_P + 8 * g);
   dst[0] = make_float4(o[0], o[1], o[2], o[3]);
-  dst[1] = make_float4(o[4], o[5], o[6], o[7]);
+  if (NOUT == 8) dst[1] = make_float4(o[4], o[5], o[6], o[7]);
 }
 
 template <class G, bool EXACT, bool BORDER>
@@ -325,34 +410,38 @@ __device__ __forceinline__ void l0_fused_tile(unsigned char* smem, int W, const 
       if (r < G::HS_H) l0_stage_a_item<G, EXACT, BORDER>(sU8, sHs, ts, r, 4 * half + sub, x0, W);
     }
     if (tid < G::HS_H) l0_stage_a_item<G, EXACT, BORDER>(sU8, sHs, ts, tid, 8, x0, W);   // 9th group
+    else if (G::NX && tid < 2 * G::HS_H)                                                   // col x0+68
+      l0_stage_a_item<G, EXACT, BORDER, 4>(sU8, sHs, ts, tid - G::HS_H, 9, x0, W);
   }
 }
 
 template <class G, bool EXACT, bool BORDER>
 __device__ __forceinline__ void l0_fused_tile_rest(unsigned char* smem, int W, int H, const TapsF& ts,
-                                                   const TapsF& tg, const TapsF& td,
+                                                   const TapsF& tg, const TapsF& td, const TapsF& tp,
                                                    float* __restrict__ out_img,
                                                    float* __restrict__ out_gx,
-                                                   float* __restrict__ out_gy, int opitch, int x0,
-                                                   int y0) {
-  constexpr int RS = G::RS, RG = G::RG;
+                                                   float* __restrict__ out_gy, int opitch,
+                                                   float* __restrict__ out_l1, int l1pitch, int W1, int H1,
+                                                   int x0, int y0) {
+  constexpr int RS = G::RS, RG = G::RG, XR = G::XR;
   float* sHs = reinterpret_cast<float*>(smem + G::OFF_HS);
   float* sL0 = reinterpret_cast<float*>(smem + G::OFF_L0);
   float* sHd = reinterpret_cast<float*>(smem + G::OFF_HD);
   float* sHg = reinterpret_cast<float*>(smem + G::OFF_HG);
+  float* sN1 = reinterpret_cast<float*>(smem + G::OFF_N1);
   const int tid = threadIdx.x;
 
   // ---- stage B: vertical Gaussian, Hs -> L0 (shared + HBM) ------------------------------------
-  // 18 column groups of 4 (col c <-> x0-4+c) x NBLK row blocks of PYB (14 x 5 for the 64-row tile).
+  // NGB column groups of 4 (col c <-> x0-4+c) x NBLK row blocks of PYB (14 x 5 for the 64-row tile).
   // The first 16 * NBLK threads take groups 0..15 (a quarter warp = 8 consecutive groups of one row
-  // block: contiguous 128 B), the next 2 * NBLK the two halo groups.
-  constexpr int NBLK = G::L0_H / G::PYB;
-  if (tid < 18 * NBLK) {
+  // block: contiguous 128 B), the next NH * NBLK the halo groups.
+  constexpr int NBLK = G::L0_H / G::PYB, NH = G::NGB - 16;
+  if (tid < G::NGB * NBLK) {
     constexpr int PY = G::PYB;
     const unsigned long long pol_img = store_policy(true);
     int blk, j;
     if (tid < 16 * NBLK) { blk = tid >> 4; j = tid & 15; }
-    else { blk = (tid - 16 * NBLK) >> 1; j = 16 + ((tid - 16 * NBLK) & 1); }
+    else { const int t2 = tid - 16 * NBLK; blk = t2 / NH; j = 16 + (t2 - blk * NH); }
     float4 acc[PY];
 #pragma unroll
     for (int q = 0; q < PY; ++q) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -370,12 +459,12 @@ __device__ __forceinline__ void l0_fused_tile_rest(unsigned char* smem, int W, i
 #pragma unroll
     for (int q = 0; q < PY; ++q) {
       const int rr = blk * PY + q;
-      const int yg = y0 - RG + rr;
+      const int yg = y0 - RG - XR + rr;
       if (BORDER) {
         if (yg < RS || yg >= H - RS) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
       }
       *reinterpret_cast<float4*>(sL0 + rr * G::L0_P + 4 * j) = acc[q];
-      if (j >= 1 && j <= 16 && rr >= RG && rr < RG + G::TY) {
+      if (j >= 1 && j <= 16 && rr >= RG + XR && rr < RG + XR + G::TY) {
         if (!BORDER || (xg < W && yg < H))
           stg128(out_img + (size_t)yg * opitch + xg, acc[q], pol_img);
       }
@@ -383,10 +472,12 @@ __device__ __forceinline__ void l0_fused_tile_rest(unsigned char* smem, int W, i
   }
   tile_sync();
 
-  stage_hgrad<EXACT, BORDER, G::TX, G::L0_H, G::L0_P, G::HG_P>(sL0, sHd, sHg, tg, td, x0, W);
+  stage_hgrad<EXACT, BORDER, G::TX, G::HG_H, G::L0_P, G::HG_P>(sL0 + XR * G::L0_P, sHd, sHg, tg, td, x0, W);
+  if (G::NX) stage_hnext<EXACT, BORDER, G::TX, G::L0_H, G::L0_P, G::N1_P>(sL0, sN1, tp, x0, W);
   tile_sync();
   stage_vgrad_both<EXACT, BORDER, G::TX, G::TY, G::PYD, G::HG_P>(sHd, sHg, tg, td, out_gx, out_gy, opitch,
                                                             x0, y0, W, H);
+  if (G::NX) stage_vnext<EXACT, BORDER, G::TX, G::TY, G::N1_P>(sN1, tp, out_l1, l1pitch, x0, y0, H, W1, H1);
 }
 
 // Tiles are handed out dynamically: a launch covers the tiles [tile0, ntiles) (whole tile rows when
@@ -400,7 +491,8 @@ __global__ void __launch_bounds__(256, G::CPS)
 l0_fused_kernel(const __grid_constant__ CUtensorMap map, int W, int H, int tiles_x, int tile0, int ntiles,
                 unsigned* __restrict__ counter, unsigned base,
                 TapsF ts, TapsF tg, TapsF td, float* __restrict__ out_img,
-                float* __restrict__ out_gx, float* __restrict__ out_gy, int opitch) {
+                float* __restrict__ out_gx, float* __restrict__ out_gy, int opitch,
+                TapsF tp, float* __restrict__ out_l1, int l1pitch, int W1, int H1) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem_raw + G::OFF_BAR);
   volatile int* s_next = reinterpret_cast<volatile int*>(smem_raw + G::OFF_BAR + 8);
@@ -421,7 +513,7 @@ l0_fused_kernel(const __grid_constant__ CUtensorMap map, int W, int H, int tiles
     if (t < ntiles) {
       mbar_expect_tx(bar, G::U8_W * G::U8_H);
       tma_load_2d(smem_raw + G::OFF_U8, &map, (t % tiles_x) * G::TX - 16,
-                  (t / tiles_x) * G::TY - (G::RS + G::RG), bar);
+                  (t / tiles_x) * G::TY - (G::RS + G::RG + G::XR), bar);
     }
   }
   __syncthreads();
@@ -443,12 +535,16 @@ l0_fused_kernel(const __grid_constant__ CUtensorMap map, int W, int H, int tiles
       if (t < ntiles) {
         mbar_expect_tx(bar, G::U8_W * G::U8_H);
         tma_load_2d(smem_raw + G::OFF_U8, &map, (t % tiles_x) * G::TX - 16,
-                    (t / tiles_x) * G::TY - (G::RS + G::RG), bar);
+                    (t / tiles_x) * G::TY - (G::RS + G::RG + G::XR), bar);
       }
     }
     if (!waited) { pdl_wait(); waited = true; }
-    if (border) l0_fused_tile_rest<G, EXACT, true>(smem_raw, W, H, ts, tg, td, out_img, out_gx, out_gy, opitch, x0, y0);
-    else l0_fused_tile_rest<G, EXACT, false>(smem_raw, W, H, ts, tg, td, out_img, out_gx, out_gy, opitch, x0, y0);
+    if (border)
+      l0_fused_tile_rest<G, EXACT, true>(smem_raw, W, H, ts, tg, td, tp, out_img, out_gx, out_gy, opitch, out_l1, l1pitch,
+                                         W1, H1, x0, y0);
+    else
+      l0_fused_tile_rest<G, EXACT, false>(smem_raw, W, H, ts, tg, td, tp, out_img, out_gx, out_gy, opitch, out_l1, l1pitch,
+                                          W1, H1, x0, y0);
     // stage D reads Hd (aliased on Hs) and Hg: the next tile's stage A must not start before
     __syncthreads();
     tile = *s_next;
@@ -665,3 +761,97 @@ level_fused_kernel(const __grid_constant__ CUtensorMap map, int Wsrc, int Hsrc, 
   pdl_launch_dependents();            // queue empty: the next kernel of the chain may move in
 }
 
+// ============================================================================================
+// levels >= 1 of a subsampling-2, radius-5 pyramid whose level 0 came from the NX geometry:
+// L_l -> gx_l, gy_l (+ L_{l+1} when NX).  The pyramid step of level l has already been done by the
+// previous kernel of the chain, from the tile it held on chip, so a tile only loads its own part of
+// L_l plus the halo of the two passes (76 x 41 floats for 64 x 32) and runs two stages:
+//   1: horizontal DoG / Gaussian (stage_hgrad) + horizontal pass of the next level
+//   2: vertical Gaussian / DoG (stage_vgrad_both) + vertical pass and store of the next level
+// ============================================================================================
+template <int TX, int TY>
+struct ChGeo {
+  static constexpr int RG = FUSED_RG, RN = NEXT_R;
+  static constexpr int SW = TX + 12, SH = TY + 2 * RN - 1;             // col c <-> x0-4+c, row r <-> y0-4+r
+  static constexpr int HP = TX + 4, GH = TY + 2 * RG;                  // Hd / Hg: col c <-> x0+c, row r <-> y0-3+r
+  static constexpr int NP = TX / 2 + 4;                                // next level's horizontal pass
+  static_assert(SW >= TX + 2 * RN - 1 && (SW / 4) % 2 == 1 && (HP / 4) % 2 == 1, "box width / odd chunk pitches");
+  static_assert(RN - 1 - RG >= 0, "the gradient rows lie inside the box");
+  static constexpr int OFF_SRC = 0;
+  static constexpr int OFF_HD = OFF_SRC + SW * SH * 4;
+  static constexpr int OFF_HG = OFF_HD + GH * HP * 4;
+  static constexpr int OFF_N = OFF_HG + GH * HP * 4;
+  static constexpr int OFF_BAR = OFF_N + SH * NP * 4;
+  static constexpr int SMEM = OFF_BAR + 16;
+};
+
+// W,H: size of level l; Wn,Hn: size of level l+1 (unused without NX).  Dynamic tile scheduler and
+// programmatic dependent launch as in level_fused_kernel.
+template <int TX, int TY, bool NX, bool EXACT>
+__global__ void __launch_bounds__(256, 4)
+level_chain_kernel(const __grid_constant__ CUtensorMap map, int W, int H, int Wn, int Hn,
+                   int tiles_x, int tile0, int ntiles, unsigned* __restrict__ counter, unsigned base,
+                   TapsF tp, TapsF tg, TapsF td, float* __restrict__ out_gx, float* __restrict__ out_gy,
+                   int opitch, float* __restrict__ out_next, int npitch) {
+  using G = ChGeo<TX, TY>;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem_raw + G::OFF_BAR);
+  volatile int* s_next = reinterpret_cast<volatile int*>(smem_raw + G::OFF_BAR + 8);
+  const float* sL = reinterpret_cast<const float*>(smem_raw + G::OFF_SRC);
+  float* sHd = reinterpret_cast<float*>(smem_raw + G::OFF_HD);
+  float* sHg = reinterpret_cast<float*>(smem_raw + G::OFF_HG);
+  float* sN = reinterpret_cast<float*>(smem_raw + G::OFF_N);
+  const int tid = threadIdx.x;
+  if (tid == 0) {
+    mbar_init(bar, 1);
+    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<unsigned long long>(&map)) : "memory");
+  }
+  pdl_wait();                         // L_l is written by the previous kernel
+  if (tid == 0) {
+    const int t = tile0 + (int)(atomicAdd(counter, 1u) - base);
+    *s_next = t;
+    if (t < ntiles) {
+      mbar_expect_tx(bar, G::SW * G::SH * 4);
+      tma_load_2d(smem_raw + G::OFF_SRC, &map, (t % tiles_x) * TX - 4, (t / tiles_x) * TY + 1 - G::RN, bar);
+    }
+  }
+  __syncthreads();
+  int tile = *s_next;
+  unsigned phase = 0;
+  // output rows per thread of stage 2: as few as the thread count allows (fewer rows = more items)
+  constexpr int PY = (TX / 4) * (TY / 2) <= 128 ? 2 : ((TX / 4) * (TY / 4) <= 128 ? 4 : 8);
+  while (tile < ntiles) {
+    const int x0 = (tile % tiles_x) * TX, y0 = (tile / tiles_x) * TY;
+    // tiles whose 8-pixel margin stays inside level l meet no zero band of either pass and no edge
+    const bool border = (x0 < 8) || (y0 < 8) || (x0 + TX + 8 > W) || (y0 + TY + 8 > H);
+    mbar_wait(bar, phase);
+    phase ^= 1;
+    const float* sLg = sL + (G::RN - 1 - G::RG) * G::SW;
+    if (border) {
+      stage_hgrad<EXACT, true, TX, G::GH, G::SW, G::HP>(sLg, sHd, sHg, tg, td, x0, W);
+      if (NX) stage_hnext<EXACT, true, TX, G::SH, G::SW, G::NP>(sL, sN, tp, x0, W);
+    } else {
+      stage_hgrad<EXACT, false, TX, G::GH, G::SW, G::HP>(sLg, sHd, sHg, tg, td, x0, W);
+      if (NX) stage_hnext<EXACT, false, TX, G::SH, G::SW, G::NP>(sL, sN, tp, x0, W);
+    }
+    __syncthreads();                 // source box consumed; everybody has read s_next
+    if (tid == 0) {
+      const int t = tile0 + (int)(atomicAdd(counter, 1u) - base);
+      *s_next = t;
+      if (t < ntiles) {
+        mbar_expect_tx(bar, G::SW * G::SH * 4);
+        tma_load_2d(smem_raw + G::OFF_SRC, &map, (t % tiles_x) * TX - 4, (t / tiles_x) * TY + 1 - G::RN, bar);
+      }
+    }
+    if (border) {
+      stage_vgrad_both<EXACT, true, TX, TY, PY, G::HP>(sHd, sHg, tg, td, out_gx, out_gy, opitch, x0, y0, W, H);
+      if (NX) stage_vnext<EXACT, true, TX, TY, G::NP>(sN, tp, out_next, npitch, x0, y0, H, Wn, Hn);
+    } else {
+      stage_vgrad_both<EXACT, false, TX, TY, PY, G::HP>(sHd, sHg, tg, td, out_gx, out_gy, opitch, x0, y0, W, H);
+      if (NX) stage_vnext<EXACT, false, TX, TY, G::NP>(sN, tp, out_next, npitch, x0, y0, H, Wn, Hn);
+    }
+    __syncthreads();                 // Hd / Hg / next-level buffer free for the next tile
+    tile = *s_next;
+  }
+  pdl_launch_dependents();            // queue empty: the next kernel of the chain may move in
+}
