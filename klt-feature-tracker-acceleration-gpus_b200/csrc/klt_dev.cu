@@ -1222,6 +1222,8 @@ static constexpr int KLT_BAND_EVENTS = 64; // events cycled by the banded frame 
 
 static constexpr int KLT_SNAP_MAX = 64;
 static constexpr int KLT_HOST_REGS = 32; // pageable frame buffers remembered per context
+static constexpr int KLT_TILE_QUEUES = 16;
+static_assert(KLT_DEV_MAX_LEVELS <= KLT_TILE_QUEUES, "one tile queue per pyramid level");
 struct Level {
   int w, h, pitch;           // pitch in floats
   float *img, *gx, *gy;
@@ -1248,7 +1250,7 @@ struct klt_dev {
   cudaEvent_t ev_join;
   char err[512];
   unsigned long long launches;
-  int last_path, force_generic, no_fused, last_fused, track7_off, overlap_l0_ctas;
+  int last_path, force_generic, no_fused, last_fused, track7_off;
   // geometry
   int W, H, L, ss;
   PyrSet set[KLT_DEV_SLOTS];
@@ -1295,8 +1297,8 @@ struct klt_dev {
   int* rank_list; int* sel_state;      // candidates still uncovered (ranks, ascending) / [0..2] walk state, [4] their number
   int no_filter; int replace_filter;
   int enforce_attr;            // enforce_mindist_kernel's shared-memory attribute set on this device
-  // dynamic tile scheduler of the persistent kernels: one counter per launch site
-  unsigned* d_tile_ctr; unsigned tile_base[16];
+  // tile queues of the persistent pyramid kernels: one counter per pyramid level
+  unsigned* d_tile_ctr; unsigned tile_base[KLT_TILE_QUEUES];
   // timing
   cudaEvent_t ev_a, ev_b; int ev_made;
   // per-kernel profiling (klt_dev_profile_*)
@@ -1469,7 +1471,6 @@ extern "C" int klt_dev_create(int device, klt_dev** out) {
   if (e != cudaSuccess) { free(c); return fail(nullptr, "cudaStreamCreate: %s", cudaGetErrorString(e)); }
   c->tstream = c->stream;
   c->fb_n = -1;
-  c->overlap_l0_ctas = getenv("KLT_B200_OVERLAP_L0_CTAS") ? atoi(getenv("KLT_B200_OVERLAP_L0_CTAS")) : 0;
   e = cudaMalloc(&c->d_live, sizeof(unsigned long long));
   if (e == cudaSuccess) e = cudaMemsetAsync(c->d_live, 0, sizeof(unsigned long long), c->stream);
   c->pdl = getenv("KLT_B200_PDL") ? atoi(getenv("KLT_B200_PDL")) : 1;
@@ -1487,8 +1488,8 @@ extern "C" int klt_dev_create(int device, klt_dev** out) {
     cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want);
     fprintf(stderr, "(KLT/B200) persisting L2: %zu MB of max %d MB\n", want >> 20, maxb >> 20);
   }
-  if (e == cudaSuccess) e = cudaMalloc(&c->d_tile_ctr, 16 * sizeof(unsigned));
-  if (e == cudaSuccess) e = cudaMemsetAsync(c->d_tile_ctr, 0, 16 * sizeof(unsigned), c->stream);
+  if (e == cudaSuccess) e = cudaMalloc(&c->d_tile_ctr, KLT_TILE_QUEUES * sizeof(unsigned));
+  if (e == cudaSuccess) e = cudaMemsetAsync(c->d_tile_ctr, 0, KLT_TILE_QUEUES * sizeof(unsigned), c->stream);
   if (e != cudaSuccess) { cudaStreamDestroy(c->stream); free(c); return fail(nullptr, "cudaMalloc: %s", cudaGetErrorString(e)); }
   *out = c;
   return 0;
@@ -1829,17 +1830,19 @@ static bool fused_grad_taps_ok(const TapsR& tg, const TapsR& td) {
 // ---- fused kernels: plan (tensor maps, tile shapes) + launches over whole tile rows ------------
 // A launch covers the tile rows [jr0, jr1) of one level, so that a frame can be built band by band
 // behind its upload (klt_dev_build with a host frame) or in one go (jr0 = 0, jr1 = tiles_y).
-enum LevelShape { SHAPE_NONE = 0, SHAPE_2_5_64_32, SHAPE_2_5_64_16, SHAPE_2_5_32_16, SHAPE_4_10_32_16, SHAPE_2_5_64_24 };
+enum LevelShape { SHAPE_NONE = 0, SHAPE_2_5_64_32, SHAPE_2_5_64_16, SHAPE_2_5_32_16, SHAPE_4_10_32_16 };
 struct FusedPlan {
-  const unsigned char* src; int spitch;
   bool l0_ok;                                   // level 0 runs on l0_fused_kernel
   int shape[KLT_DEV_MAX_LEVELS];                // LevelShape of level l >= 1 (SHAPE_NONE: not fused)
   CUtensorMap map[KLT_DEV_MAX_LEVELS];          // source of level l (u8 frame for l = 0, L_{l-1} else)
   int TX[KLT_DEV_MAX_LEVELS], TY[KLT_DEV_MAX_LEVELS], tiles_x[KLT_DEV_MAX_LEVELS], tiles_y[KLT_DEV_MAX_LEVELS];
-  int SS, R;                                    // pyramid step geometry of the fused level kernels
   bool l0_march;                                // level 0 on l0_march_kernel (strips x segments) instead of tiles
   bool chain;                                   // level 0 on L0GeoC (also makes L1), levels >= 1 on
                                                 // level_chain_kernel (map[l]: L_l itself)
+  // band schedule: tile row j of level l reads rows [0, need_mul * (j + 1) + need_add) of plane src_plane[l]
+  // and completes rows [0, made_mul * j) of the plane level l + 1 reads (plane 0: the u8 frame, k + 1: L_k)
+  int src_plane[KLT_DEV_MAX_LEVELS], need_mul[KLT_DEV_MAX_LEVELS], need_add[KLT_DEV_MAX_LEVELS],
+      made_mul[KLT_DEV_MAX_LEVELS];
 };
 
 static int level_shape_for(int ss, int r, int w, int h, int num_sms) {
@@ -1849,25 +1852,26 @@ static int level_shape_for(int ss, int r, int w, int h, int num_sms) {
     // (4K level 2: 960x540) the wave count decides: 64x32 tiles when they all fit into ONE wave of
     // 2 CTAs per SM (255 tiles: 10.6 us), else 64x16 tiles at 3 CTAs per SM (510 tiles = 1.15
     // waves: 12.7 us; measured on the 4K step: 74.1 -> 72.8 us).
-    static int force = getenv("KLT_B200_LEVEL_TILE") ? atoi(getenv("KLT_B200_LEVEL_TILE")) : 0;
     const long px = (long)w * h;
     const long tiles_64x32 = (long)((w + 63) / 64) * ((h + 31) / 32);
-    const int mid = tiles_64x32 <= 2L * num_sms ? 1 : 2;
-    const int shape = force ? force : (px >= 1500000 ? 1 : (px >= 300000 ? mid : 3));
-    return shape == 1 ? SHAPE_2_5_64_32 : (shape == 2 ? SHAPE_2_5_64_16 : (shape == 4 ? SHAPE_2_5_64_24 : SHAPE_2_5_32_16));
+    if (px >= 1500000) return SHAPE_2_5_64_32;
+    if (px >= 300000) return tiles_64x32 <= 2L * num_sms ? SHAPE_2_5_64_32 : SHAPE_2_5_64_16;
+    return SHAPE_2_5_32_16;
   }
   if (ss == 4 && r == 10) return SHAPE_4_10_32_16;
   return SHAPE_NONE;
 }
-template <int TX, int TY>
-static bool chain_map(CUtensorMap* m, const Level& a) {
-  using G = ChGeo<TX, TY>;
-  return make_tensor_map(m, a.img, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.w, a.h, (size_t)a.pitch * 4, G::SW, G::SH);
-}
-template <int SS, int R, int TX, int TY>
-static bool level_map(CUtensorMap* m, const Level& a) {
-  using G = LvGeo<SS, R, TX, TY>;
-  return make_tensor_map(m, a.img, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.w, a.h, (size_t)a.pitch * 4, G::SW, G::SH);
+template <int SS_, int R_, int TX_, int TY_>
+struct TileShape { static constexpr int SS = SS_, R = R_, TX = TX_, TY = TY_; };
+// The one place where a LevelShape (never SHAPE_NONE) becomes template arguments: f(TileShape<...>()).
+template <class F>
+static auto with_shape(int shape, F f) {
+  switch (shape) {
+    case SHAPE_2_5_64_32: return f(TileShape<2, 5, 64, 32>());
+    case SHAPE_2_5_64_16: return f(TileShape<2, 5, 64, 16>());
+    case SHAPE_2_5_32_16: return f(TileShape<2, 5, 32, 16>());
+    default: return f(TileShape<4, 10, 32, 16>());       // SHAPE_4_10_32_16
+  }
 }
 
 using L0GeoB = L0GeoT<48, 6, 6, 4>;      // 48-row tiles: 2 even passes in stages A / C, 54 KB of shared memory, 4 CTAs / SM
@@ -1884,27 +1888,24 @@ static int l0_variant() {
 }
 extern "C" void klt_dev_set_l0_kernel(int variant) { g_l0_variant = variant; }
 extern "C" int klt_dev_l0_kernel(void) { return l0_variant(); }
-// which levels of this build can run on the fused kernels, and their tensor maps
+// which levels of this build can run on the fused kernels, their tensor maps and band schedule
 static void fused_plan(klt_dev* d, const PyrSet& S, const unsigned char* src, int spitch,
                        const klt_dev_build_desc* q, const TapsR& ts, const TapsR& tp, const TapsR& tg,
-                       const TapsR& td, FusedPlan* P, int force_shape) {
+                       const TapsR& td, FusedPlan* P) {
   memset(P, 0, sizeof(*P));
   if (d->force_generic || d->no_fused || !fused_grad_taps_ok(tg, td)) return;
   const int W = q->ncols, H = q->nrows;
-  P->src = src; P->spitch = spitch;
   const int l0_ty = l0_variant() == 1 ? L0GeoB::TY : L0Geo::TY, l0_u8h = l0_variant() == 1 ? L0GeoB::U8_H : L0Geo::U8_H;
   if (l0_variant() == 2 && q->smooth && ts.w == 2 * MarchGeo::RS + 1 &&
       make_tensor_map(&P->map[0], src, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, W, H, (size_t)spitch, MarchGeo::IN_W, MarchGeo::PU)) {
     // strips of 120 columns x segments of rows, one task per team of the grid when the frame is big
     // enough (4K: 32 strips x 37 segments of 59 rows = 1184 tasks = 148 SMs x 2 CTAs x 4 teams)
-    static int force_seg = getenv("KLT_B200_L0_SEG") ? atoi(getenv("KLT_B200_L0_SEG")) : 0;
     const int nstrips = (W + MarchGeo::SWI - 1) / MarchGeo::SWI;
     const int teams = MarchGeo::CPS * d->num_sms * MarchGeo::TEAMS;
     int nseg = teams / nstrips;
     if (nseg < 1) nseg = 1;
     int seg_rows = (H + nseg - 1) / nseg;
     if (seg_rows < 16) seg_rows = 16;
-    if (force_seg > 0) seg_rows = force_seg;
     P->l0_ok = true; P->l0_march = true;
     P->TX[0] = MarchGeo::SWI; P->TY[0] = seg_rows;
     P->tiles_x[0] = nstrips; P->tiles_y[0] = (H + seg_rows - 1) / seg_rows;
@@ -1914,6 +1915,7 @@ static void fused_plan(klt_dev* d, const PyrSet& S, const unsigned char* src, in
     P->TX[0] = L0Geo::TX; P->TY[0] = l0_ty;
     P->tiles_x[0] = (W + L0Geo::TX - 1) / L0Geo::TX; P->tiles_y[0] = (H + l0_ty - 1) / l0_ty;
   }
+  P->need_add[0] = L0Geo::RS + L0Geo::RG;       // u8 rows a level-0 tile row reads below its last output row
   // Chained pyramid: level 0 makes L1, level l makes L_{l+1}, so every level >= 1 reads only its own
   // plane.  The default level-0 variant with subsampling 2 / radius 5 and every level fused; builds of
   // one level keep L0GeoB.
@@ -1929,188 +1931,130 @@ static void fused_plan(klt_dev* d, const PyrSet& S, const unsigned char* src, in
       P->map[0] = m0;
       P->TY[0] = L0GeoC::TY;
       P->tiles_y[0] = (H + L0GeoC::TY - 1) / L0GeoC::TY;
+      P->need_add[0] = L0GeoC::U8_H - L0GeoC::TY - (L0GeoC::RS + L0GeoC::RG + L0GeoC::XR);
     }
   }
-  P->SS = q->subsampling; P->R = tp.w / 2;
+  P->need_mul[0] = P->TY[0];
+  P->made_mul[0] = P->chain ? P->TY[0] / 2 : P->TY[0];
   for (int l = 1; l < q->nlevels_built; ++l) {
-    const Level& a = S.lv[l - 1];
-    const Level& b = S.lv[l];
-    int shape = force_shape != SHAPE_NONE ? force_shape : level_shape_for(q->subsampling, tp.w / 2, b.w, b.h, d->num_sms);
-    bool ok = false;
-    if (P->chain) {
-      switch (shape) {
-        case SHAPE_2_5_64_32: ok = chain_map<64, 32>(&P->map[l], b); P->TX[l] = 64; P->TY[l] = 32; break;
-        case SHAPE_2_5_64_24: ok = chain_map<64, 24>(&P->map[l], b); P->TX[l] = 64; P->TY[l] = 24; break;
-        case SHAPE_2_5_64_16: ok = chain_map<64, 16>(&P->map[l], b); P->TX[l] = 64; P->TY[l] = 16; break;
-        case SHAPE_2_5_32_16: ok = chain_map<32, 16>(&P->map[l], b); P->TX[l] = 32; P->TY[l] = 16; break;
-        default: break;
+    const int shape = level_shape_for(q->subsampling, tp.w / 2, S.lv[l].w, S.lv[l].h, d->num_sms);
+    if (shape == SHAPE_NONE) continue;
+    const Level& a = S.lv[P->chain ? l : l - 1];             // the plane the level's tiles read
+    const bool ok = with_shape(shape, [&](auto s) {
+      using T = decltype(s);
+      P->TX[l] = T::TX; P->TY[l] = T::TY;
+      if (P->chain) {                                         // L_l -> gx_l, gy_l, L_{l+1}
+        using G = ChGeo<T::TX, T::TY>;
+        P->src_plane[l] = l + 1;
+        P->need_mul[l] = T::TY; P->need_add[l] = 1 - G::RN + G::SH - T::TY; P->made_mul[l] = T::TY / 2;
+        return make_tensor_map(&P->map[l], a.img, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.w, a.h, (size_t)a.pitch * 4,
+                               G::SW, G::SH);
       }
-      if (!ok) { memset(P, 0, sizeof(*P)); return; }   // tensor map refused: nothing runs fused
-      P->shape[l] = shape;
-      P->tiles_x[l] = (b.w + P->TX[l] - 1) / P->TX[l];
-      P->tiles_y[l] = (b.h + P->TY[l] - 1) / P->TY[l];
+      using G = LvGeo<T::SS, T::R, T::TX, T::TY>;            // L_{l-1} -> L_l, gx_l, gy_l
+      P->src_plane[l] = l;
+      P->need_mul[l] = T::SS * T::TY; P->need_add[l] = G::YOFF + G::SH - T::SS * T::TY; P->made_mul[l] = T::TY;
+      return make_tensor_map(&P->map[l], a.img, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.w, a.h, (size_t)a.pitch * 4,
+                             G::SW, G::SH);
+    });
+    if (!ok) {
+      if (P->chain) { memset(P, 0, sizeof(*P)); return; }   // tensor map refused: nothing runs fused
       continue;
     }
-    switch (shape) {
-      case SHAPE_2_5_64_32: ok = level_map<2, 5, 64, 32>(&P->map[l], a); P->TX[l] = 64; P->TY[l] = 32; break;
-      case SHAPE_2_5_64_24: ok = level_map<2, 5, 64, 24>(&P->map[l], a); P->TX[l] = 64; P->TY[l] = 24; break;
-      case SHAPE_2_5_64_16: ok = level_map<2, 5, 64, 16>(&P->map[l], a); P->TX[l] = 64; P->TY[l] = 16; break;
-      case SHAPE_2_5_32_16: ok = level_map<2, 5, 32, 16>(&P->map[l], a); P->TX[l] = 32; P->TY[l] = 16; break;
-      case SHAPE_4_10_32_16: ok = level_map<4, 10, 32, 16>(&P->map[l], a); P->TX[l] = 32; P->TY[l] = 16; break;
-      default: break;
-    }
-    if (!ok) { shape = SHAPE_NONE; continue; }
     P->shape[l] = shape;
-    P->tiles_x[l] = (b.w + P->TX[l] - 1) / P->TX[l];
-    P->tiles_y[l] = (b.h + P->TY[l] - 1) / P->TY[l];
+    P->tiles_x[l] = (S.lv[l].w + P->TX[l] - 1) / P->TX[l];
+    P->tiles_y[l] = (S.lv[l].h + P->TY[l] - 1) / P->TY[l];
   }
 }
 
-// fused level 0 (u8 -> L0, gx0, gy0 (+ L1 with G::NX)), tile rows [jr0, jr1)
+// One launch of a persistent pyramid kernel K: ctas is what the work can use, the grid is at most what
+// the SMs hold.  K's shared-memory attribute and resident CTAs per SM are looked up once per device.
+template <auto K, typename... Args>
+static int launch_persistent(klt_dev* d, int kid, int nth, int smem, int ctas, int* grid, Args... args) {
+  static int cps_dev[64] = {};                   // (function attributes are per device; 0: not set yet)
+  int& cps = cps_dev[d->device & 63];
+  if (!cps) {
+    int n = 0;
+    CU(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, K, nth, smem));
+    cps = n < 1 ? 1 : n;
+  }
+  *grid = ctas < cps * d->num_sms ? ctas : cps * d->num_sms;
+  Launch l(d, kid);
+  CU(launch_k(K, dim3(*grid), dim3(nth), smem, d->stream, d->pdl != 0, args...));
+  return 0;
+}
+// K over the tile rows [jr0, jr1) of pyramid level `level`, from that level's tile queue.  QUEUE marks
+// where K takes its TileQueue among args.
+struct QueueSlot {};
+static constexpr QueueSlot QUEUE{};
+template <class T> static T fill_queue(T a, const TileQueue&) { return a; }
+static TileQueue fill_queue(QueueSlot, const TileQueue& q) { return q; }
+template <auto K, typename... Args>
+static int launch_tiles(klt_dev* d, int kid, int level, int nth, int smem, int tiles_x, int jr0, int jr1,
+                        Args... args) {
+  const int n = (jr1 - jr0) * tiles_x;
+  const TileQueue q = {tiles_x, jr0 * tiles_x, jr1 * tiles_x, d->d_tile_ctr + level, d->tile_base[level]};
+  int grid = 0;
+  if (launch_persistent<K>(d, kid, nth, smem, n, &grid, fill_queue(args, q)...)) return 1;
+  d->tile_base[level] += (unsigned)(n + grid);
+  return 0;
+}
+
+// level 0 (u8 -> L0, gx0, gy0 (+ L1 when the plan is chained)), tile rows [jr0, jr1)
 template <class G, bool EXACT>
-static int l0_fused_launch_t(klt_dev* d, const FusedPlan& P, int W, int H, const TapsR& ts, const TapsR& tg,
-                             const TapsR& td, const TapsR& tp, const Level& lv, const Level* l1, int jr0, int jr1) {
-  static bool attr_dev[64] = {};                 // function attributes are per device
-  bool& attr_set = attr_dev[d->device & 63];
-  static int cps = 0;
-  if (!attr_set) {
-    CU(cudaFuncSetAttribute(l0_fused_kernel<G, EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cps, l0_fused_kernel<G, EXACT>, 256, G::SMEM));
-    if (cps < 1) cps = 1;
-    attr_set = true;
-  }
-  const int tiles_x = P.tiles_x[0];
-  const int tile0 = jr0 * tiles_x, tile1 = jr1 * tiles_x, n = tile1 - tile0;
-  const int per_sm = (d->overlap && d->overlap_l0_ctas > 0) ? d->overlap_l0_ctas : cps;
-  const int grid = n < per_sm * d->num_sms ? n : per_sm * d->num_sms;         // persistent
-  { Launch l(d, KID_L0_FUSED);
-    CU(launch_k(l0_fused_kernel<G, EXACT>, dim3(grid), dim3(256), G::SMEM, d->stream, d->pdl != 0, P.map[0], W, H,
-                tiles_x, tile0, tile1, d->d_tile_ctr, d->tile_base[0], to_fused(ts), to_fused(tg), to_fused(td), lv.img,
-                lv.gx, lv.gy, lv.pitch, to_fused(tp), l1 ? l1->img : nullptr, l1 ? l1->pitch : 0, l1 ? l1->w : 0,
-                l1 ? l1->h : 0));
-    d->tile_base[0] += (unsigned)(n + grid); }
-  return 0;
+static int l0_tiles_launch(klt_dev* d, const FusedPlan& P, int W, int H, const TapsR& ts, const TapsR& tg,
+                           const TapsR& td, const TapsR& tp, const Level& lv, const Level* l1, int jr0, int jr1) {
+  return launch_tiles<l0_fused_kernel<G, EXACT>>(
+      d, KID_L0_FUSED, 0, 256, G::SMEM, P.tiles_x[0], jr0, jr1, P.map[0], W, H, QUEUE, to_fused(ts), to_fused(tg),
+      to_fused(td), lv.img, lv.gx, lv.gy, lv.pitch, to_fused(tp), l1 ? l1->img : nullptr, l1 ? l1->pitch : 0,
+      l1 ? l1->w : 0, l1 ? l1->h : 0);
 }
-// level 0 on the marching kernel, segments [jr0, jr1)
-template <bool EXACT>
-static int l0_march_launch(klt_dev* d, const FusedPlan& P, int W, int H, const TapsR& ts, const TapsR& tg,
-                           const TapsR& td, const Level& lv, int jr0, int jr1) {
-  using G = MarchGeo;
-  static bool attr_dev[64] = {};                 // function attributes are per device
-  bool& attr_set = attr_dev[d->device & 63];
-  static int cps = 0;
-  if (!attr_set) {
-    CU(cudaFuncSetAttribute(l0_march_kernel<EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cps, l0_march_kernel<EXACT>, G::NTH, G::SMEM));
-    if (cps < 1) cps = 1;
-    attr_set = true;
-  }
-  const int nstrips = P.tiles_x[0];
-  const int task0 = jr0 * nstrips, task1 = jr1 * nstrips, n = task1 - task0;
-  const int ctas = (n + G::TEAMS - 1) / G::TEAMS;
-  const int grid = ctas < cps * d->num_sms ? ctas : cps * d->num_sms;
-  { Launch l(d, KID_L0_FUSED);
-    CU(launch_k(l0_march_kernel<EXACT>, dim3(grid), dim3(G::NTH), G::SMEM, d->stream, d->pdl != 0, P.map[0], W, H,
-                nstrips, P.TY[0], task0, task1, to_fused(ts), to_fused(tg), to_fused(td), lv.img, lv.gx, lv.gy, lv.pitch)); }
-  return 0;
-}
-// l1: level 1, made by the same kernel when the plan is chained (else unused)
 template <bool EXACT>
 static int l0_fused_launch(klt_dev* d, const FusedPlan& P, int W, int H, const TapsR& ts, const TapsR& tg,
-                           const TapsR& td, const TapsR& tp, const Level& lv, const Level& l1, int jr0, int jr1) {
+                           const TapsR& td, const TapsR& tp, const PyrSet& S, int jr0, int jr1) {
   if (jr1 <= jr0) return 0;
-  if (P.l0_march) return l0_march_launch<EXACT>(d, P, W, H, ts, tg, td, lv, jr0, jr1);
-  if (P.chain) return l0_fused_launch_t<L0GeoC, EXACT>(d, P, W, H, ts, tg, td, tp, lv, &l1, jr0, jr1);
-  switch (P.TY[0]) {
-    case L0GeoB::TY: return l0_fused_launch_t<L0GeoB, EXACT>(d, P, W, H, ts, tg, td, tp, lv, nullptr, jr0, jr1);
-    default: return l0_fused_launch_t<L0Geo, EXACT>(d, P, W, H, ts, tg, td, tp, lv, nullptr, jr0, jr1);
+  if (P.l0_march) {                              // segments [jr0, jr1) of every strip, TEAMS tasks per CTA
+    using G = MarchGeo;
+    const int nstrips = P.tiles_x[0], task0 = jr0 * nstrips, task1 = jr1 * nstrips;
+    int grid = 0;
+    return launch_persistent<l0_march_kernel<EXACT>>(
+        d, KID_L0_FUSED, G::NTH, G::SMEM, (task1 - task0 + G::TEAMS - 1) / G::TEAMS, &grid, P.map[0], W, H, nstrips,
+        P.TY[0], task0, task1, to_fused(ts), to_fused(tg), to_fused(td), S.lv[0].img, S.lv[0].gx, S.lv[0].gy,
+        S.lv[0].pitch);
   }
+  if (P.chain) return l0_tiles_launch<L0GeoC, EXACT>(d, P, W, H, ts, tg, td, tp, S.lv[0], &S.lv[1], jr0, jr1);
+  if (P.TY[0] == L0GeoB::TY) return l0_tiles_launch<L0GeoB, EXACT>(d, P, W, H, ts, tg, td, tp, S.lv[0], nullptr, jr0, jr1);
+  return l0_tiles_launch<L0Geo, EXACT>(d, P, W, H, ts, tg, td, tp, S.lv[0], nullptr, jr0, jr1);
 }
 
-// fused coarser level (L_{l-1} -> L_l, gx_l, gy_l), tile rows [jr0, jr1)
-template <int SS, int R, int TX, int TY, bool EXACT>
-static int level_fused_launch_t(klt_dev* d, const FusedPlan& P, int level, const Level& a, const Level& b,
-                                const TapsR& tp, const TapsR& tg, const TapsR& td, int jr0, int jr1) {
-  using G = LvGeo<SS, R, TX, TY>;
-  static bool attr_dev[64] = {};                 // function attributes are per device
-  bool& attr_set = attr_dev[d->device & 63];
-  static int cps = 0;                                                       // resident CTAs per SM
-  if (!attr_set) {
-    CU(cudaFuncSetAttribute(level_fused_kernel<SS, R, TX, TY, EXACT>,
-                            cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cps, level_fused_kernel<SS, R, TX, TY, EXACT>,
-                                                     lv_threads<SS, R, TX, TY>(), G::SMEM));
-    if (cps < 1) cps = 1;
-    attr_set = true;
-  }
-  const int tiles_x = P.tiles_x[level];
-  const int tile0 = jr0 * tiles_x, tile1 = jr1 * tiles_x, n = tile1 - tile0;
-  const int grid = n < cps * d->num_sms ? n : cps * d->num_sms;             // persistent
-  // (accounted per pyramid level: every level runs its own template instantiation / tile shape)
-  { Launch l(d, level <= 1 ? KID_LEVEL_FUSED : level == 2 ? KID_LEVEL_FUSED_L2 : KID_LEVEL_FUSED_L3);
-    CU(launch_k(level_fused_kernel<SS, R, TX, TY, EXACT>, dim3(grid), dim3(lv_threads<SS, R, TX, TY>()), G::SMEM, d->stream, d->pdl != 0,
-                P.map[level], a.w, a.h, b.w, b.h, tiles_x, tile0, tile1, d->d_tile_ctr + (level & 15),
-                d->tile_base[level & 15], to_fused(tp), to_fused(tg), to_fused(td), b.img, b.gx, b.gy, b.pitch));
-    d->tile_base[level & 15] += (unsigned)(n + grid); }
-  return 0;
-}
+// level l >= 1, tile rows [jr0, jr1): chained (L_l -> gx_l, gy_l (+ L_{l+1} below the coarsest level))
+// or not (L_{l-1} -> L_l, gx_l, gy_l).  Accounted per pyramid level: every level runs its own
+// template instantiation / tile shape.
 template <bool EXACT>
-static int level_fused_launch(klt_dev* d, const FusedPlan& P, int level, const Level& a, const Level& b,
-                              const TapsR& tp, const TapsR& tg, const TapsR& td, int jr0, int jr1) {
+static int level_launch(klt_dev* d, const FusedPlan& P, const PyrSet& S, int level, int nb, const TapsR& tp,
+                        const TapsR& tg, const TapsR& td, int jr0, int jr1) {
   if (jr1 <= jr0) return 0;
-  switch (P.shape[level]) {
-    case SHAPE_2_5_64_32: return level_fused_launch_t<2, 5, 64, 32, EXACT>(d, P, level, a, b, tp, tg, td, jr0, jr1);
-    case SHAPE_2_5_64_24: return level_fused_launch_t<2, 5, 64, 24, EXACT>(d, P, level, a, b, tp, tg, td, jr0, jr1);
-    case SHAPE_2_5_64_16: return level_fused_launch_t<2, 5, 64, 16, EXACT>(d, P, level, a, b, tp, tg, td, jr0, jr1);
-    case SHAPE_2_5_32_16: return level_fused_launch_t<2, 5, 32, 16, EXACT>(d, P, level, a, b, tp, tg, td, jr0, jr1);
-    case SHAPE_4_10_32_16: return level_fused_launch_t<4, 10, 32, 16, EXACT>(d, P, level, a, b, tp, tg, td, jr0, jr1);
-    default: return fail(d, "level %d has no fused kernel", level);
-  }
-}
-
-// chained level l >= 1 (L_l -> gx_l, gy_l (+ L_{l+1} when nx)), tile rows [jr0, jr1)
-template <int TX, int TY, bool NX, bool EXACT>
-static int level_chain_launch_t(klt_dev* d, const FusedPlan& P, int level, const Level& a, const Level* nx,
-                                const TapsR& tp, const TapsR& tg, const TapsR& td, int jr0, int jr1) {
-  using G = ChGeo<TX, TY>;
-  static bool attr_dev[64] = {};                 // function attributes are per device
-  bool& attr_set = attr_dev[d->device & 63];
-  static int cps = 0;                                                       // resident CTAs per SM
-  if (!attr_set) {
-    CU(cudaFuncSetAttribute(level_chain_kernel<TX, TY, NX, EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cps, level_chain_kernel<TX, TY, NX, EXACT>, 256, G::SMEM));
-    if (cps < 1) cps = 1;
-    attr_set = true;
-  }
+  if (P.shape[level] == SHAPE_NONE) return fail(d, "level %d has no fused kernel", level);
+  const Level& a = S.lv[level - 1];
+  const Level& b = S.lv[level];
+  const Level* nx = P.chain && level + 1 < nb ? &S.lv[level + 1] : nullptr;
+  const int kid = level <= 1 ? KID_LEVEL_FUSED : level == 2 ? KID_LEVEL_FUSED_L2 : KID_LEVEL_FUSED_L3;
   const int tiles_x = P.tiles_x[level];
-  const int tile0 = jr0 * tiles_x, tile1 = jr1 * tiles_x, n = tile1 - tile0;
-  const int grid = n < cps * d->num_sms ? n : cps * d->num_sms;             // persistent
-  { Launch l(d, level <= 1 ? KID_LEVEL_FUSED : level == 2 ? KID_LEVEL_FUSED_L2 : KID_LEVEL_FUSED_L3);
-    CU(launch_k(level_chain_kernel<TX, TY, NX, EXACT>, dim3(grid), dim3(256), G::SMEM, d->stream, d->pdl != 0,
-                P.map[level], a.w, a.h, nx ? nx->w : 0, nx ? nx->h : 0, tiles_x, tile0, tile1,
-                d->d_tile_ctr + (level & 15), d->tile_base[level & 15], to_fused(tp), to_fused(tg), to_fused(td),
-                a.gx, a.gy, a.pitch, nx ? nx->img : nullptr, nx ? nx->pitch : 0));
-    d->tile_base[level & 15] += (unsigned)(n + grid); }
-  return 0;
-}
-template <int TX, int TY, bool EXACT>
-static int level_chain_launch_s(klt_dev* d, const FusedPlan& P, int level, const Level& a, const Level* nx,
-                                const TapsR& tp, const TapsR& tg, const TapsR& td, int jr0, int jr1) {
-  return nx ? level_chain_launch_t<TX, TY, true, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1)
-            : level_chain_launch_t<TX, TY, false, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
-}
-// nx: level l+1, null for the coarsest level
-template <bool EXACT>
-static int level_chain_launch(klt_dev* d, const FusedPlan& P, int level, const Level& a, const Level* nx,
-                              const TapsR& tp, const TapsR& tg, const TapsR& td, int jr0, int jr1) {
-  if (jr1 <= jr0) return 0;
-  switch (P.shape[level]) {
-    case SHAPE_2_5_64_32: return level_chain_launch_s<64, 32, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
-    case SHAPE_2_5_64_24: return level_chain_launch_s<64, 24, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
-    case SHAPE_2_5_64_16: return level_chain_launch_s<64, 16, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
-    case SHAPE_2_5_32_16: return level_chain_launch_s<32, 16, EXACT>(d, P, level, a, nx, tp, tg, td, jr0, jr1);
-    default: return fail(d, "level %d has no chained kernel", level);
-  }
+  return with_shape(P.shape[level], [&](auto s) {
+    using T = decltype(s);
+    constexpr int TX = T::TX, TY = T::TY;
+    if (!P.chain)
+      return launch_tiles<level_fused_kernel<T::SS, T::R, TX, TY, EXACT>>(
+          d, kid, level, lv_threads<T::SS, T::R, TX, TY>(), LvGeo<T::SS, T::R, TX, TY>::SMEM, tiles_x, jr0, jr1,
+          P.map[level], a.w, a.h, b.w, b.h, QUEUE, to_fused(tp), to_fused(tg), to_fused(td), b.img, b.gx, b.gy, b.pitch);
+    if (nx)
+      return launch_tiles<level_chain_kernel<TX, TY, true, EXACT>>(
+          d, kid, level, 256, ChGeo<TX, TY>::SMEM, tiles_x, jr0, jr1, P.map[level], b.w, b.h, nx->w, nx->h, QUEUE,
+          to_fused(tp), to_fused(tg), to_fused(td), b.gx, b.gy, b.pitch, nx->img, nx->pitch);
+    return launch_tiles<level_chain_kernel<TX, TY, false, EXACT>>(
+        d, kid, level, 256, ChGeo<TX, TY>::SMEM, tiles_x, jr0, jr1, P.map[level], b.w, b.h, 0, 0, QUEUE,
+        to_fused(tp), to_fused(tg), to_fused(td), b.gx, b.gy, b.pitch, nullptr, 0);
+  });
 }
 
 // generic two-kernel separable pass through d->tmp
@@ -2343,66 +2287,39 @@ static int build_impl(klt_dev* d, PyrSet& S, const unsigned char* src, int spitc
   FusedPlan P;
   d->last_fused = 0;
   d->last_bands = 0;
-  fused_plan(d, S, src, spitch, q, ts, tp, tg, td, &P, SHAPE_NONE);
+  fused_plan(d, S, src, spitch, q, ts, tp, tg, td, &P);
   bool all_fused = P.l0_ok;
   for (int l = 1; l < nb; ++l) all_fused = all_fused && P.shape[l] != SHAPE_NONE;
 
   if (all_fused) {
     // every level runs on the fused kernels: launch whole tile rows as soon as their source rows
     // exist -- all at once for a resident frame, band by band behind the upload of a host frame
-    int rows_done[KLT_DEV_MAX_LEVELS] = {0}, valid[KLT_DEV_MAX_LEVELS] = {0};
-    const int SS = P.SS, R = P.R, RG = FUSED_RG;
-    // u8 rows a level-0 tile row reads below its last output row
-    const int l0_reach = P.chain ? L0GeoC::U8_H - L0GeoC::TY - (L0GeoC::RS + L0GeoC::RG + L0GeoC::XR)
-                                 : L0Geo::RS + L0Geo::RG;
-    int u8_rows = feed ? 0 : H;
+    int rows_done[KLT_DEV_MAX_LEVELS] = {0};
+    int valid[KLT_DEV_MAX_LEVELS + 1] = {0};          // rows written so far of each plane of P's band schedule
+    auto plane_h = [&](int p) { return p == 0 ? H : S.lv[p - 1].h; };
+    valid[0] = feed ? 0 : H;
     if (feed && feed_enqueue_copies(d, feed)) return 1;
     do {
-      if (feed && feed_wait(d, feed, false, &u8_rows)) return 1;
-      int j = rows_done[0];
-      while (j < P.tiles_y[0]) {
-        int need = P.TY[0] * (j + 1) + l0_reach;
-        if (need > H) need = H;
-        if (need > u8_rows) break;
-        ++j;
-      }
-      if (l0_fused_launch<EXACT>(d, P, W, H, ts, tg, td, tp, S.lv[0], S.lv[nb > 1 ? 1 : 0], rows_done[0], j)) return 1;
-      rows_done[0] = j;
-      valid[0] = P.TY[0] * j < H ? P.TY[0] * j : H;
-      if (P.chain) {
-        // tile row j of level l makes rows TY_l/2 * j .. of L_{l+1} and reads L_l rows up to TY_l*(j+1)+4
-        valid[1] = P.TY[0] / 2 * rows_done[0] < S.lv[1].h ? P.TY[0] / 2 * rows_done[0] : S.lv[1].h;
-        for (int l = 1; l < nb; ++l) {
-          const Level& a = S.lv[l];
-          j = rows_done[l];
-          while (j < P.tiles_y[l]) {
-            int need = P.TY[l] * (j + 1) + NEXT_R;
-            if (need > a.h) need = a.h;
-            if (need > valid[l]) break;
-            ++j;
-          }
-          if (level_chain_launch<EXACT>(d, P, l, a, l + 1 < nb ? &S.lv[l + 1] : nullptr, tp, tg, td, rows_done[l], j))
-            return 1;
-          rows_done[l] = j;
-          if (l + 1 < nb) valid[l + 1] = P.TY[l] / 2 * j < S.lv[l + 1].h ? P.TY[l] / 2 * j : S.lv[l + 1].h;
-        }
-        continue;
-      }
-      for (int l = 1; l < nb; ++l) {
-        const Level& a = S.lv[l - 1];
-        const Level& b = S.lv[l];
-        j = rows_done[l];
+      if (feed && feed_wait(d, feed, false, &valid[0])) return 1;
+      for (int l = 0; l < nb; ++l) {
+        const int sp = P.src_plane[l];
+        int j = rows_done[l];
         while (j < P.tiles_y[l]) {
-          int need = SS * (P.TY[l] * (j + 1) - 1 + RG) + SS / 2 + R + 1;
-          if (need > a.h) need = a.h;
-          if (need > valid[l - 1]) break;
+          int need = P.need_mul[l] * (j + 1) + P.need_add[l];
+          if (need > plane_h(sp)) need = plane_h(sp);
+          if (need > valid[sp]) break;
           ++j;
         }
-        if (level_fused_launch<EXACT>(d, P, l, a, b, tp, tg, td, rows_done[l], j)) return 1;
+        if (l == 0 ? l0_fused_launch<EXACT>(d, P, W, H, ts, tg, td, tp, S, rows_done[0], j)
+                   : level_launch<EXACT>(d, P, S, l, nb, tp, tg, td, rows_done[l], j))
+          return 1;
         rows_done[l] = j;
-        valid[l] = P.TY[l] * j < b.h ? P.TY[l] * j : b.h;
+        if (l + 1 < nb) {
+          const int np = P.src_plane[l + 1];
+          valid[np] = P.made_mul[l] * j < plane_h(np) ? P.made_mul[l] * j : plane_h(np);
+        }
       }
-    } while (u8_rows < H);
+    } while (valid[0] < H);
     if (feed) {
       d->last_bands = feed->nbands;
       CU(cudaEventRecord(d->ev_frame_free[d->frame_idx], d->stream));
@@ -2424,7 +2341,7 @@ static int build_impl(klt_dev* d, PyrSet& S, const unsigned char* src, int spitc
   }
   int grad_from = 0;                 // first level whose gradients are still to be computed
   if (P.l0_ok) {
-    if (l0_fused_launch<EXACT>(d, P, W, H, ts, tg, td, tp, S.lv[0], S.lv[0], 0, P.tiles_y[0])) return 1;
+    if (l0_fused_launch<EXACT>(d, P, W, H, ts, tg, td, tp, S, 0, P.tiles_y[0])) return 1;
     grad_from = 1;
   }
   d->last_fused = grad_from;
@@ -2455,7 +2372,7 @@ static int build_impl(klt_dev* d, PyrSet& S, const unsigned char* src, int spitc
     const Level& a = S.lv[l - 1];
     const Level& b = S.lv[l];
     if (P.shape[l] != SHAPE_NONE) {
-      if (level_fused_launch<EXACT>(d, P, l, a, b, tp, tg, td, 0, P.tiles_y[l])) return 1;
+      if (level_launch<EXACT>(d, P, S, l, nb, tp, tg, td, 0, P.tiles_y[l])) return 1;
       grads_done[l] = true; d->last_fused += 1;
       continue;
     }

@@ -149,8 +149,76 @@ static constexpr int FUSED_RG = 3;       // gradient radius the fused kernels ar
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
-// barrier among the 256 threads that compute a tile (== __syncthreads() in the 256-thread kernels;
-// pyramid_mega_kernel carries a ninth, scheduling warp that must stay out of it)
+// ---- the persistent tile queue of the fused kernels -----------------------------------------------
+// Tiles are handed out dynamically: a launch covers the tiles [tile0, ntiles) (whole tile rows when
+// a frame is built band by band behind its upload); tile0 + counter[0] - base is the next tile
+// index.  Every CTA performs (tiles it processed + 1) atomicAdds, so after the launch the counter
+// stands at base + (ntiles - tile0) + gridDim.x, which the host uses as the next launch's base (no
+// reset needed).
+// (The kernels take it __grid_constant__, so that each field is read from the parameter bank where it
+// is used, like a scalar parameter.)
+struct TileQueue {
+  int tiles_x;                       // tile (x, y) is tile index y * tiles_x + x
+  int tile0, ntiles;
+  unsigned* counter;
+  unsigned base;
+};
+// One CTA's loop over the queue, tile origin (x0, y0) = (tile % tiles_x, tile / tiles_x) * (TX, TY),
+// b = border(x0, y0) (the tile meets a zero band or an image edge):
+//   front(x0, y0, b): the stages that consume the source box; barrier; claim of the next tile and the
+//                     TMA load of its box (box(x0, y0): the box's start coordinates) into box_dst;
+//   back(x0, y0, b):  the remaining stages; barrier.
+// The claim is made one tile ahead, so the next box's load latency hides behind the back stages.
+// sched: 16 B of shared memory (the mbarrier, then the next tile index).  WAIT_FIRST: griddepcontrol.wait
+// before the first claim (the kernel reads what its predecessor wrote); else in front of the first back
+// stage, i.e. after the first load and front stages.  Dependents are released when the queue is empty.
+template <int TX, int TY, bool WAIT_FIRST, class Border, class Box, class Front, class Back>
+__device__ __forceinline__ void tile_queue(const TileQueue& q, const CUtensorMap* map, void* box_dst,
+                                           unsigned box_bytes, unsigned char* sched, Border border, Box box,
+                                           Front front, Back back) {
+  unsigned long long* bar = reinterpret_cast<unsigned long long*>(sched);
+  volatile int* s_next = reinterpret_cast<volatile int*>(sched + 8);
+  const int tid = threadIdx.x, tiles_x = q.tiles_x;
+  auto claim = [&]() {
+    if (tid == 0) {
+      const int t = q.tile0 + (int)(atomicAdd(q.counter, 1u) - q.base);
+      *s_next = t;
+      if (t < q.ntiles) {
+        mbar_expect_tx(bar, box_bytes);
+        const int2 c = box((t % tiles_x) * TX, (t / tiles_x) * TY);
+        tma_load_2d(box_dst, map, c.x, c.y, bar);
+      }
+    }
+  };
+  if (tid == 0) {
+    mbar_init(bar, 1);
+    // descriptor fetch overlaps the predecessor's tail (we may be resident before it has finished)
+    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<unsigned long long>(map)) : "memory");
+  }
+  if (WAIT_FIRST) pdl_wait();
+  claim();
+  __syncthreads();
+  int tile = *s_next;
+  unsigned phase = 0;
+  bool waited = WAIT_FIRST;
+  while (tile < q.ntiles) {
+    const int x0 = (tile % tiles_x) * TX, y0 = (tile / tiles_x) * TY;
+    const bool b = border(x0, y0);
+    mbar_wait(bar, phase);
+    phase ^= 1;
+    front(x0, y0, b);
+    __syncthreads();                 // source box consumed; everybody has read s_next
+    claim();
+    if (!waited) { pdl_wait(); waited = true; }
+    back(x0, y0, b);
+    __syncthreads();                 // the back stages' buffers are free for the next tile
+    tile = *s_next;
+  }
+  if (!waited) pdl_wait();            // (a CTA that got no tile)
+  pdl_launch_dependents();            // queue empty: the next kernel of the chain may move in
+}
+
+// barrier among the NTH threads of a tile (== __syncthreads())
 template <int NTH = 256>
 __device__ __forceinline__ void tile_sync() { asm volatile("bar.sync 1, %0;" ::"n"(NTH) : "memory"); }
 
@@ -480,77 +548,36 @@ __device__ __forceinline__ void l0_fused_tile_rest(unsigned char* smem, int W, i
   if (G::NX) stage_vnext<EXACT, BORDER, G::TX, G::TY, G::N1_P>(sN1, tp, out_l1, l1pitch, x0, y0, H, W1, H1);
 }
 
-// Tiles are handed out dynamically: a launch covers the tiles [tile0, ntiles) (whole tile rows when
-// a frame is built band by band behind its upload); tile0 + counter[0] - base is the next tile
-// index.  Every CTA performs (tiles it processed + 1) atomicAdds, so after the launch the counter
-// stands at base + (ntiles - tile0) + gridDim.x, which the host uses as the next launch's base (no
-// reset needed).
-// The claim for the NEXT tile is made one tile ahead, so its TMA load can be issued early.
 template <class G, bool EXACT>
 __global__ void __launch_bounds__(256, G::CPS)
-l0_fused_kernel(const __grid_constant__ CUtensorMap map, int W, int H, int tiles_x, int tile0, int ntiles,
-                unsigned* __restrict__ counter, unsigned base,
+l0_fused_kernel(const __grid_constant__ CUtensorMap map, int W, int H, const __grid_constant__ TileQueue q,
                 TapsF ts, TapsF tg, TapsF td, float* __restrict__ out_img,
                 float* __restrict__ out_gx, float* __restrict__ out_gy, int opitch,
                 TapsF tp, float* __restrict__ out_l1, int l1pitch, int W1, int H1) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem_raw + G::OFF_BAR);
-  volatile int* s_next = reinterpret_cast<volatile int*>(smem_raw + G::OFF_BAR + 8);
-  const int tid = threadIdx.x;
-  if (tid == 0) {
-    mbar_init(bar, 1);
-    // descriptor fetch overlaps the predecessor's tail (we may be resident before it has finished)
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<unsigned long long>(&map)) : "memory");
-  }
+  // tiles whose 8-pixel margin stays inside the image never meet a zero band
+  auto border = [&](int x0, int y0) { return (x0 < 8) || (y0 < 8) || (x0 + G::TX + 8 > W) || (y0 + G::TY + 8 > H); };
   // Nothing this kernel READS comes from its predecessor in the stream (the u8 frame is resident, or
   // its upload is ordered by an event the launch itself waited for); only the pyramid slot it WRITES
   // may still be in use (the previous frame's tracker reads the other two slots and the feature
   // arrays).  So the first tile's load and horizontal pass run before griddepcontrol.wait -- under
   // the predecessor's tail -- and the wait sits in front of the first global store.
-  if (tid == 0) {
-    const int t = tile0 + (int)(atomicAdd(counter, 1u) - base);
-    *s_next = t;
-    if (t < ntiles) {
-      mbar_expect_tx(bar, G::U8_W * G::U8_H);
-      tma_load_2d(smem_raw + G::OFF_U8, &map, (t % tiles_x) * G::TX - 16,
-                  (t / tiles_x) * G::TY - (G::RS + G::RG + G::XR), bar);
-    }
-  }
-  __syncthreads();
-  int tile = *s_next;
-  unsigned phase = 0;
-  bool waited = false;
-  while (tile < ntiles) {
-    const int x0 = (tile % tiles_x) * G::TX, y0 = (tile / tiles_x) * G::TY;
-    // tiles whose 8-pixel margin stays inside the image never meet a zero band
-    const bool border = (x0 < 8) || (y0 < 8) || (x0 + G::TX + 8 > W) || (y0 + G::TY + 8 > H);
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    if (border) l0_fused_tile<G, EXACT, true>(smem_raw, W, ts, x0);
-    else l0_fused_tile<G, EXACT, false>(smem_raw, W, ts, x0);
-    __syncthreads();                 // u8 tile consumed; everybody has read s_next
-    if (tid == 0) {
-      const int t = tile0 + (int)(atomicAdd(counter, 1u) - base);
-      *s_next = t;
-      if (t < ntiles) {
-        mbar_expect_tx(bar, G::U8_W * G::U8_H);
-        tma_load_2d(smem_raw + G::OFF_U8, &map, (t % tiles_x) * G::TX - 16,
-                    (t / tiles_x) * G::TY - (G::RS + G::RG + G::XR), bar);
-      }
-    }
-    if (!waited) { pdl_wait(); waited = true; }
-    if (border)
-      l0_fused_tile_rest<G, EXACT, true>(smem_raw, W, H, ts, tg, td, tp, out_img, out_gx, out_gy, opitch, out_l1, l1pitch,
-                                         W1, H1, x0, y0);
-    else
-      l0_fused_tile_rest<G, EXACT, false>(smem_raw, W, H, ts, tg, td, tp, out_img, out_gx, out_gy, opitch, out_l1, l1pitch,
-                                          W1, H1, x0, y0);
-    // stage D reads Hd (aliased on Hs) and Hg: the next tile's stage A must not start before
-    __syncthreads();
-    tile = *s_next;
-  }
-  if (!waited) pdl_wait();            // (a CTA that got no tile)
-  pdl_launch_dependents();            // queue empty: the next kernel of the chain may move in
+  tile_queue<G::TX, G::TY, false>(
+      q, &map, smem_raw + G::OFF_U8, G::U8_W * G::U8_H, smem_raw + G::OFF_BAR, border,
+      [&](int x0, int y0) { return make_int2(x0 - 16, y0 - (G::RS + G::RG + G::XR)); },
+      [&](int x0, int y0, bool border) {
+        if (border) l0_fused_tile<G, EXACT, true>(smem_raw, W, ts, x0);
+        else l0_fused_tile<G, EXACT, false>(smem_raw, W, ts, x0);
+      },
+      // (stage D reads Hd, aliased on Hs, and Hg: the barrier after it keeps the next stage A out)
+      [&](int x0, int y0, bool border) {
+        if (border)
+          l0_fused_tile_rest<G, EXACT, true>(smem_raw, W, H, ts, tg, td, tp, out_img, out_gx, out_gy, opitch, out_l1,
+                                             l1pitch, W1, H1, x0, y0);
+        else
+          l0_fused_tile_rest<G, EXACT, false>(smem_raw, W, H, ts, tg, td, tp, out_img, out_gx, out_gy, opitch, out_l1,
+                                              l1pitch, W1, H1, x0, y0);
+      });
 }
 
 // ============================================================================================
@@ -698,7 +725,6 @@ __device__ __forceinline__ void lv_stage_rest(unsigned char* smem, const TapsF& 
 }
 
 // W,H: size of the level being produced; Wsrc,Hsrc: size of the level it is made from.
-// Dynamic tile scheduler as in l0_fused_kernel.
 // NTH threads per CTA: 256, or 512 for the big-tile shapes whose shared-memory footprint allows only two
 // CTAs per SM (16 warps per SM leave the tile's four-stage chain latency bound; 32 do not).
 template <int SS, int R, int TX, int TY>
@@ -706,59 +732,28 @@ __host__ __device__ constexpr int lv_threads() { return (LvGeo<SS, R, TX, TY>::S
 template <int SS, int R, int TX, int TY, bool EXACT>
 __global__ void __launch_bounds__((lv_threads<SS, R, TX, TY>()), (LvGeo<SS, R, TX, TY>::SMEM <= 75 * 1024) ? 3 : 2)
 level_fused_kernel(const __grid_constant__ CUtensorMap map, int Wsrc, int Hsrc, int W, int H,
-                   int tiles_x, int tile0, int ntiles, unsigned* __restrict__ counter, unsigned base,
-                   TapsF tp, TapsF tg, TapsF td,
+                   const __grid_constant__ TileQueue q, TapsF tp, TapsF tg, TapsF td,
                    float* __restrict__ out_img, float* __restrict__ out_gx,
                    float* __restrict__ out_gy, int opitch) {
   using G = LvGeo<SS, R, TX, TY>;
   constexpr int NTH = lv_threads<SS, R, TX, TY>();
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem_raw + G::OFF_BAR);
-  volatile int* s_next = reinterpret_cast<volatile int*>(smem_raw + G::OFF_BAR + 8);
-  const int tid = threadIdx.x;
-  if (tid == 0) {
-    mbar_init(bar, 1);
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<unsigned long long>(&map)) : "memory");
-  }
-  pdl_wait();                         // the source level is written by the previous kernel
-  if (tid == 0) {
-    const int t = tile0 + (int)(atomicAdd(counter, 1u) - base);
-    *s_next = t;
-    if (t < ntiles) {
-      mbar_expect_tx(bar, G::SW * G::SH * 4);
-      tma_load_2d(smem_raw + G::OFF_SRC, &map, SS * (t % tiles_x) * TX + G::XOFF,
-                  SS * (t / tiles_x) * TY + G::YOFF, bar);
-    }
-  }
-  __syncthreads();
-  int tile = *s_next;
-  unsigned phase = 0;
-  while (tile < ntiles) {
-    const int x0 = (tile % tiles_x) * TX, y0 = (tile / tiles_x) * TY;
-    // interior tiles (margins derived in DESIGN.md) never meet a zero band at either level
-    const bool border = (x0 < 8) || (y0 < 8) || (x0 + TX + 16 > W) || (y0 + TY + 16 > H);
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    if (border) lv_stage_p1<EXACT, true, SS, R, TX, TY, NTH>(smem_raw, tp, x0, Wsrc);
-    else lv_stage_p1<EXACT, false, SS, R, TX, TY, NTH>(smem_raw, tp, x0, Wsrc);
-    __syncthreads();                 // source box consumed; everybody has read s_next
-    if (tid == 0) {
-      const int t = tile0 + (int)(atomicAdd(counter, 1u) - base);
-      *s_next = t;
-      if (t < ntiles) {
-        mbar_expect_tx(bar, G::SW * G::SH * 4);
-        tma_load_2d(smem_raw + G::OFF_SRC, &map, SS * (t % tiles_x) * TX + G::XOFF,
-                    SS * (t / tiles_x) * TY + G::YOFF, bar);
-      }
-    }
-    if (border)
-      lv_stage_rest<EXACT, true, SS, R, TX, TY, NTH>(smem_raw, tp, tg, td, Hsrc, W, H, out_img, out_gx, out_gy, opitch, x0, y0);
-    else
-      lv_stage_rest<EXACT, false, SS, R, TX, TY, NTH>(smem_raw, tp, tg, td, Hsrc, W, H, out_img, out_gx, out_gy, opitch, x0, y0);
-    __syncthreads();                 // Hp / L / Hd / Hg free for the next tile
-    tile = *s_next;
-  }
-  pdl_launch_dependents();            // queue empty: the next kernel of the chain may move in
+  // interior tiles (margins derived in DESIGN.md) never meet a zero band at either level
+  auto border = [&](int x0, int y0) { return (x0 < 8) || (y0 < 8) || (x0 + TX + 16 > W) || (y0 + TY + 16 > H); };
+  // (waits before its first claim: the source level is written by the previous kernel)
+  tile_queue<TX, TY, true>(
+      q, &map, smem_raw + G::OFF_SRC, G::SW * G::SH * 4, smem_raw + G::OFF_BAR, border,
+      [&](int x0, int y0) { return make_int2(SS * x0 + G::XOFF, SS * y0 + G::YOFF); },
+      [&](int x0, int y0, bool border) {
+        if (border) lv_stage_p1<EXACT, true, SS, R, TX, TY, NTH>(smem_raw, tp, x0, Wsrc);
+        else lv_stage_p1<EXACT, false, SS, R, TX, TY, NTH>(smem_raw, tp, x0, Wsrc);
+      },
+      [&](int x0, int y0, bool border) {
+        if (border)
+          lv_stage_rest<EXACT, true, SS, R, TX, TY, NTH>(smem_raw, tp, tg, td, Hsrc, W, H, out_img, out_gx, out_gy, opitch, x0, y0);
+        else
+          lv_stage_rest<EXACT, false, SS, R, TX, TY, NTH>(smem_raw, tp, tg, td, Hsrc, W, H, out_img, out_gx, out_gy, opitch, x0, y0);
+      });
 }
 
 // ============================================================================================
@@ -785,73 +780,43 @@ struct ChGeo {
   static constexpr int SMEM = OFF_BAR + 16;
 };
 
-// W,H: size of level l; Wn,Hn: size of level l+1 (unused without NX).  Dynamic tile scheduler and
-// programmatic dependent launch as in level_fused_kernel.
+// W,H: size of level l; Wn,Hn: size of level l+1 (unused without NX).
 template <int TX, int TY, bool NX, bool EXACT>
 __global__ void __launch_bounds__(256, 4)
 level_chain_kernel(const __grid_constant__ CUtensorMap map, int W, int H, int Wn, int Hn,
-                   int tiles_x, int tile0, int ntiles, unsigned* __restrict__ counter, unsigned base,
-                   TapsF tp, TapsF tg, TapsF td, float* __restrict__ out_gx, float* __restrict__ out_gy,
-                   int opitch, float* __restrict__ out_next, int npitch) {
+                   const __grid_constant__ TileQueue q, TapsF tp, TapsF tg, TapsF td, float* __restrict__ out_gx,
+                   float* __restrict__ out_gy, int opitch, float* __restrict__ out_next, int npitch) {
   using G = ChGeo<TX, TY>;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem_raw + G::OFF_BAR);
-  volatile int* s_next = reinterpret_cast<volatile int*>(smem_raw + G::OFF_BAR + 8);
   const float* sL = reinterpret_cast<const float*>(smem_raw + G::OFF_SRC);
+  const float* sLg = sL + (G::RN - 1 - G::RG) * G::SW;
   float* sHd = reinterpret_cast<float*>(smem_raw + G::OFF_HD);
   float* sHg = reinterpret_cast<float*>(smem_raw + G::OFF_HG);
   float* sN = reinterpret_cast<float*>(smem_raw + G::OFF_N);
-  const int tid = threadIdx.x;
-  if (tid == 0) {
-    mbar_init(bar, 1);
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<unsigned long long>(&map)) : "memory");
-  }
-  pdl_wait();                         // L_l is written by the previous kernel
-  if (tid == 0) {
-    const int t = tile0 + (int)(atomicAdd(counter, 1u) - base);
-    *s_next = t;
-    if (t < ntiles) {
-      mbar_expect_tx(bar, G::SW * G::SH * 4);
-      tma_load_2d(smem_raw + G::OFF_SRC, &map, (t % tiles_x) * TX - 4, (t / tiles_x) * TY + 1 - G::RN, bar);
-    }
-  }
-  __syncthreads();
-  int tile = *s_next;
-  unsigned phase = 0;
   // output rows per thread of stage 2: as few as the thread count allows (fewer rows = more items)
   constexpr int PY = (TX / 4) * (TY / 2) <= 128 ? 2 : ((TX / 4) * (TY / 4) <= 128 ? 4 : 8);
-  while (tile < ntiles) {
-    const int x0 = (tile % tiles_x) * TX, y0 = (tile / tiles_x) * TY;
-    // tiles whose 8-pixel margin stays inside level l meet no zero band of either pass and no edge
-    const bool border = (x0 < 8) || (y0 < 8) || (x0 + TX + 8 > W) || (y0 + TY + 8 > H);
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    const float* sLg = sL + (G::RN - 1 - G::RG) * G::SW;
-    if (border) {
-      stage_hgrad<EXACT, true, TX, G::GH, G::SW, G::HP>(sLg, sHd, sHg, tg, td, x0, W);
-      if (NX) stage_hnext<EXACT, true, TX, G::SH, G::SW, G::NP>(sL, sN, tp, x0, W);
-    } else {
-      stage_hgrad<EXACT, false, TX, G::GH, G::SW, G::HP>(sLg, sHd, sHg, tg, td, x0, W);
-      if (NX) stage_hnext<EXACT, false, TX, G::SH, G::SW, G::NP>(sL, sN, tp, x0, W);
-    }
-    __syncthreads();                 // source box consumed; everybody has read s_next
-    if (tid == 0) {
-      const int t = tile0 + (int)(atomicAdd(counter, 1u) - base);
-      *s_next = t;
-      if (t < ntiles) {
-        mbar_expect_tx(bar, G::SW * G::SH * 4);
-        tma_load_2d(smem_raw + G::OFF_SRC, &map, (t % tiles_x) * TX - 4, (t / tiles_x) * TY + 1 - G::RN, bar);
-      }
-    }
-    if (border) {
-      stage_vgrad_both<EXACT, true, TX, TY, PY, G::HP>(sHd, sHg, tg, td, out_gx, out_gy, opitch, x0, y0, W, H);
-      if (NX) stage_vnext<EXACT, true, TX, TY, G::NP>(sN, tp, out_next, npitch, x0, y0, H, Wn, Hn);
-    } else {
-      stage_vgrad_both<EXACT, false, TX, TY, PY, G::HP>(sHd, sHg, tg, td, out_gx, out_gy, opitch, x0, y0, W, H);
-      if (NX) stage_vnext<EXACT, false, TX, TY, G::NP>(sN, tp, out_next, npitch, x0, y0, H, Wn, Hn);
-    }
-    __syncthreads();                 // Hd / Hg / next-level buffer free for the next tile
-    tile = *s_next;
-  }
-  pdl_launch_dependents();            // queue empty: the next kernel of the chain may move in
+  // tiles whose 8-pixel margin stays inside level l meet no zero band of either pass and no edge
+  auto border = [&](int x0, int y0) { return (x0 < 8) || (y0 < 8) || (x0 + TX + 8 > W) || (y0 + TY + 8 > H); };
+  // (waits before its first claim: L_l is written by the previous kernel)
+  tile_queue<TX, TY, true>(
+      q, &map, smem_raw + G::OFF_SRC, G::SW * G::SH * 4, smem_raw + G::OFF_BAR, border,
+      [&](int x0, int y0) { return make_int2(x0 - 4, y0 + 1 - G::RN); },
+      [&](int x0, int y0, bool border) {
+        if (border) {
+          stage_hgrad<EXACT, true, TX, G::GH, G::SW, G::HP>(sLg, sHd, sHg, tg, td, x0, W);
+          if (NX) stage_hnext<EXACT, true, TX, G::SH, G::SW, G::NP>(sL, sN, tp, x0, W);
+        } else {
+          stage_hgrad<EXACT, false, TX, G::GH, G::SW, G::HP>(sLg, sHd, sHg, tg, td, x0, W);
+          if (NX) stage_hnext<EXACT, false, TX, G::SH, G::SW, G::NP>(sL, sN, tp, x0, W);
+        }
+      },
+      [&](int x0, int y0, bool border) {
+        if (border) {
+          stage_vgrad_both<EXACT, true, TX, TY, PY, G::HP>(sHd, sHg, tg, td, out_gx, out_gy, opitch, x0, y0, W, H);
+          if (NX) stage_vnext<EXACT, true, TX, TY, G::NP>(sN, tp, out_next, npitch, x0, y0, H, Wn, Hn);
+        } else {
+          stage_vgrad_both<EXACT, false, TX, TY, PY, G::HP>(sHd, sHg, tg, td, out_gx, out_gy, opitch, x0, y0, W, H);
+          if (NX) stage_vnext<EXACT, false, TX, TY, G::NP>(sN, tp, out_next, npitch, x0, y0, H, Wn, Hn);
+        }
+      });
 }
