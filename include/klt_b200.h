@@ -47,6 +47,39 @@ float KLTB200GetForwardBackward(KLT_TrackingContext tc);
 void KLTB200ForwardBackwardResult(KLT_TrackingContext tc, int n, float *xb, float *yb, float *err,
                                   int *back_val);
 
+/* Motion prior of every tracking call on tc (the calls above).  A feature with a guess g of its position
+ * in frame 2 starts its pyramid descent from g instead of from zero motion, so that it can be found
+ * farther away than the pyramid alone reaches; everything else, the status codes included, is the
+ * reference's loop, and a guess equal to the feature's position changes nothing.  A guess whose window
+ * leaves a level loses the feature as KLT_OOB.  Guesses come from:
+ *   KLT_B200_PREDICT_VELOCITY: the feature's last displacement, for a feature whose val is KLT_TRACKED
+ *     and which still sits where the last tracking call on tc left it (so not for features that were
+ *     just selected or replaced, or that the caller moved).  The displacement is recorded after the
+ *     forward-backward check and before the affine check by every call that runs with the prior
+ *     (velocity mode, or explicit guesses in any mode), and forgotten by a call with neither and by
+ *     a change of frame size.
+ *   KLTB200SetGuesses: explicit guesses for the next KLTTrackFeatures, KLTTrackFeaturesDevice or
+ *     KLTB200ResidentStep on tc, one per feature (NaN: none for that feature); they take precedence
+ *     over the velocity.  That call ends in KLTError unless it has n features, and so does
+ *     KLTTrackFeaturesSequence while guesses are set (through this call or klt_dev_set_guesses: they
+ *     share one queue).  gx, gy are host arrays, or device arrays when on_device != 0; a device
+ *     array must be complete when this is called.  Guesses for the next KLTB200ResidentStep may be
+ *     set before the previous step has run; a third set waits until the device has finished the
+ *     step that read the first.
+ * With the forward-backward check, the backward leg of a feature that used g starts from the mirrored
+ * prior xout - (g - x0).  Default mode: environment variable KLT_B200_PREDICT (none | velocity) when
+ * tc's state is created, else none; any other value ends in KLTError. */
+#define KLT_B200_PREDICT_NONE      0
+#define KLT_B200_PREDICT_VELOCITY  1
+void KLTB200SetPrediction(KLT_TrackingContext tc, int mode);
+int  KLTB200GetPrediction(KLT_TrackingContext tc);
+void KLTB200SetGuesses(KLT_TrackingContext tc, int n, const float *gx, const float *gy, int on_device);
+/* Per feature of the last tracking call on tc (the last frame of a sequence or resident step), into the
+ * non-NULL arrays: the guess it started from and its source (0 none, 1 velocity, 2 explicit);
+ * gx = gy = -1 without one.  Synchronises.  KLTError when that call ran without prediction or had a
+ * number of features other than n. */
+void KLTB200PredictionResult(KLT_TrackingContext tc, int n, float *gx, float *gy, int *source);
+
 /* the device context behind tc (created on demand) */
 klt_dev *KLTB200Device(KLT_TrackingContext tc);
 /* slot (0/1) holding tc's previous-frame pyramids, -1 if none */

@@ -73,6 +73,7 @@ typedef struct {
                                   (reference src/V1/trackFeatures.c:125-220, :433-437, :466-468) */
   float fb_max_error;          /* > 0: forward-backward check in the same launch (klt_dev_fb_results);
                                   0: off */
+  int   predict;               /* motion prior: 0 none, 1 constant velocity (klt_dev_prediction_results) */
 } klt_dev_track_params;
 
 /* replaces the scalar arguments of _KLTSelectGoodFeatures /
@@ -137,6 +138,28 @@ int klt_dev_features_download(klt_dev *d, int n, float *x, float *y, int *val); 
  * back_val = 1 for a feature the check did not run on.  Fails unless that call ran the check on
  * exactly n features.  Synchronises. */
 int klt_dev_fb_results(klt_dev *d, int n, float *xb, float *yb, float *err, int *back_val);
+/* Motion prior: a feature with a guess g of its frame-2 position starts its pyramid descent from g
+ * (scaled through the levels as its own position is) instead of from zero motion; everything else is
+ * the reference loop.  A feature uses, in this order, its explicit guess (klt_dev_set_guesses; both
+ * coordinates finite, NaN = none), or with predict = 1 its constant-velocity guess x0 + (dx, dy): the
+ * device keeps one record {px, py, dx, dy} per feature index, written by every call with the prior
+ * as {xout, yout, xout - x0, yout - y0} for a feature that ends KLT_TRACKED (after the
+ * forward-backward check, before the affine check) and invalid for every other one; a feature uses
+ * it when its input val is KLT_TRACKED and it still starts at (px, py).  Records are invalid when
+ * allocated, after a call without the prior and after a change of frame geometry.  With the
+ * forward-backward check, the backward leg of a feature that used g starts from xout - (g - x0).
+ * klt_dev_set_guesses queues n guesses for the next klt_dev_track* call, which consumes them and
+ * fails unless it has n features: host arrays are staged and copied H2D, device arrays (on_device != 0)
+ * D2D on the library's copy stream, so they must be complete when this is called.  Two sets of
+ * guesses can be in flight: queuing a third waits until the tracking call that read the first has
+ * finished on the device, so a pipelined driver may queue guesses for step k + 1 before step k ran.
+ * klt_dev_prediction_results copies the per-feature records of the last klt_dev_track* call into the
+ * non-NULL arrays: the guess (gx, gy) and its source (0 none, 1 velocity, 2 explicit); -1, -1, 0
+ * without a guess.  Fails unless that call ran with prediction on exactly n features.  Synchronises. */
+int klt_dev_set_guesses(klt_dev *d, int n, const float *gx, const float *gy, int on_device);
+/* the number of guesses queued for the next klt_dev_track* call, -1 when none are */
+int klt_dev_guesses_pending(const klt_dev *d);
+int klt_dev_prediction_results(klt_dev *d, int n, float *gx, float *gy, int *source);
 /* Ring of pinned snapshots of the resident features for pipelined drivers
  * (KLTTrackFeaturesSequence): klt_dev_snapshot_ring sizes it (depth <= 64 slots),
  * klt_dev_snapshot_push queues a copy of the current x | y | val into a slot behind the work

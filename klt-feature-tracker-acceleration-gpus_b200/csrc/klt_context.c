@@ -63,6 +63,13 @@ klt_tc_state *klt_state_get(KLT_TrackingContext tc)
     free(s);
     KLTError("(KLT/B200) KLT_B200_FB_MAX_ERROR = %s is not a number of pixels", e);
   }
+  e = getenv("KLT_B200_PREDICT");
+  s->predict = KLT_B200_PREDICT_NONE;
+  if (e && strcmp(e, "velocity") == 0) s->predict = KLT_B200_PREDICT_VELOCITY;
+  else if (e && strcmp(e, "none") != 0) {
+    free(s);
+    KLTError("(KLT/B200) KLT_B200_PREDICT = %s (must be none or velocity)", e);
+  }
   pthread_mutex_lock(&g_lock);
   s->next = g_states;
   g_states = s;
@@ -142,6 +149,32 @@ void KLTB200ForwardBackwardResult(KLT_TrackingContext tc, int n, float *xb, floa
     KLTError("(KLTB200ForwardBackwardResult) no tracking call on this context ran the check");
   if (klt_dev_fb_results(s->dev, n, xb, yb, err, back_val) != 0)
     KLTError("(KLTB200ForwardBackwardResult) %s", klt_dev_error(s->dev));
+}
+
+/* a setting of the tracker's launch only, like the forward-backward check */
+void KLTB200SetPrediction(KLT_TrackingContext tc, int mode)
+{
+  if (mode != KLT_B200_PREDICT_NONE && mode != KLT_B200_PREDICT_VELOCITY)
+    KLTError("(KLTB200SetPrediction) mode %d (must be KLT_B200_PREDICT_NONE or KLT_B200_PREDICT_VELOCITY)", mode);
+  klt_state_get(tc)->predict = mode;
+}
+
+int KLTB200GetPrediction(KLT_TrackingContext tc) { return klt_state_get(tc)->predict; }
+
+void KLTB200SetGuesses(KLT_TrackingContext tc, int n, const float *gx, const float *gy, int on_device)
+{
+  klt_tc_state *s = klt_state_get(tc);
+  if (klt_dev_set_guesses(klt_state_device(s), n, gx, gy, on_device) != 0)
+    KLTError("(KLTB200SetGuesses) %s", klt_dev_error(s->dev));
+}
+
+void KLTB200PredictionResult(KLT_TrackingContext tc, int n, float *gx, float *gy, int *source)
+{
+  klt_tc_state *s = klt_state_find(tc);
+  if (s == NULL || s->dev == NULL)
+    KLTError("(KLTB200PredictionResult) no tracking call on this context ran with prediction");
+  if (klt_dev_prediction_results(s->dev, n, gx, gy, source) != 0)
+    KLTError("(KLTB200PredictionResult) %s", klt_dev_error(s->dev));
 }
 klt_dev *KLTB200Device(KLT_TrackingContext tc) { return klt_state_device(klt_state_get(tc)); }
 int KLTB200LastSlot(KLT_TrackingContext tc)

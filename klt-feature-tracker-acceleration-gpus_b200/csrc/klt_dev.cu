@@ -855,6 +855,86 @@ __device__ __forceinline__ FbRec fb_unchecked() {
   return r;
 }
 
+// Motion prior: a per-feature guess g of the frame-2 position, where the descent starts instead of
+// at the feature's own position.  Velocity record of a feature index, written by every tracker that
+// runs with the prior: {xout, yout, xout - x0, yout - y0} for a KLT_TRACKED result (after the
+// forward-backward check), px = NaN (invalid) for any other.
+struct __align__(16) PredVel { float px, py, dx, dy; };
+// Per feature of the last call (klt_dev_prediction_results): the guess and where it came from
+// (PRED_NONE: (-1, -1)).
+enum { PRED_NONE = 0, PRED_VELOCITY = 1, PRED_EXPLICIT = 2 };
+struct PredRec { float gx, gy; int source; };
+// The prior's kernel argument, after FbArgs (so that the PRED = false kernels keep their layout):
+// explicit guesses of this call (NaN: none for that feature; gx == nullptr: none at all), the velocity
+// records (read for f < vel_n; vel_n = 0 when velocity prediction is off or no record is valid) and
+// the result records.
+struct PredArgs { const float* gx; const float* gy; PredVel* vel; PredRec* rec; int vel_n; };
+
+// The start of feature f's forward leg (input position (x0, y0), input status val_in) at the coarsest
+// level: {x0, y0, gx, gy}, the guess g being (x0, y0) without one.  Records the guess in rec[f].  Run
+// by one lane of the feature's group before the descent.  Out of line and with scalar arguments: the
+// division's slow path is a call, and inlined, the values live across those calls make the PRED
+// kernels spill; across this one call only what the FB kernels keep across theirs is live.
+__device__ __noinline__ float4 pred_start(const float* egx, const float* egy, const PredVel* vel, PredRec* rec,
+                                          int vel_n, int nlevels, float ss, int f, int val_in, float x0, float y0) {
+  int src = PRED_NONE;
+  float gx = x0, gy = y0;
+  if (egx && isfinite(egx[f]) && isfinite(egy[f])) {
+    gx = egx[f]; gy = egy[f]; src = PRED_EXPLICIT;
+  } else if (val_in == KLT_TRACKED && f < vel_n) {
+    const PredVel v = vel[f];
+    if (x0 == v.px && y0 == v.py) { gx = __fadd_rn(x0, v.dx); gy = __fadd_rn(y0, v.dy); src = PRED_VELOCITY; }
+  }
+  PredRec r;
+  r.gx = src ? gx : -1.0f; r.gy = src ? gy : -1.0f; r.source = src;
+  rec[f] = r;
+  float4 c = make_float4(x0, y0, gx, gy);
+  for (int l = nlevels - 1; l >= 0; --l) {        // divided by ss once per level, as the descent divides the start
+    c.x = __fdiv_rn(c.x, ss); c.y = __fdiv_rn(c.y, ss); c.z = __fdiv_rn(c.z, ss); c.w = __fdiv_rn(c.w, ss);
+  }
+  return c;
+}
+// The start of the backward leg from (xout, yout) at the coarsest level: {xout, yout, gbx, gby}, with the
+// mirrored prior gb = xout - (g - x0) when the forward leg used a guess g (read back from rec[f]), else
+// gb = xout.
+__device__ __noinline__ float4 pred_back_start(const PredRec* rec, int nlevels, float ss, int f, float x0, float y0,
+                                               float xout, float yout) {
+  const PredRec r = rec[f];
+  float4 c = make_float4(xout, yout, xout, yout);
+  if (r.source != PRED_NONE) { c.z = __fsub_rn(xout, __fsub_rn(r.gx, x0)); c.w = __fsub_rn(yout, __fsub_rn(r.gy, y0)); }
+  for (int l = nlevels - 1; l >= 0; --l) {
+    c.x = __fdiv_rn(c.x, ss); c.y = __fdiv_rn(c.y, ss); c.z = __fdiv_rn(c.z, ss); c.w = __fdiv_rn(c.w, ss);
+  }
+  return c;
+}
+__device__ __forceinline__ float4 shfl4(float4 c, int width) {
+  c.x = __shfl_sync(0xffffffffu, c.x, 0, width); c.y = __shfl_sync(0xffffffffu, c.y, 0, width);
+  c.z = __shfl_sync(0xffffffffu, c.z, 0, width); c.w = __shfl_sync(0xffffffffu, c.w, 0, width);
+  return c;
+}
+// Velocity record of feature f after its call, from its result v before the affine check.  (x0, y0)
+// is read again from the input rather than kept in registers across the descent.
+__device__ __forceinline__ void pred_velocity(const PredArgs& pr, const FeatIO& io, int f, int v,
+                                              float xout, float yout) {
+  PredVel w;
+  if (v == KLT_TRACKED) {
+    w.px = xout; w.py = yout;
+    w.dx = __fsub_rn(xout, io.x[(size_t)f * io.istride]); w.dy = __fsub_rn(yout, io.y[(size_t)f * io.istride]);
+  } else {
+    w.px = __int_as_float(0x7fffffff); w.py = w.px; w.dx = 0.0f; w.dy = 0.0f;
+  }
+  pr.vel[f] = w;
+}
+// a feature the tracker does not run on: no guess, no velocity
+__device__ __forceinline__ void pred_skip(const PredArgs& pr, int f) {
+  PredRec r;
+  r.gx = -1.0f; r.gy = -1.0f; r.source = PRED_NONE;
+  pr.rec[f] = r;
+  PredVel w;
+  w.px = __int_as_float(0x7fffffff); w.py = w.px; w.dx = 0.0f; w.dy = 0.0f;
+  pr.vel[f] = w;
+}
+
 // bilinear weights of _interpolate (trackFeatures.c:31-57): the four products
 // (1-ax)(1-ay), ax(1-ay), (1-ax)ay, ax*ay are rounded first, then multiplied by
 // the pixels and summed left to right.
@@ -949,15 +1029,19 @@ __device__ __forceinline__ LiGain li_gain(const float (&g1)[PPL], const float (&
 // level and kept in registers.
 // The pyramid descent of one feature from (x, y) in p1's frame into p2's frame (:1343-1378): the
 // status of the finest level reached and the end position (xend, yend), before the border test.
-template <bool EXACT, int PPL>
+// G: (x, y) and the guess (gx, gy) the descent starts from are given at the coarsest level (pred_start);
+// a guess equal to the start gives the descent without one.
+template <bool EXACT, int PPL, bool G = false>
 __device__ __forceinline__ int track_descent(const PyrView& p1, const PyrView& p2, const TrackArgs& a, int lane,
                                              const float (&offi)[PPL], const float (&offj)[PPL],
                                              float* swx, float* swy, float* swd,
-                                             float x, float y, float& xend, float& yend) {
+                                             float x, float y, float& xend, float& yend,
+                                             float gx = 0.0f, float gy = 0.0f) {
   const int ww = a.ww, wh = a.wh, hw = ww / 2, hh = wh / 2, npix = ww * wh;
   float xloc = x, yloc = y;
-  for (int r = a.nlevels - 1; r >= 0; --r) { xloc = __fdiv_rn(xloc, a.ss); yloc = __fdiv_rn(yloc, a.ss); }
-  float xout = xloc, yout = yloc;
+  if (!G)
+    for (int r = a.nlevels - 1; r >= 0; --r) { xloc = __fdiv_rn(xloc, a.ss); yloc = __fdiv_rn(yloc, a.ss); }
+  float xout = G ? gx : xloc, yout = G ? gy : yloc;
   int status = KLT_TRACKED;
 
   for (int r = a.nlevels - 1; r >= 0; --r) {
@@ -1151,17 +1235,20 @@ __device__ __forceinline__ int track_descent(const PyrView& p1, const PyrView& p
 }
 
 // FB: the forward-backward check runs in the same warp after the forward leg (klt_dev_fb_results)
-template <bool EXACT, int PPL, bool FB>
+// PRED: the descent starts from the feature's guess (PredArgs, klt_dev_prediction_results)
+template <bool EXACT, int PPL, bool FB, bool PRED = false>
 __global__ void __launch_bounds__(128)
 track_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
-             unsigned long long* __restrict__ live_total, FbArgs fb) {
+             unsigned long long* __restrict__ live_total, FbArgs fb, PredArgs pr) {
   extern __shared__ float s_win[];     // EXACT only: [warps][3][npix]
   const int lane = threadIdx.x & 31;
   const int wib = threadIdx.x >> 5;
   const int f = blockIdx.x * (blockDim.x >> 5) + wib;
   if (f >= n) return;
-  if (io.val[(size_t)f * io.istride] < 0) {                   // only features that are not lost (:1346)
+  const int val_in = io.val[(size_t)f * io.istride];
+  if (val_in < 0) {                                           // only features that are not lost (:1346)
     if (FB && lane == 0) fb.rec[f] = fb_unchecked();
+    if (PRED && lane == 0) pred_skip(pr, f);
     return;
   }
   if (lane == 0) atomicAdd(live_total, 1ULL);
@@ -1182,19 +1269,30 @@ track_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
   }
 
   const float x0 = io.x[(size_t)f * io.istride], y0 = io.y[(size_t)f * io.istride];
+  float4 s0 = make_float4(x0, y0, 0.0f, 0.0f);              // PRED: start and guess at the coarsest level
+  if (PRED) {
+    if (lane == 0) s0 = pred_start(pr.gx, pr.gy, pr.vel, pr.rec, pr.vel_n, a.nlevels, a.ss, f, val_in, x0, y0);
+    s0 = shfl4(s0, 32);
+  }
   float xout, yout;
-  int v = track_outcome(a, track_descent<EXACT, PPL>(p1, p2, a, lane, offi, offj, swx, swy, swd, x0, y0, xout, yout),
-                        xout, yout);
+  int v = track_outcome(a, track_descent<EXACT, PPL, PRED>(p1, p2, a, lane, offi, offj, swx, swy, swd, s0.x, s0.y,
+                                                           xout, yout, s0.z, s0.w), xout, yout);
   if (FB) {
     FbRec r = fb_unchecked();
     if (v == KLT_TRACKED) {                                   // the backward leg: frame 2 into frame 1
       float xb, yb;
-      const int vb = track_outcome(a, track_descent<EXACT, PPL>(p2, p1, a, lane, offi, offj, swx, swy, swd,
-                                                                xout, yout, xb, yb), xb, yb);
+      float4 sb = make_float4(xout, yout, 0.0f, 0.0f);        // PRED: from the mirrored prior
+      if (PRED) {
+        if (lane == 0) sb = pred_back_start(pr.rec, a.nlevels, a.ss, f, x0, y0, xout, yout);
+        sb = shfl4(sb, 32);
+      }
+      const int vb = track_outcome(a, track_descent<EXACT, PPL, PRED>(p2, p1, a, lane, offi, offj, swx, swy, swd,
+                                                                      sb.x, sb.y, xb, yb, sb.z, sb.w), xb, yb);
       if (!fb_keep(fb.max_error, x0, y0, xb, yb, vb, r)) v = KLT_B200_FB_INCONSISTENT;
     }
     if (lane == 0) fb.rec[f] = r;
   }
+  if (PRED && lane == 0) pred_velocity(pr, io, f, v, xout, yout);
   if (lane == 0) record_feature(io, f, v, xout, yout);     // record (:1383-1437)
 }
 
@@ -1314,6 +1412,15 @@ struct klt_dev {
   unsigned long long* d_live;
   // forward-backward check: one FbRec per feature of the last tracking call that ran it (fb_n >= 0)
   FbRec* d_fb; int fb_cap, fb_n; float fb_max_error;   // (fb_max_error: of the tracker being launched)
+  // motion prior: per feature index a velocity record (valid for indices < vel_n) and the record of
+  // the last tracking call that ran with the prior (pred_n >= 0); explicit guesses gx | gy queued for
+  // the next tracking call (guess_n >= 0) in slot guess_slot of a two-slot ring (device buffers and
+  // pinned staging, slot s at s * 2 * guess_cap); ev_guess[s] is recorded behind the last copy into
+  // slot s and again behind the tracker that reads it, so a slot is refilled only once both are done
+  PredVel* d_vel; PredRec* d_pred; int pred_cap, pred_n, vel_n;
+  float* d_guess; float* h_guess; int guess_cap, guess_n, guess_slot;
+  cudaEvent_t ev_guess[2]; int guess_busy[2];
+  PredArgs pred;                // (of the tracker being launched)
 };
 
 // RAII around one kernel launch: counts it and, in profiling mode, brackets it
@@ -1471,6 +1578,7 @@ extern "C" int klt_dev_create(int device, klt_dev** out) {
   if (e != cudaSuccess) { free(c); return fail(nullptr, "cudaStreamCreate: %s", cudaGetErrorString(e)); }
   c->tstream = c->stream;
   c->fb_n = -1;
+  c->pred_n = -1; c->guess_n = -1;
   e = cudaMalloc(&c->d_live, sizeof(unsigned long long));
   if (e == cudaSuccess) e = cudaMemsetAsync(c->d_live, 0, sizeof(unsigned long long), c->stream);
   c->pdl = getenv("KLT_B200_PDL") ? atoi(getenv("KLT_B200_PDL")) : 1;
@@ -1538,6 +1646,8 @@ extern "C" void klt_dev_destroy(klt_dev* d) {
   cudaFree(d->frame_buf[0]); cudaFree(d->frame_buf[1]);
   guarded_free(d, d->d_x);
   guarded_free(d, d->d_fb);
+  guarded_free(d, d->d_vel); guarded_free(d, d->d_pred); guarded_free(d, d->d_guess); cudaFreeHost(d->h_guess);
+  for (int i = 0; i < 2; ++i) if (d->ev_guess[i]) cudaEventDestroy(d->ev_guess[i]);
   cudaFreeHost(d->h_x);
   for (int i = 0; i < 2; ++i) { guarded_free(d, d->c_val[i]); guarded_free(d, d->c_idx[i]); }
   cudaFree(d->cub_tmp); guarded_free(d, d->fmap); guarded_free(d, d->open_slots); guarded_free(d, d->rank_list); guarded_free(d, d->sel_state);
@@ -1573,6 +1683,7 @@ static int ensure_geometry(klt_dev* d, int W, int H, int L, int ss) {
   memset(d->read_pending, 0, sizeof(d->read_pending));
   memset(d->built_pending, 0, sizeof(d->built_pending));
   free_geometry(d);
+  d->vel_n = 0;                        // a velocity from frames of another size predicts nothing
   size_t per_set = 0;
   int w = W, h = H;
   int ws[KLT_DEV_MAX_LEVELS], hs[KLT_DEV_MAX_LEVELS], ps[KLT_DEV_MAX_LEVELS];
@@ -2685,50 +2796,54 @@ static FbArgs fb_args(const klt_dev* d) {
   return f;
 }
 
-template <bool EXACT, int PPL, bool FB>
+template <bool EXACT, int PPL, bool FB, bool PRED>
 static int launch_track(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n) {
   const int warps = 4;
   const size_t smem = EXACT ? (size_t)warps * 3 * a.ww * a.wh * sizeof(float) : 0;
-  if (set_smem(d, track_kernel<EXACT, PPL, FB>, smem)) return 1;
+  if (set_smem(d, track_kernel<EXACT, PPL, FB, PRED>, smem)) return 1;
   { Launch l(d, KID_TRACK, d->tstream);
-    track_kernel<EXACT, PPL, FB><<<(n + warps - 1) / warps, warps * 32, smem, d->tstream>>>(
-        v1, v2, a, n, feat_io(d), d->d_live, fb_args(d)); }
+    track_kernel<EXACT, PPL, FB, PRED><<<(n + warps - 1) / warps, warps * 32, smem, d->tstream>>>(
+        v1, v2, a, n, feat_io(d), d->d_live, fb_args(d), d->pred); }
   return 0;
 }
 template <bool EXACT, int PPL>
-static int launch_track(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb) {
-  return fb ? launch_track<EXACT, PPL, true>(d, v1, v2, a, n) : launch_track<EXACT, PPL, false>(d, v1, v2, a, n);
+static int launch_track(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb, bool pred) {
+  if (pred) return fb ? launch_track<EXACT, PPL, true, true>(d, v1, v2, a, n) : launch_track<EXACT, PPL, false, true>(d, v1, v2, a, n);
+  return fb ? launch_track<EXACT, PPL, true, false>(d, v1, v2, a, n) : launch_track<EXACT, PPL, false, false>(d, v1, v2, a, n);
 }
 
+template <int WW, int RPL, bool FB, bool PRED>
+static void launch_track_fast_t(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n) {
+  track_fast_kernel<WW, RPL, FB, PRED><<<(8 * n + 127) / 128, 128, 0, d->tstream>>>(
+      v1, v2, a, n, feat_io(d), d->d_live, fb_args(d), d->pred);
+}
 template <int WW, int RPL>
-static void launch_track_fast_t(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb) {
+static void launch_track_fast_t(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb, bool pred) {
   Launch l(d, KID_TRACK_FAST, d->tstream);
-  if (fb)
-    track_fast_kernel<WW, RPL, true><<<(8 * n + 127) / 128, 128, 0, d->tstream>>>(
-        v1, v2, a, n, feat_io(d), d->d_live, fb_args(d));
-  else
-    track_fast_kernel<WW, RPL, false><<<(8 * n + 127) / 128, 128, 0, d->tstream>>>(
-        v1, v2, a, n, feat_io(d), d->d_live, fb_args(d));
+  if (pred) fb ? launch_track_fast_t<WW, RPL, true, true>(d, v1, v2, a, n) : launch_track_fast_t<WW, RPL, false, true>(d, v1, v2, a, n);
+  else fb ? launch_track_fast_t<WW, RPL, true, false>(d, v1, v2, a, n) : launch_track_fast_t<WW, RPL, false, false>(d, v1, v2, a, n);
 }
 // square odd windows up to 15x15; returns false if this window has no instantiation
-static bool launch_track_fast(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb) {
+static bool launch_track_fast(klt_dev* d, const PyrView& v1, const PyrView& v2, const TrackArgs& a, int n, bool fb, bool pred) {
   switch (a.ww) {
-    case 3: launch_track_fast_t<3, 1>(d, v1, v2, a, n, fb); return true;
-    case 5: launch_track_fast_t<5, 1>(d, v1, v2, a, n, fb); return true;
+    case 3: launch_track_fast_t<3, 1>(d, v1, v2, a, n, fb, pred); return true;
+    case 5: launch_track_fast_t<5, 1>(d, v1, v2, a, n, fb, pred); return true;
     case 7:
-      if (d->track7_off) { launch_track_fast_t<7, 1>(d, v1, v2, a, n, fb); return true; }
+      if (d->track7_off) { launch_track_fast_t<7, 1>(d, v1, v2, a, n, fb, pred); return true; }
       if (!d->no_track7w) {                                  // one warp per feature, scalar loads
         Launch l(d, KID_TRACK7W, d->tstream);
-        launch_k(fb ? track7w_kernel<true> : track7w_kernel<false>, dim3((n + 3) / 4), dim3(128), 0, d->tstream,
-                 d->pdl != 0 && !d->overlap, v1, v2, a, n, feat_io(d), d->d_live, fb_args(d));
+        launch_k(pred ? (fb ? track7w_kernel<true, true> : track7w_kernel<false, true>)
+                      : (fb ? track7w_kernel<true, false> : track7w_kernel<false, false>),
+                 dim3((n + 3) / 4), dim3(128), 0, d->tstream,
+                 d->pdl != 0 && !d->overlap, v1, v2, a, n, feat_io(d), d->d_live, fb_args(d), d->pred);
         return true;
       }
-      launch_track_fast_t<7, 1>(d, v1, v2, a, n, fb);
+      launch_track_fast_t<7, 1>(d, v1, v2, a, n, fb, pred);
       return true;
-    case 9: launch_track_fast_t<9, 2>(d, v1, v2, a, n, fb); return true;
-    case 11: launch_track_fast_t<11, 2>(d, v1, v2, a, n, fb); return true;
-    case 13: launch_track_fast_t<13, 2>(d, v1, v2, a, n, fb); return true;
-    case 15: launch_track_fast_t<15, 2>(d, v1, v2, a, n, fb); return true;
+    case 9: launch_track_fast_t<9, 2>(d, v1, v2, a, n, fb, pred); return true;
+    case 11: launch_track_fast_t<11, 2>(d, v1, v2, a, n, fb, pred); return true;
+    case 13: launch_track_fast_t<13, 2>(d, v1, v2, a, n, fb, pred); return true;
+    case 15: launch_track_fast_t<15, 2>(d, v1, v2, a, n, fb, pred); return true;
     default: return false;
   }
 }
@@ -2755,6 +2870,14 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
   const bool fb = p->fb_max_error > 0.0f;
   d->fb_n = fb ? n : -1;
   d->fb_max_error = p->fb_max_error;
+  const int guess_n = d->guess_n;                    // explicit guesses are consumed by this call
+  d->guess_n = -1;
+  if (p->predict < 0 || p->predict > 1) return fail(d, "klt_dev_track: predict = %d (0: none, 1: velocity)", p->predict);
+  if (guess_n >= 0 && guess_n != n)
+    return fail(d, "klt_dev_track: %d guesses queued for a call on %d features", guess_n, n);
+  const bool pred = p->predict != 0 || guess_n >= 0;
+  d->pred_n = pred ? n : -1;
+  if (!pred) d->vel_n = 0;                           // this call leaves the velocity records behind
   if (n == 0) return 0;
   if (fb && d->fb_cap < n) {                         // the check's result records (klt_dev_fb_results)
     if (sync_all(d)) return fail(d, "stream synchronisation failed");
@@ -2763,6 +2886,21 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
     CU(guarded_malloc(d, &d->d_fb, (size_t)cap * sizeof(FbRec)));
     d->fb_cap = cap;
   }
+  if (pred && d->pred_cap < n) {                     // the prior's records: new ones hold no velocity
+    if (sync_all(d)) return fail(d, "stream synchronisation failed");
+    guarded_free(d, d->d_vel); guarded_free(d, d->d_pred); d->d_vel = nullptr; d->d_pred = nullptr;
+    d->pred_cap = 0; d->vel_n = 0;
+    const int cap = (n + 1023) / 1024 * 1024;
+    CU(guarded_malloc(d, &d->d_vel, (size_t)cap * sizeof(PredVel)));
+    CU(guarded_malloc(d, &d->d_pred, (size_t)cap * sizeof(PredRec)));
+    d->pred_cap = cap;
+  }
+  float* const guesses = d->d_guess + (size_t)d->guess_slot * 2 * d->guess_cap;
+  d->pred.gx = guess_n >= 0 ? guesses : nullptr;
+  d->pred.gy = guess_n >= 0 ? guesses + d->guess_cap : nullptr;
+  d->pred.vel = d->d_vel; d->pred.rec = d->d_pred;
+  d->pred.vel_n = p->predict == 1 ? d->vel_n : 0;
+  if (pred) d->vel_n = n;                            // the tracker writes the records of features 0 .. n-1
   if (feat_flush(d)) return 1;
   if (d->feat_pending) {                             // features uploaded on the copy stream
     CU(cudaStreamWaitEvent(d->tstream, d->ev_feat, 0));
@@ -2785,22 +2923,23 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
   const int ppl = (npix + 31) / 32;
   int rc;
   if (p->exact) {
-    if (ppl <= 2) rc = launch_track<true, 2>(d, v1, v2, a, n, fb);
-    else if (ppl <= 4) rc = launch_track<true, 4>(d, v1, v2, a, n, fb);
-    else if (ppl <= 8) rc = launch_track<true, 8>(d, v1, v2, a, n, fb);
-    else if (ppl <= 16) rc = launch_track<true, 16>(d, v1, v2, a, n, fb);
+    if (ppl <= 2) rc = launch_track<true, 2>(d, v1, v2, a, n, fb, pred);
+    else if (ppl <= 4) rc = launch_track<true, 4>(d, v1, v2, a, n, fb, pred);
+    else if (ppl <= 8) rc = launch_track<true, 8>(d, v1, v2, a, n, fb, pred);
+    else if (ppl <= 16) rc = launch_track<true, 16>(d, v1, v2, a, n, fb, pred);
     else return fail(d, "tracking window %d x %d too large (max 512 pixels)", a.ww, a.wh);
-  } else if (!d->force_generic && !a.lighting && a.ww == a.wh && a.ww <= 15 && launch_track_fast(d, v1, v2, a, n, fb)) {
+  } else if (!d->force_generic && !a.lighting && a.ww == a.wh && a.ww <= 15 && launch_track_fast(d, v1, v2, a, n, fb, pred)) {
     rc = 0;
   } else {
-    if (ppl <= 2) rc = launch_track<false, 2>(d, v1, v2, a, n, fb);
-    else if (ppl <= 4) rc = launch_track<false, 4>(d, v1, v2, a, n, fb);
-    else if (ppl <= 8) rc = launch_track<false, 8>(d, v1, v2, a, n, fb);
-    else if (ppl <= 16) rc = launch_track<false, 16>(d, v1, v2, a, n, fb);
+    if (ppl <= 2) rc = launch_track<false, 2>(d, v1, v2, a, n, fb, pred);
+    else if (ppl <= 4) rc = launch_track<false, 4>(d, v1, v2, a, n, fb, pred);
+    else if (ppl <= 8) rc = launch_track<false, 8>(d, v1, v2, a, n, fb, pred);
+    else if (ppl <= 16) rc = launch_track<false, 16>(d, v1, v2, a, n, fb, pred);
     else return fail(d, "tracking window %d x %d too large (max 512 pixels)", a.ww, a.wh);
   }
   if (rc) return rc;
   CU(cudaGetLastError());
+  if (guess_n >= 0) CU(cudaEventRecord(d->ev_guess[d->guess_slot], d->tstream));   // the slot's last reader
   if (d->overlap) {
     CU(cudaEventRecord(d->ev_read[slot_prev], d->tstream));
     CU(cudaEventRecord(d->ev_read[slot_cur], d->tstream));
@@ -2824,6 +2963,69 @@ extern "C" int klt_dev_fb_results(klt_dev* d, int n, float* xb, float* yb, float
     if (yb) yb[i] = h[i].yb;
     if (err) err[i] = h[i].err;
     if (back_val) back_val[i] = h[i].back_val;
+  }
+  free(h);
+  return 0;
+}
+
+// Pipelined drivers queue the guesses of step k + 1 while step k's tracker may not have run yet: the
+// guesses go into the other slot of the ring, and a slot is refilled only after the tracker that
+// read it (and the copy that filled it) has finished -- the host waits for that, so it runs at most
+// two tracking calls with explicit guesses ahead of the device.
+extern "C" int klt_dev_set_guesses(klt_dev* d, int n, const float* gx, const float* gy, int on_device) {
+  CU(cudaSetDevice(d->device));
+  if (n < 0 || (n > 0 && (!gx || !gy))) return fail(d, "set_guesses: bad count or NULL array");
+  if (!d->ev_guess[0])
+    for (int i = 0; i < 2; ++i) CU(cudaEventCreateWithFlags(&d->ev_guess[i], cudaEventDisableTiming));
+  if (d->guess_cap < n) {
+    if (sync_all(d)) return fail(d, "stream synchronisation failed");
+    guarded_free(d, d->d_guess); cudaFreeHost(d->h_guess);
+    d->d_guess = nullptr; d->h_guess = nullptr; d->guess_cap = 0; d->guess_busy[0] = d->guess_busy[1] = 0;
+    const int cap = (n + 1023) / 1024 * 1024;
+    CU(guarded_malloc(d, &d->d_guess, (size_t)cap * 4 * sizeof(float)));
+    CU(cudaMallocHost(&d->h_guess, (size_t)cap * 4 * sizeof(float)));
+    d->guess_cap = cap;
+  }
+  const int s = d->guess_slot ^ 1;
+  if (d->guess_busy[s]) { CU(cudaEventSynchronize(d->ev_guess[s])); d->guess_busy[s] = 0; }
+  float* dst = d->d_guess + (size_t)s * 2 * d->guess_cap;
+  if (n > 0) {                 // on the copy stream like the feature upload: the tracker waits for ev_feat
+    const float *sx = gx, *sy = gy;
+    cudaMemcpyKind kind = cudaMemcpyDeviceToDevice;
+    if (!on_device) {          // through pinned staging: the copy is asynchronous, the caller's arrays free
+      float* h = d->h_guess + (size_t)s * 2 * d->guess_cap;
+      memcpy(h, gx, (size_t)n * sizeof(float));
+      memcpy(h + d->guess_cap, gy, (size_t)n * sizeof(float));
+      sx = h; sy = h + d->guess_cap; kind = cudaMemcpyHostToDevice;
+    }
+    CU(cudaMemcpyAsync(dst, sx, (size_t)n * sizeof(float), kind, d->cstream));
+    CU(cudaMemcpyAsync(dst + d->guess_cap, sy, (size_t)n * sizeof(float), kind, d->cstream));
+    CU(cudaEventRecord(d->ev_guess[s], d->cstream));
+    d->guess_busy[s] = 1;
+    CU(cudaEventRecord(d->ev_feat, d->cstream));
+    d->feat_pending = 1;
+  }
+  d->guess_n = n;
+  d->guess_slot = s;
+  return 0;
+}
+
+extern "C" int klt_dev_guesses_pending(const klt_dev* d) { return d->guess_n; }
+
+extern "C" int klt_dev_prediction_results(klt_dev* d, int n, float* gx, float* gy, int* source) {
+  CU(cudaSetDevice(d->device));
+  if (d->pred_n < 0) return fail(d, "prediction_results: the last tracking call ran without prediction");
+  if (n != d->pred_n) return fail(d, "prediction_results: %d features requested, the last tracking call had %d", n, d->pred_n);
+  if (n == 0) return 0;
+  PredRec* h = (PredRec*)malloc((size_t)n * sizeof(PredRec));
+  if (!h) return fail(d, "out of host memory");
+  cudaError_t e = cudaMemcpyAsync(h, d->d_pred, (size_t)n * sizeof(PredRec), cudaMemcpyDeviceToHost, d->tstream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(d->tstream);
+  if (e != cudaSuccess) { free(h); return fail(d, "prediction_results: %s", cudaGetErrorString(e)); }
+  for (int i = 0; i < n; ++i) {
+    if (gx) gx[i] = h[i].gx;
+    if (gy) gy[i] = h[i].gy;
+    if (source) source[i] = h[i].source;
   }
   free(h);
   return 0;

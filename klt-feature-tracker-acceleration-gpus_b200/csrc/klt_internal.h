@@ -15,6 +15,7 @@ typedef struct klt_tc_state {
   int device;            /* CUDA device ordinal, -1 = KLT_B200_DEVICE / current */
   int exact;             /* arithmetic mode for tracking pyramids            */
   float fb_max_error;    /* forward-backward check, > 0: on (KLTB200SetForwardBackward) */
+  int predict;           /* motion prior: KLT_B200_PREDICT_* (KLTB200SetPrediction)      */
   int last_slot;         /* slot holding the previous frame's pyramids       */
   /* affine consistency check: which host template (aff_img pointer) the device's template
    * slot i mirrors; valid for list aff_list while klt_aff_epoch == aff_epoch */

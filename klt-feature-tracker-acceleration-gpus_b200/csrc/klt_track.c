@@ -50,6 +50,16 @@ static void fill_track_params(KLT_TrackingContext tc, const klt_tc_state *s, klt
   p->exact = s->exact;
   p->lighting_insensitive = tc->lighting_insensitive ? 1 : 0;
   p->fb_max_error = s->fb_max_error > 0.0f ? s->fb_max_error : 0.0f;
+  p->predict = s->predict;
+}
+
+/* explicit guesses (KLTB200SetGuesses or klt_dev_set_guesses: one queue, on the device) are consumed
+ * by the next tracking call, which must have as many features; checked before anything is queued */
+static void check_guesses(klt_dev *dev, int n, const char *who)
+{
+  const int g = klt_dev_guesses_pending(dev);
+  if (g >= 0 && g != n)
+    KLTError("(%s) %d guesses were set (KLTB200SetGuesses) for a call on %d features", who, g, n);
 }
 
 static void check_supported(KLT_TrackingContext tc, int pipelined)
@@ -264,6 +274,7 @@ static void track_common(KLT_TrackingContext tc, const KLT_PixelType *img1,
   klt_fix_window(tc, "KLTTrackFeatures", 1);
   check_supported(tc, 0);
   dev = klt_state_device(s);
+  check_guesses(dev, n, "KLTTrackFeatures");
 
   /* Everything below is queued on the context stream without waiting: feature upload,
    * frame upload, pyramid kernels, tracker, result download; one synchronisation at the end. */
@@ -473,6 +484,9 @@ void KLTTrackFeaturesSequence(KLT_TrackingContext tc, KLT_PixelType *const *fram
 
   if (frames == NULL || nframes < 1)
     KLTError("(KLTTrackFeaturesSequence) needs at least one frame");
+  if (s->dev != NULL && klt_dev_guesses_pending(s->dev) >= 0)
+    KLTError("(KLTTrackFeaturesSequence) guesses are set (KLTB200SetGuesses): the sequence call predicts "
+             "by velocity only (KLTB200SetPrediction)");
   if (ft != NULL) {
     if (fl->nFeatures != ft->nFeatures)
       KLTError("(KLTTrackFeaturesSequence) FeatureList and FeatureTable must have the same number of features");

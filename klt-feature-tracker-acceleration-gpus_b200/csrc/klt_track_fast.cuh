@@ -46,13 +46,16 @@ __device__ __forceinline__ void sample_row(const float* __restrict__ img, int pi
 // the status of the finest level reached and the end position, before the border test.  Called by
 // all lanes of the warp; groups with alive == false only take part in the shuffles.
 // WW: window width (odd, <= 15); RPL: window rows per lane (window height <= 8 * RPL)
-template <int WW, int RPL>
+// G: (x, y) and the guess (gx, gy) the descent starts from are given at the coarsest level (pred_start).
+template <int WW, int RPL, bool G = false>
 __device__ __forceinline__ int track_fast_descent(const PyrView& p1, const PyrView& p2, const TrackArgs& a,
-                                                  int r8, bool alive, float x, float y, float& xend, float& yend) {
+                                                  int r8, bool alive, float x, float y, float& xend, float& yend,
+                                                  float gx = 0.0f, float gy = 0.0f) {
   const int wh = a.wh, hw = WW / 2, hh = wh / 2;
   float xloc = x, yloc = y;
-  for (int r = a.nlevels - 1; r >= 0; --r) { xloc = xloc / a.ss; yloc = yloc / a.ss; }
-  float xout = xloc, yout = yloc;
+  if (!G)
+    for (int r = a.nlevels - 1; r >= 0; --r) { xloc = xloc / a.ss; yloc = yloc / a.ss; }
+  float xout = G ? gx : xloc, yout = G ? gy : yloc;
   int status = KLT_TRACKED;
   bool running = alive;                                      // false once a level returned SMALL_DET / OOB
 
@@ -199,18 +202,20 @@ __device__ __forceinline__ int track_fast_descent(const PyrView& p1, const PyrVi
 }
 
 // FB: the forward-backward check runs in the same group after the forward leg (klt_dev_fb_results)
-template <int WW, int RPL, bool FB>
+// PRED: the descent starts from the feature's guess (PredArgs, klt_dev_prediction_results)
+template <int WW, int RPL, bool FB, bool PRED = false>
 __global__ void __launch_bounds__(128)
 track_fast_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
-                  unsigned long long* __restrict__ live_total, FbArgs fb) {
+                  unsigned long long* __restrict__ live_total, FbArgs fb, PredArgs pr) {
   const int lane = threadIdx.x & 31;
   const int r8 = lane & 7;                                   // lane within the feature group
   const int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 3;   // feature of this group
 
   bool alive = false;                                        // feature still being tracked
   float x0 = 0.0f, y0 = 0.0f;
+  int v0 = -1;
   if (f < n) {
-    const int v0 = io.val[(size_t)f * io.istride];
+    v0 = io.val[(size_t)f * io.istride];
     alive = v0 >= 0;                                         // only features that are not lost (:1346)
     if (alive) { x0 = io.x[(size_t)f * io.istride]; y0 = io.y[(size_t)f * io.istride]; }
   }
@@ -220,18 +225,32 @@ track_fast_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
   }
   if (!__any_sync(0xffffffffu, alive)) {
     if (FB && f < n && r8 == 0) fb.rec[f] = fb_unchecked();
+    if (PRED && f < n && r8 == 0) pred_skip(pr, f);
     return;
   }
 
+  float4 s0 = make_float4(x0, y0, 0.0f, 0.0f);              // PRED: start and guess at the coarsest level
+  if (PRED) {
+    if (r8 == 0) {
+      if (alive) s0 = pred_start(pr.gx, pr.gy, pr.vel, pr.rec, pr.vel_n, a.nlevels, a.ss, f, v0, x0, y0);
+      else if (f < n) pred_skip(pr, f);
+    }
+    s0 = shfl4(s0, 8);
+  }
   float xout, yout;
-  int v = track_fast_descent<WW, RPL>(p1, p2, a, r8, alive, x0, y0, xout, yout);
+  int v = track_fast_descent<WW, RPL, PRED>(p1, p2, a, r8, alive, s0.x, s0.y, xout, yout, s0.z, s0.w);
   if (alive) v = track_outcome(a, v, xout, yout);
   if (FB) {
     FbRec r = fb_unchecked();
     const bool back = alive && v == KLT_TRACKED;             // the backward leg: frame 2 into frame 1
     if (__any_sync(0xffffffffu, back)) {
       float xb, yb;
-      int vb = track_fast_descent<WW, RPL>(p2, p1, a, r8, back, xout, yout, xb, yb);
+      float4 sb = make_float4(xout, yout, 0.0f, 0.0f);        // PRED: from the mirrored prior
+      if (PRED) {
+        if (back && r8 == 0) sb = pred_back_start(pr.rec, a.nlevels, a.ss, f, x0, y0, xout, yout);
+        sb = shfl4(sb, 8);
+      }
+      int vb = track_fast_descent<WW, RPL, PRED>(p2, p1, a, r8, back, sb.x, sb.y, xb, yb, sb.z, sb.w);
       if (back) {
         vb = track_outcome(a, vb, xb, yb);
         if (!fb_keep(fb.max_error, x0, y0, xb, yb, vb, r)) v = KLT_B200_FB_INCONSISTENT;
@@ -239,6 +258,7 @@ track_fast_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
     }
     if (f < n && r8 == 0) fb.rec[f] = r;
   }
+  if (PRED && alive && r8 == 0) pred_velocity(pr, io, f, v, xout, yout);
   if (alive && r8 == 0) record_feature(io, f, v, xout, yout);   // record (:1383-1437)
 }
 
@@ -328,15 +348,19 @@ __device__ __forceinline__ void warp_sum4x(float& g0, float& g1, float& g2, floa
 // The pyramid descent of the warp's feature from (x, y) in p1's frame (gathers with L2 policy pol1)
 // into p2's frame (pol2): the status of the finest level reached and the end position, before the
 // border test.
+// G: (x, y) and the guess (gx, gy) the descent starts from are given at the coarsest level (pred_start).
+template <bool G = false>
 __device__ __forceinline__ int track7w_descent(const PyrView& p1, const PyrView& p2, const TrackArgs& a, int lane,
                                                unsigned long long pol1, unsigned long long pol2,
-                                               float x, float y, float& xend, float& yend) {
+                                               float x, float y, float& xend, float& yend,
+                                               float gx = 0.0f, float gy = 0.0f) {
   constexpr int hw = 3, hh = 3;
   const int r = lane >> 2, c = lane & 3;                     // footprint row, column pair
   const bool v0 = r < 7, v1 = r < 7 && c < 3;                // window samples (2c, r) and (2c + 1, r)
   float xloc = x, yloc = y;
-  for (int l = a.nlevels - 1; l >= 0; --l) { xloc = xloc / a.ss; yloc = yloc / a.ss; }
-  float xout = xloc, yout = yloc;
+  if (!G)
+    for (int l = a.nlevels - 1; l >= 0; --l) { xloc = xloc / a.ss; yloc = yloc / a.ss; }
+  float xout = G ? gx : xloc, yout = G ? gy : yloc;
   int status = KLT_TRACKED;
 
   for (int l = a.nlevels - 1; l >= 0; --l) {
@@ -436,10 +460,12 @@ __device__ __forceinline__ int track7w_descent(const PyrView& p1, const PyrView&
 // FB: the forward-backward check runs in the same warp after the forward leg (klt_dev_fb_results).
 // Its backward leg reads the new frame with the new frame's policy (evict_last) and the old frame
 // with the old frame's (evict_first), as the forward leg does.
-template <bool FB>
+// PRED: the descent starts from the feature's guess (PredArgs, klt_dev_prediction_results); lane 0
+// reads and writes the velocity record after pdl_wait, like the features.
+template <bool FB, bool PRED = false>
 __global__ void __launch_bounds__(128)
 track7w_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
-               unsigned long long* __restrict__ live_total, FbArgs fb) {
+               unsigned long long* __restrict__ live_total, FbArgs fb, PredArgs pr) {
   const int lane = threadIdx.x & 31;
   const int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const unsigned long long pol1 = l2_policy(a.l2_keep ? 2 : 0), pol2 = l2_policy(a.l2_keep ? 1 : 0);
@@ -448,23 +474,38 @@ track7w_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
   // the stream -- the next frame's level-0 kernel -- may move into the SMs as these warps retire
   pdl_launch_dependents();
   if (f >= n) return;
-  if (io.val[(size_t)f * io.istride] < 0) {                   // only features that are not lost (:1346)
+  const int val_in = io.val[(size_t)f * io.istride];
+  if (val_in < 0) {                                           // only features that are not lost (:1346)
     if (FB && lane == 0) fb.rec[f] = fb_unchecked();
+    if (PRED && lane == 0) pred_skip(pr, f);
     return;
   }
   if (lane == 0) atomicAdd(live_total, 1ULL);
   const float x0 = io.x[(size_t)f * io.istride], y0 = io.y[(size_t)f * io.istride];
+  float4 s0 = make_float4(x0, y0, 0.0f, 0.0f);              // PRED: start and guess at the coarsest level
+  if (PRED) {
+    if (lane == 0) s0 = pred_start(pr.gx, pr.gy, pr.vel, pr.rec, pr.vel_n, a.nlevels, a.ss, f, val_in, x0, y0);
+    s0 = shfl4(s0, 32);
+  }
   float xout, yout;
-  int v = track_outcome(a, track7w_descent(p1, p2, a, lane, pol1, pol2, x0, y0, xout, yout), xout, yout);
+  int v = track_outcome(a, track7w_descent<PRED>(p1, p2, a, lane, pol1, pol2, s0.x, s0.y, xout, yout, s0.z, s0.w),
+                        xout, yout);
   if (FB) {
     FbRec r = fb_unchecked();
     if (v == KLT_TRACKED) {                                   // the backward leg: frame 2 into frame 1
       float xb, yb;
-      const int vb = track_outcome(a, track7w_descent(p2, p1, a, lane, pol2, pol1, xout, yout, xb, yb), xb, yb);
+      float4 sb = make_float4(xout, yout, 0.0f, 0.0f);        // PRED: from the mirrored prior
+      if (PRED) {
+        if (lane == 0) sb = pred_back_start(pr.rec, a.nlevels, a.ss, f, x0, y0, xout, yout);
+        sb = shfl4(sb, 32);
+      }
+      const int vb = track_outcome(a, track7w_descent<PRED>(p2, p1, a, lane, pol2, pol1, sb.x, sb.y, xb, yb, sb.z, sb.w),
+                                   xb, yb);
       if (!fb_keep(fb.max_error, x0, y0, xb, yb, vb, r)) v = KLT_B200_FB_INCONSISTENT;
     }
     if (lane == 0) fb.rec[f] = r;
   }
+  if (PRED && lane == 0) pred_velocity(pr, io, f, v, xout, yout);
   if (lane == 0) record_feature(io, f, v, xout, yout);     // record (:1383-1437)
 }
 

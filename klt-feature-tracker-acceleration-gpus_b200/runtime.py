@@ -35,7 +35,8 @@ class TrackParams(C.Structure):       # klt_dev_track_params
                 ("step_factor", C.c_float), ("max_iterations", C.c_int),
                 ("min_determinant", C.c_float), ("min_displacement", C.c_float),
                 ("max_residue", C.c_float), ("borderx", C.c_int), ("bordery", C.c_int),
-                ("exact", C.c_int), ("lighting_insensitive", C.c_int), ("fb_max_error", C.c_float)]
+                ("exact", C.c_int), ("lighting_insensitive", C.c_int), ("fb_max_error", C.c_float),
+                ("predict", C.c_int)]
 
 
 class SelectParams(C.Structure):      # klt_dev_select_params
@@ -110,6 +111,9 @@ DEV_API = {
     "klt_dev_trace_get": (C.c_char_p, [C.c_void_p, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "klt_dev_live_total": (C.c_int, [C.c_void_p, C.POINTER(C.c_ulonglong), C.c_int]),
     "klt_dev_fb_results": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "klt_dev_set_guesses": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "klt_dev_guesses_pending": (C.c_int, [C.c_void_p]),
+    "klt_dev_prediction_results": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     # include/klt_b200.h
     "KLTB200SetDevice": (None, [_TC, C.c_int]),
     "KLTB200SetExact": (None, [_TC, C.c_int]),
@@ -117,6 +121,10 @@ DEV_API = {
     "KLTB200SetForwardBackward": (None, [_TC, C.c_float]),
     "KLTB200GetForwardBackward": (C.c_float, [_TC]),
     "KLTB200ForwardBackwardResult": (None, [_TC, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "KLTB200SetPrediction": (None, [_TC, C.c_int]),
+    "KLTB200GetPrediction": (C.c_int, [_TC]),
+    "KLTB200SetGuesses": (None, [_TC, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "KLTB200PredictionResult": (None, [_TC, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "KLTB200Device": (C.c_void_p, [_TC]),
     "KLTB200LastSlot": (C.c_int, [_TC]),
     "KLTTrackFeaturesDevice": (None, [_TC, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, _FL]),
@@ -209,11 +217,38 @@ class B200Library(capi.KLTLibrary):
         self.dev_check(dev, self.lib.klt_dev_read_level(dev, slot, which, level, out))
         return out
 
-    def track_params(self, tc, exact=0, fb_max_error=0.0) -> TrackParams:
+    def track_params(self, tc, exact=0, fb_max_error=0.0, predict=0) -> TrackParams:
         t = tc.contents
         return TrackParams(t.window_width, t.window_height, t.step_factor, t.max_iterations,
                            t.min_determinant, t.min_displacement, t.max_residue,
-                           t.borderx, t.bordery, exact, t.lighting_insensitive, fb_max_error)
+                           t.borderx, t.bordery, exact, t.lighting_insensitive, fb_max_error, predict)
+
+    def set_guesses(self, tc, gx, gy, on_device=False):
+        """KLTB200SetGuesses for the next tracking call on tc: float32 host arrays, or with on_device
+        contiguous float32 CUDA tensors (complete: synchronise their stream first)"""
+        if on_device:
+            if gx.numel() != gy.numel():
+                raise ValueError("gx and gy differ in size")
+            self.lib.KLTB200SetGuesses(tc, gx.numel(), C.c_void_p(gx.data_ptr()), C.c_void_p(gy.data_ptr()), 1)
+            return
+        gx = np.ascontiguousarray(gx, np.float32)
+        gy = np.ascontiguousarray(gy, np.float32)
+        if gx.shape != gy.shape:
+            raise ValueError("gx and gy differ in shape")
+        self.lib.KLTB200SetGuesses(tc, gx.size, gx.ctypes.data, gy.ctypes.data, 0)
+
+    def prediction(self, tc, n):
+        """KLTB200PredictionResult: (gx, gy, source) of the last tracking call on tc"""
+        gx, gy, src = np.empty(n, np.float32), np.empty(n, np.float32), np.empty(n, np.int32)
+        self.lib.KLTB200PredictionResult(tc, n, gx.ctypes.data, gy.ctypes.data, src.ctypes.data)
+        return gx, gy, src
+
+    def dev_prediction(self, dev, n):
+        """klt_dev_prediction_results: (gx, gy, source) of the last klt_dev_track* call on dev"""
+        gx, gy, src = np.empty(n, np.float32), np.empty(n, np.float32), np.empty(n, np.int32)
+        self.dev_check(dev, self.lib.klt_dev_prediction_results(dev, n, gx.ctypes.data, gy.ctypes.data,
+                                                                src.ctypes.data))
+        return gx, gy, src
 
     def forward_backward(self, tc, n):
         """KLTB200ForwardBackwardResult: (xb, yb, err, back_val) of the last tracking call on tc"""
