@@ -15,6 +15,9 @@ extern "C" {
 /* val of a feature the forward-backward check rejected (KLTB200SetForwardBackward) */
 #define KLT_B200_FB_INCONSISTENT  -6
 
+/* val of a feature the global motion check rejected (KLTB200SetMotionCheck) */
+#define KLT_B200_MOTION_OUTLIER  -7
+
 /* CUDA device the context's work runs on.  Default: environment variable
  * KLT_B200_DEVICE, else the calling thread's current device.  Must be called
  * before the first Select/Track call on tc. */
@@ -79,6 +82,40 @@ void KLTB200SetGuesses(KLT_TrackingContext tc, int n, const float *gx, const flo
  * gx = gy = -1 without one.  Synchronises.  KLTError when that call ran without prediction or had a
  * number of features other than n. */
 void KLTB200PredictionResult(KLT_TrackingContext tc, int n, float *gx, float *gy, int *source);
+
+/* Global motion check of every tracking call on tc (the calls above; each frame of
+ * KLTTrackFeaturesSequence counts as one call).  After the tracker and the forward-backward check, and
+ * before the affine check, a RANSAC homography is fitted on the device to the call's correspondences:
+ * the features that entered with val >= 0 and are KLT_TRACKED, from where they started to where they
+ * were tracked.  `hypotheses` fixed samples of 4 correspondences are solved and scored, the one with
+ * the most inliers (reprojection distance <= max_error pixels) wins, and a least-squares fit over its
+ * inliers refines it.  When the final model keeps at least 8 features, every other correspondence is
+ * lost as x = y = -1, val = KLT_B200_MOTION_OUTLIER, so that KLTReplaceLostFeatures refills the slot
+ * and the affine check releases its template; the features it keeps are exactly as with the check off.
+ * With fewer, nothing is dropped.  The arithmetic is the same in both arithmetic modes.
+ * max_error <= 0 switches the check off; hypotheses == 0 means 1024, else 1 .. 65536.  NaN or a
+ * hypothesis count out of range ends in KLTError.  Default: environment variable
+ * KLT_B200_MOTION_MAX_ERROR when tc's state is created, else off.  The check makes the tracker write
+ * its results on the device, so the per-call API downloads them instead of receiving posted writes. */
+typedef struct {
+  float H[9];       /* row-major, maps frame-1 pixel coordinates to frame 2, H[8] = 1; NaN when !valid */
+  int   valid;      /* 1: a model was found and applied                                            */
+  int   tracked;    /* features that entered the check (val == KLT_TRACKED after the tracker / FB)  */
+  int   inliers;    /* features kept by the final model                                             */
+  int   hypothesis; /* index of the winning hypothesis, -1 when none                                */
+} KLT_B200_MotionModel;
+void  KLTB200SetMotionCheck(KLT_TrackingContext tc, float max_error, int hypotheses);
+float KLTB200GetMotionCheck(KLT_TrackingContext tc, int *hypotheses);
+/* Per feature of the last tracking call on tc (the last frame of a sequence or resident step): its
+ * reprojection distance under the final model, -1 for a feature the check did not evaluate, +inf for
+ * one the model maps behind the camera.  Synchronises.  KLTError when that call ran without the check
+ * or had a number of features other than n. */
+void  KLTB200MotionResult(KLT_TrackingContext tc, int n, float *err);
+/* The models of the last `count` tracking calls on tc that ran the check, oldest first, with no
+ * per-frame synchronisation in between (a sequence call yields one per frame).  The device keeps the
+ * last 4096; a call without the check clears them.  Synchronises.  KLTError when count is larger
+ * than recorded. */
+void  KLTB200MotionModels(KLT_TrackingContext tc, int count, KLT_B200_MotionModel *out);
 
 /* the device context behind tc (created on demand) */
 klt_dev *KLTB200Device(KLT_TrackingContext tc);

@@ -74,7 +74,18 @@ typedef struct {
   float fb_max_error;          /* > 0: forward-backward check in the same launch (klt_dev_fb_results);
                                   0: off */
   int   predict;               /* motion prior: 0 none, 1 constant velocity (klt_dev_prediction_results) */
+  float motion_max_error;      /* > 0: global motion check behind the tracker (klt_dev_motion_results); 0: off */
+  int   motion_hypotheses;     /* its RANSAC hypotheses, 1 .. 65536; 0: 1024 */
 } klt_dev_track_params;
+
+/* one tracking call's global motion model (klt_dev_motion_models); the layout of KLT_B200_MotionModel */
+typedef struct {
+  float H[9];                  /* row-major, frame-1 pixel coordinates to frame 2, H[8] = 1; NaN when !valid */
+  int   valid;                 /* 1: a model was found and applied */
+  int   tracked;               /* features that entered the check */
+  int   inliers;               /* features kept by the final model */
+  int   hypothesis;            /* index of the winning hypothesis, -1 when none */
+} klt_dev_motion_model;
 
 /* replaces the scalar arguments of _KLTSelectGoodFeatures /
  * _enforceMinimumDistance (reference src/V1/selectGoodFeatures.c:297-453). */
@@ -160,6 +171,25 @@ int klt_dev_set_guesses(klt_dev *d, int n, const float *gx, const float *gy, int
 /* the number of guesses queued for the next klt_dev_track* call, -1 when none are */
 int klt_dev_guesses_pending(const klt_dev *d);
 int klt_dev_prediction_results(klt_dev *d, int n, float *gx, float *gy, int *source);
+/* Global motion check (motion_max_error > 0): three kernels behind the tracker of the same call fit a
+ * homography to the call's correspondences -- features with input val >= 0 that the tracker (and the
+ * forward-backward check) left KLT_TRACKED -- by RANSAC over motion_hypotheses fixed samples, refine it
+ * by least squares over the winner's inliers, and, when it keeps at least 8 features, record every
+ * other correspondence as (-1, -1, KLT_B200_MOTION_OUTLIER); the affine check runs after it.  The
+ * positions before the tracker are kept by one D2D copy (shared with the affine check), and the
+ * tracker writes to the device arrays (feature download by D2H copy); record mode is refused.  The
+ * algorithm is fixed and deterministic (DESIGN.md 4, "Global motion check").
+ * klt_dev_motion_results copies the per-feature reprojection distance of the last klt_dev_track* call
+ * under its final model (-1 for a feature the check did not evaluate, +inf when the model maps it
+ * behind the camera); fails unless that call ran the check on exactly n features.  Synchronises.
+ * klt_dev_motion_models copies the models of the last `count` tracking calls that ran the check,
+ * oldest first; the device keeps the last 4096, a call without the check clears them, and asking for
+ * more than are recorded fails.  Synchronises.
+ * klt_dev_motion_counts (test support) copies the last checked call's number of correspondences m and
+ * each hypothesis' inlier count under the scoring rule (-1: no model), for exactly its hyps. */
+int klt_dev_motion_results(klt_dev *d, int n, float *err);
+int klt_dev_motion_models(klt_dev *d, int count, klt_dev_motion_model *out);
+int klt_dev_motion_counts(klt_dev *d, int hyps, int *m, int *counts);
 /* Ring of pinned snapshots of the resident features for pipelined drivers
  * (KLTTrackFeaturesSequence): klt_dev_snapshot_ring sizes it (depth <= 64 slots),
  * klt_dev_snapshot_push queues a copy of the current x | y | val into a slot behind the work

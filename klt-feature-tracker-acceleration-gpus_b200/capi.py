@@ -20,6 +20,7 @@ KLT_MAX_ITERATIONS = -3
 KLT_OOB = -4
 KLT_LARGE_RESIDUE = -5
 KLT_B200_FB_INCONSISTENT = -6      # include/klt_b200.h: rejected by the forward-backward check
+KLT_B200_MOTION_OUTLIER = -7       # include/klt_b200.h: rejected by the global motion check
 
 STATUS_NAMES = {
     0: "TRACKED", -1: "NOT_FOUND", -2: "SMALL_DET", -3: "MAX_ITERATIONS",

@@ -63,6 +63,12 @@ klt_tc_state *klt_state_get(KLT_TrackingContext tc)
     free(s);
     KLTError("(KLT/B200) KLT_B200_FB_MAX_ERROR = %s is not a number of pixels", e);
   }
+  e = getenv("KLT_B200_MOTION_MAX_ERROR");
+  s->motion_max_error = e ? strtof(e, NULL) : 0.0f;
+  if (isnan(s->motion_max_error)) {
+    free(s);
+    KLTError("(KLT/B200) KLT_B200_MOTION_MAX_ERROR = %s is not a number of pixels", e);
+  }
   e = getenv("KLT_B200_PREDICT");
   s->predict = KLT_B200_PREDICT_NONE;
   if (e && strcmp(e, "velocity") == 0) s->predict = KLT_B200_PREDICT_VELOCITY;
@@ -175,6 +181,43 @@ void KLTB200PredictionResult(KLT_TrackingContext tc, int n, float *gx, float *gy
     KLTError("(KLTB200PredictionResult) no tracking call on this context ran with prediction");
   if (klt_dev_prediction_results(s->dev, n, gx, gy, source) != 0)
     KLTError("(KLTB200PredictionResult) %s", klt_dev_error(s->dev));
+}
+
+/* a setting of the tracking calls only, like the forward-backward check */
+void KLTB200SetMotionCheck(KLT_TrackingContext tc, float max_error, int hypotheses)
+{
+  klt_tc_state *s;
+  if (isnan(max_error)) KLTError("(KLTB200SetMotionCheck) max_error is NaN");
+  if (hypotheses < 0 || hypotheses > 65536)
+    KLTError("(KLTB200SetMotionCheck) %d hypotheses (1 .. 65536, 0: 1024)", hypotheses);
+  s = klt_state_get(tc);
+  s->motion_max_error = max_error;
+  s->motion_hypotheses = hypotheses;
+}
+
+float KLTB200GetMotionCheck(KLT_TrackingContext tc, int *hypotheses)
+{
+  klt_tc_state *s = klt_state_get(tc);
+  if (hypotheses) *hypotheses = s->motion_hypotheses == 0 ? 1024 : s->motion_hypotheses;
+  return s->motion_max_error;
+}
+
+void KLTB200MotionResult(KLT_TrackingContext tc, int n, float *err)
+{
+  klt_tc_state *s = klt_state_find(tc);
+  if (s == NULL || s->dev == NULL)
+    KLTError("(KLTB200MotionResult) no tracking call on this context ran the check");
+  if (klt_dev_motion_results(s->dev, n, err) != 0)
+    KLTError("(KLTB200MotionResult) %s", klt_dev_error(s->dev));
+}
+
+void KLTB200MotionModels(KLT_TrackingContext tc, int count, KLT_B200_MotionModel *out)
+{
+  klt_tc_state *s = klt_state_find(tc);
+  if (s == NULL || s->dev == NULL)
+    KLTError("(KLTB200MotionModels) no tracking call on this context ran the check");
+  if (klt_dev_motion_models(s->dev, count, (klt_dev_motion_model *)out) != 0)
+    KLTError("(KLTB200MotionModels) %s", klt_dev_error(s->dev));
 }
 klt_dev *KLTB200Device(KLT_TrackingContext tc) { return klt_state_device(klt_state_get(tc)); }
 int KLTB200LastSlot(KLT_TrackingContext tc)

@@ -1299,6 +1299,7 @@ track_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
 #include "klt_track_fast.cuh"
 
 #include "klt_affine.cuh"
+#include "klt_motion.cuh"
 
 // ---------------------------------------------------------------------------
 // host side of the C-ABI
@@ -1306,12 +1307,13 @@ track_kernel(PyrView p1, PyrView p2, TrackArgs a, int n, FeatIO io,
 // kernel classes, for launch accounting and per-kernel event timing
 enum KernelId {
   KID_SMOOTH_U8 = 0, KID_GRAD, KID_PYRDOWN, KID_TRACK, KID_MINEIG, KID_SORT, KID_STAMP,
-  KID_ENFORCE, KID_GENERIC_H, KID_GENERIC_V, KID_U8_TO_F32, KID_L0_FUSED, KID_LEVEL_FUSED, KID_LEVEL_FUSED_L2, KID_LEVEL_FUSED_L3, KID_TRACK_FAST, KID_TRACK7W, KID_AFFINE, KID_FILTER, KID_COPY_H2D, KID_COPY_D2H, KID_COUNT
+  KID_ENFORCE, KID_GENERIC_H, KID_GENERIC_V, KID_U8_TO_F32, KID_L0_FUSED, KID_LEVEL_FUSED, KID_LEVEL_FUSED_L2, KID_LEVEL_FUSED_L3, KID_TRACK_FAST, KID_TRACK7W, KID_AFFINE, KID_FILTER, KID_MOTION_PREP, KID_MOTION_SCORE, KID_MOTION_REFINE, KID_COPY_H2D, KID_COPY_D2H, KID_COUNT
 };
 static const char* const kKernelNames[KID_COUNT] = {
   "smooth_u8_tile", "grad_tile", "pyrdown_tile", "track_kernel", "mineig_kernel",
   "cub_radix_sort", "stamp_existing_kernel", "enforce_mindist_kernel",
   "conv_h_generic", "conv_v_generic", "u8_to_f32_kernel", "l0_fused_kernel", "level_fused_kernel[level 1]", "level_fused_kernel[level 2]", "level_fused_kernel[level 3+]", "track_fast_kernel", "track7w_kernel", "affine_check_kernel", "cub_select_uncovered",
+  "motion_prep_kernel", "motion_score_kernel", "motion_refine_kernel",
   "copy_h2d", "copy_d2h"          // not kernels: timed in profiling mode, never counted as launches
 };
 static constexpr int PROF_POOL = 2048;     // event pairs in flight before folding
@@ -1383,8 +1385,11 @@ struct klt_dev {
   cudaEvent_t ev_feat; int feat_pending;   // feature upload queued on the copy stream
   // ... or not queued yet: it goes BEHIND the bands of the frame that is built next (feat_flush)
   int feat_deferred; void* feat_def_dst; const void* feat_def_src; size_t feat_def_bytes;
-  // affine consistency check (klt_dev_affine_*): per-feature state + templates, positions before tracking
-  AffState* d_aff_st; AffState* h_aff_st; float* d_aff_tmpl; float* d_x0; int aff_cap, aff_tsz, aff_x0_cap;
+  // affine consistency check (klt_dev_affine_*): per-feature state + templates
+  AffState* d_aff_st; AffState* h_aff_st; float* d_aff_tmpl; int aff_cap, aff_tsz;
+  // x | y | val before the tracker (stride x0_cap), read by the affine and the global motion check;
+  // x0_kept: the copy for the next tracker is queued already (klt_dev_affine_begin / _keep_positions)
+  float* d_x0; int x0_cap, x0_kept;
   // ring of pinned feature snapshots (klt_dev_snapshot_*)
   unsigned char* snap_ring; size_t snap_bytes; int snap_depth, snap_events; cudaEvent_t ev_snap[KLT_SNAP_MAX];
   // selection
@@ -1421,7 +1426,16 @@ struct klt_dev {
   float* d_guess; float* h_guess; int guess_cap, guess_n, guess_slot;
   cudaEvent_t ev_guess[2]; int guess_busy[2];
   PredArgs pred;                // (of the tracker being launched)
+  // global motion check: correspondences {x0, y0, x1, y1} and their feature indices (motion_cap
+  // each), per-feature err of the last tracking call that ran it (motion_n >= 0), hypothesis state
+  // (MotionHyp, hyp_cap hypotheses) and a ring of KLT_MOTION_RING model records: the next one goes
+  // to ring_next, ring_n of them belong to the calls since the last call without the check
+  float4* d_mcorr; int* d_mcidx; float* d_merr; int motion_cap, motion_n;
+  int* d_mhyp; int hyp_cap, motion_hyps;
+  MotionModelRec* d_mring; int ring_next, ring_n;
 };
+static constexpr int KLT_MOTION_RING = 4096;
+static_assert(sizeof(MotionModelRec) == sizeof(klt_dev_motion_model), "motion model layout");
 
 // RAII around one kernel launch: counts it and, in profiling mode, brackets it
 // with CUDA events on the context stream.
@@ -1579,6 +1593,7 @@ extern "C" int klt_dev_create(int device, klt_dev** out) {
   c->tstream = c->stream;
   c->fb_n = -1;
   c->pred_n = -1; c->guess_n = -1;
+  c->motion_n = -1;
   e = cudaMalloc(&c->d_live, sizeof(unsigned long long));
   if (e == cudaSuccess) e = cudaMemsetAsync(c->d_live, 0, sizeof(unsigned long long), c->stream);
   c->pdl = getenv("KLT_B200_PDL") ? atoi(getenv("KLT_B200_PDL")) : 1;
@@ -1666,6 +1681,8 @@ extern "C" void klt_dev_destroy(klt_dev* d) {
   cudaFreeHost(d->h_frame);
   cudaFreeHost(d->snap_ring);
   cudaFree(d->d_aff_st); cudaFreeHost(d->h_aff_st); cudaFree(d->d_aff_tmpl); cudaFree(d->d_x0);
+  guarded_free(d, d->d_mcorr); guarded_free(d, d->d_mcidx); guarded_free(d, d->d_merr);
+  guarded_free(d, d->d_mhyp); guarded_free(d, d->d_mring);
   for (int i = 0; i < d->snap_events; ++i) cudaEventDestroy(d->ev_snap[i]);
   cudaStreamDestroy(d->cstream);
   cudaStreamDestroy(d->stream);
@@ -2771,6 +2788,16 @@ static void make_view(const PyrSet& S, int L, PyrView* v) {
   }
 }
 
+// the buffer of the positions before the tracker (d_x0), as large as the feature arrays
+static int ensure_x0(klt_dev* d) {
+  if (d->x0_cap >= d->feat_cap) return 0;
+  if (sync_all(d)) return fail(d, "stream synchronisation failed");
+  cudaFree(d->d_x0); d->d_x0 = nullptr; d->x0_cap = 0;
+  CU(cudaMalloc(&d->d_x0, (size_t)d->feat_cap * 12));
+  d->x0_cap = d->feat_cap;
+  return 0;
+}
+
 // where the tracker records its results: the device arrays (resident pipelines) or, for the
 // synchronous API, straight into the pinned host staging area (posted writes over PCIe, no D2H copy)
 static FeatIO feat_io(klt_dev* d) {
@@ -2859,6 +2886,96 @@ static void fill_track_args(const klt_dev* d, const klt_dev_track_params* p, Tra
   { static int keep = getenv("KLT_TRACK_L2_KEEP") ? atoi(getenv("KLT_TRACK_L2_KEEP")) : 1; a->l2_keep = keep; }
 }
 extern "C" void klt_dev_disable_track7w(klt_dev* d, int on) { d->no_track7w = on; }
+
+// ---- global motion check (klt_motion.cuh) ----------------------------------------------------
+static int ensure_motion(klt_dev* d, int n, int hyps) {
+  if (!d->d_mring) {
+    CU(guarded_malloc(d, &d->d_mring, (size_t)KLT_MOTION_RING * sizeof(MotionModelRec)));
+    d->ring_next = 0; d->ring_n = 0;
+  }
+  if (d->motion_cap < n) {
+    if (sync_all(d)) return fail(d, "stream synchronisation failed");
+    guarded_free(d, d->d_mcorr); guarded_free(d, d->d_mcidx); guarded_free(d, d->d_merr);
+    d->d_mcorr = nullptr; d->d_mcidx = nullptr; d->d_merr = nullptr; d->motion_cap = 0;
+    const int cap = (n + 1023) / 1024 * 1024;
+    CU(guarded_malloc(d, &d->d_mcorr, (size_t)cap * sizeof(float4)));
+    CU(guarded_malloc(d, &d->d_mcidx, (size_t)cap * sizeof(int)));
+    CU(guarded_malloc(d, &d->d_merr, (size_t)cap * sizeof(float)));
+    d->motion_cap = cap;
+  }
+  if (d->hyp_cap < hyps) {
+    if (sync_all(d)) return fail(d, "stream synchronisation failed");
+    guarded_free(d, d->d_mhyp); d->d_mhyp = nullptr; d->hyp_cap = 0;
+    const int cap = (hyps + 1023) / 1024 * 1024;
+    CU(guarded_malloc(d, &d->d_mhyp, (size_t)(1 + 10 * (size_t)cap) * sizeof(int)));
+    d->hyp_cap = cap;
+  }
+  return 0;
+}
+
+// the three launches of the check behind the tracker of a call on n features; the model record goes
+// to ring slot ring_next
+static int motion_launch(klt_dev* d, const klt_dev_track_params* p, int n) {
+  MotionGeo g;
+  g.cx = 0.5 * d->W; g.cy = 0.5 * d->H;
+  g.s = 2.0 / (d->W > d->H ? d->W : d->H);
+  const float e2 = p->motion_max_error * p->motion_max_error;
+  const int hyps = d->motion_hyps;
+  MotionHyp hyp;
+  hyp.base = d->d_mhyp; hyp.cap = d->hyp_cap;
+  { Launch l(d, KID_MOTION_PREP, d->tstream);
+    motion_prep_kernel<<<1, MOTION_PREP_THREADS, 0, d->tstream>>>(n, d->feat_cap, d->d_x0, d->d_x, d->d_y, d->d_val,
+                                                                 d->d_mcorr, d->d_mcidx, d->d_merr, hyp, hyps); }
+  { Launch l(d, KID_MOTION_SCORE, d->tstream);
+    const dim3 grid((hyps + MOTION_SCORE_THREADS - 1) / MOTION_SCORE_THREADS, n > 0 ? (n + MOTION_CHUNK - 1) / MOTION_CHUNK : 1);
+    motion_score_kernel<<<grid, MOTION_SCORE_THREADS, 0, d->tstream>>>(d->d_mcorr, hyp, hyps, e2, g); }
+  { Launch l(d, KID_MOTION_REFINE, d->tstream);
+    motion_refine_kernel<<<1, MOTION_REFINE_THREADS, 0, d->tstream>>>(d->d_mcorr, d->d_mcidx, hyp, hyps, e2, g,
+                                                                      d->d_x, d->d_y, d->d_val, d->d_merr,
+                                                                      d->d_mring + d->ring_next); }
+  CU(cudaGetLastError());
+  d->ring_next = (d->ring_next + 1) % KLT_MOTION_RING;
+  if (d->ring_n < KLT_MOTION_RING) d->ring_n += 1;
+  return 0;
+}
+
+extern "C" int klt_dev_motion_results(klt_dev* d, int n, float* err) {
+  CU(cudaSetDevice(d->device));
+  if (d->motion_n < 0) return fail(d, "motion_results: the last tracking call did not run the global motion check");
+  if (n != d->motion_n) return fail(d, "motion_results: %d features requested, the last tracking call had %d", n, d->motion_n);
+  if (n == 0) return 0;
+  if (!err) return fail(d, "motion_results: NULL array");
+  CU(cudaMemcpyAsync(err, d->d_merr, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, d->tstream));
+  CU(cudaStreamSynchronize(d->tstream));
+  return 0;
+}
+
+extern "C" int klt_dev_motion_models(klt_dev* d, int count, klt_dev_motion_model* out) {
+  CU(cudaSetDevice(d->device));
+  if (count < 0 || count > d->ring_n)
+    return fail(d, "motion_models: %d models requested, %d recorded since the last call without the check", count, d->ring_n);
+  if (count == 0) return 0;
+  if (!out) return fail(d, "motion_models: NULL array");
+  const int first = (d->ring_next - count + KLT_MOTION_RING) % KLT_MOTION_RING;
+  const int head = count < KLT_MOTION_RING - first ? count : KLT_MOTION_RING - first;   // up to the ring's end
+  CU(cudaMemcpyAsync(out, d->d_mring + first, (size_t)head * sizeof(MotionModelRec), cudaMemcpyDeviceToHost, d->tstream));
+  if (head < count)
+    CU(cudaMemcpyAsync(out + head, d->d_mring, (size_t)(count - head) * sizeof(MotionModelRec), cudaMemcpyDeviceToHost, d->tstream));
+  CU(cudaStreamSynchronize(d->tstream));
+  return 0;
+}
+
+extern "C" int klt_dev_motion_counts(klt_dev* d, int hyps, int* m, int* counts) {
+  CU(cudaSetDevice(d->device));
+  if (d->motion_n < 0) return fail(d, "motion_counts: the last tracking call did not run the global motion check");
+  if (hyps != d->motion_hyps) return fail(d, "motion_counts: %d hypotheses requested, the last call had %d", hyps, d->motion_hyps);
+  if (!m || !counts) return fail(d, "motion_counts: NULL array");
+  CU(cudaMemcpyAsync(m, d->d_mhyp, sizeof(int), cudaMemcpyDeviceToHost, d->tstream));
+  CU(cudaMemcpyAsync(counts, d->d_mhyp + 1, (size_t)hyps * sizeof(int), cudaMemcpyDeviceToHost, d->tstream));
+  CU(cudaStreamSynchronize(d->tstream));
+  return 0;
+}
+
 extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
                                       const klt_dev_track_params* p) {
   CU(cudaSetDevice(d->device));
@@ -2878,7 +2995,20 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
   const bool pred = p->predict != 0 || guess_n >= 0;
   d->pred_n = pred ? n : -1;
   if (!pred) d->vel_n = 0;                           // this call leaves the velocity records behind
-  if (n == 0) return 0;
+  const bool motion = p->motion_max_error > 0.0f;
+  const int x0_kept = d->x0_kept;                    // (the affine check's copy serves this call only)
+  d->x0_kept = 0;
+  d->motion_n = motion ? n : -1;
+  if (!motion) d->ring_n = 0;                        // the model history is of consecutive checked calls
+  if (motion) {
+    const int hyps = p->motion_hypotheses == 0 ? 1024 : p->motion_hypotheses;
+    if (hyps < 1 || hyps > 65536) return fail(d, "klt_dev_track: motion_hypotheses = %d (1 .. 65536, 0: 1024)", hyps);
+    if (d->feat_out_host == 2) return fail(d, "klt_dev_track: the global motion check needs the features on the device, not in record mode");
+    d->feat_out_host = 0;                            // the check rewrites the tracker's answers on the device
+    d->motion_hyps = hyps;
+    if (ensure_motion(d, n, hyps)) return 1;
+  }
+  if (n == 0) return motion ? motion_launch(d, p, 0) : 0;
   if (fb && d->fb_cap < n) {                         // the check's result records (klt_dev_fb_results)
     if (sync_all(d)) return fail(d, "stream synchronisation failed");
     guarded_free(d, d->d_fb); d->d_fb = nullptr; d->fb_cap = 0;
@@ -2905,6 +3035,10 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
   if (d->feat_pending) {                             // features uploaded on the copy stream
     CU(cudaStreamWaitEvent(d->tstream, d->ev_feat, 0));
     d->feat_pending = 0;
+  }
+  if (motion && !x0_kept) {                          // the start positions of the correspondences
+    if (ensure_x0(d)) return 1;
+    CU(cudaMemcpyAsync(d->d_x0, d->d_x, (size_t)d->feat_cap * 12, cudaMemcpyDeviceToDevice, d->tstream));
   }
   if (d->overlap) {                                  // the pyramids are produced on the other stream
     const int sl[2] = {slot_prev, slot_cur};
@@ -2940,6 +3074,7 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
   if (rc) return rc;
   CU(cudaGetLastError());
   if (guess_n >= 0) CU(cudaEventRecord(d->ev_guess[d->guess_slot], d->tstream));   // the slot's last reader
+  if (motion && motion_launch(d, p, n)) return 1;
   if (d->overlap) {
     CU(cudaEventRecord(d->ev_read[slot_prev], d->tstream));
     CU(cudaEventRecord(d->ev_read[slot_cur], d->tstream));
@@ -3064,12 +3199,7 @@ extern "C" int klt_dev_affine_begin(klt_dev* d, int n, const klt_dev_affine_para
     CU(cudaMalloc(&d->d_aff_tmpl, (size_t)cap * 3 * tsz * sizeof(float)));
     d->aff_cap = cap; d->aff_tsz = tsz;
   }
-  if (d->aff_x0_cap < d->feat_cap) {
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    cudaFree(d->d_x0); d->d_x0 = nullptr; d->aff_x0_cap = 0;
-    CU(cudaMalloc(&d->d_x0, (size_t)d->feat_cap * 12));
-    d->aff_x0_cap = d->feat_cap;
-  }
+  if (ensure_x0(d)) return 1;
   if (d->feat_out_host == 2) return fail(d, "affine_begin: record-mode features (use the staging area)");
   d->feat_out_host = 0;                              // the check needs the tracker's answers on the device
   if (feat_flush(d)) return 1;
@@ -3078,6 +3208,7 @@ extern "C" int klt_dev_affine_begin(klt_dev* d, int n, const klt_dev_affine_para
     d->feat_pending = 0;
   }
   CU(cudaMemcpyAsync(d->d_x0, d->d_x, (size_t)d->feat_cap * 12, cudaMemcpyDeviceToDevice, d->tstream));
+  d->x0_kept = 1;
   *staging = reinterpret_cast<klt_dev_affine_state*>(d->h_aff_st);
   return 0;
 }
@@ -3113,8 +3244,9 @@ extern "C" int klt_dev_affine_upload_states(klt_dev* d, int n) {
 }
 extern "C" int klt_dev_affine_keep_positions(klt_dev* d) {
   CU(cudaSetDevice(d->device));
-  if (!d->d_x0 || d->aff_x0_cap < d->feat_cap) return fail(d, "affine_keep_positions without affine_begin");
+  if (!d->d_x0 || d->x0_cap < d->feat_cap) return fail(d, "affine_keep_positions without affine_begin");
   CU(cudaMemcpyAsync(d->d_x0, d->d_x, (size_t)d->feat_cap * 12, cudaMemcpyDeviceToDevice, d->tstream));
+  d->x0_kept = 1;
   return 0;
 }
 extern "C" int klt_dev_affine_check_resident(klt_dev* d, int slot_prev, int slot_cur, const klt_dev_track_params* tp,

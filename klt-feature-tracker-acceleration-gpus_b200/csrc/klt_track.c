@@ -51,6 +51,8 @@ static void fill_track_params(KLT_TrackingContext tc, const klt_tc_state *s, klt
   p->lighting_insensitive = tc->lighting_insensitive ? 1 : 0;
   p->fb_max_error = s->fb_max_error > 0.0f ? s->fb_max_error : 0.0f;
   p->predict = s->predict;
+  p->motion_max_error = s->motion_max_error > 0.0f ? s->motion_max_error : 0.0f;
+  p->motion_hypotheses = s->motion_hypotheses;
 }
 
 /* explicit guesses (KLTB200SetGuesses or klt_dev_set_guesses: one queue, on the device) are consumed
@@ -286,7 +288,8 @@ static void track_common(KLT_TrackingContext tc, const KLT_PixelType *img1,
    * packed into the staging area first (a few microseconds) for the same order on the copy stream. */
   slot_prev = prepare_previous(tc, s, img1, on_device, pitch, ncols, nrows);
   slot_cur = (slot_prev + 1) % KLT_DEV_SLOTS;
-  records = n > 0 && !affine && klt_list_is_pinned(fl) && fl->feature[n - 1] == fl->feature[0] + (n - 1);
+  /* (the global motion check rewrites the tracker's answers on the device: no record mode) */
+  records = n > 0 && !affine && !(s->motion_max_error > 0.0f) && klt_list_is_pinned(fl) && fl->feature[n - 1] == fl->feature[0] + (n - 1);
   if (records) {
     DEVCALL(s, klt_dev_features_commit_records(dev, n, fl->feature[0], sizeof(KLT_FeatureRec)));
   } else {

@@ -36,7 +36,12 @@ class TrackParams(C.Structure):       # klt_dev_track_params
                 ("min_determinant", C.c_float), ("min_displacement", C.c_float),
                 ("max_residue", C.c_float), ("borderx", C.c_int), ("bordery", C.c_int),
                 ("exact", C.c_int), ("lighting_insensitive", C.c_int), ("fb_max_error", C.c_float),
-                ("predict", C.c_int)]
+                ("predict", C.c_int), ("motion_max_error", C.c_float), ("motion_hypotheses", C.c_int)]
+
+
+class MotionModel(C.Structure):       # klt_dev_motion_model / KLT_B200_MotionModel
+    _fields_ = [("H", C.c_float * 9), ("valid", C.c_int), ("tracked", C.c_int), ("inliers", C.c_int),
+                ("hypothesis", C.c_int)]
 
 
 class SelectParams(C.Structure):      # klt_dev_select_params
@@ -114,6 +119,9 @@ DEV_API = {
     "klt_dev_set_guesses": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
     "klt_dev_guesses_pending": (C.c_int, [C.c_void_p]),
     "klt_dev_prediction_results": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "klt_dev_motion_results": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "klt_dev_motion_models": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "klt_dev_motion_counts": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     # include/klt_b200.h
     "KLTB200SetDevice": (None, [_TC, C.c_int]),
     "KLTB200SetExact": (None, [_TC, C.c_int]),
@@ -125,6 +133,10 @@ DEV_API = {
     "KLTB200GetPrediction": (C.c_int, [_TC]),
     "KLTB200SetGuesses": (None, [_TC, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
     "KLTB200PredictionResult": (None, [_TC, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "KLTB200SetMotionCheck": (None, [_TC, C.c_float, C.c_int]),
+    "KLTB200GetMotionCheck": (C.c_float, [_TC, C.POINTER(C.c_int)]),
+    "KLTB200MotionResult": (None, [_TC, C.c_int, C.c_void_p]),
+    "KLTB200MotionModels": (None, [_TC, C.c_int, C.c_void_p]),
     "KLTB200Device": (C.c_void_p, [_TC]),
     "KLTB200LastSlot": (C.c_int, [_TC]),
     "KLTTrackFeaturesDevice": (None, [_TC, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, _FL]),
@@ -217,11 +229,51 @@ class B200Library(capi.KLTLibrary):
         self.dev_check(dev, self.lib.klt_dev_read_level(dev, slot, which, level, out))
         return out
 
-    def track_params(self, tc, exact=0, fb_max_error=0.0, predict=0) -> TrackParams:
+    def track_params(self, tc, exact=0, fb_max_error=0.0, predict=0, motion_max_error=0.0,
+                     motion_hypotheses=0) -> TrackParams:
         t = tc.contents
         return TrackParams(t.window_width, t.window_height, t.step_factor, t.max_iterations,
                            t.min_determinant, t.min_displacement, t.max_residue,
-                           t.borderx, t.bordery, exact, t.lighting_insensitive, fb_max_error, predict)
+                           t.borderx, t.bordery, exact, t.lighting_insensitive, fb_max_error, predict,
+                           motion_max_error, motion_hypotheses)
+
+    @staticmethod
+    def _models(models) -> dict:
+        """{H: (count, 3, 3) float32, valid, tracked, inliers, hypothesis: (count,) int32}"""
+        raw = np.frombuffer(models, np.uint8).reshape(len(models), C.sizeof(MotionModel))
+        return {"H": raw[:, :36].copy().view(np.float32).reshape(-1, 3, 3),
+                **{k: raw[:, 36 + 4 * i:40 + 4 * i].copy().view(np.int32).ravel()
+                   for i, k in enumerate(("valid", "tracked", "inliers", "hypothesis"))}}
+
+    def motion_result(self, tc, n):
+        """KLTB200MotionResult: per-feature reprojection distance of the last tracking call on tc"""
+        err = np.empty(n, np.float32)
+        self.lib.KLTB200MotionResult(tc, n, err.ctypes.data)
+        return err
+
+    def motion_models(self, tc, count):
+        """KLTB200MotionModels: the models of the last `count` checked calls on tc, oldest first"""
+        out = (MotionModel * count)()
+        self.lib.KLTB200MotionModels(tc, count, C.cast(out, C.c_void_p))
+        return self._models(out)
+
+    def dev_motion_results(self, dev, n):
+        """klt_dev_motion_results: per-feature reprojection distance of the last klt_dev_track* call"""
+        err = np.empty(n, np.float32)
+        self.dev_check(dev, self.lib.klt_dev_motion_results(dev, n, err.ctypes.data))
+        return err
+
+    def dev_motion_models(self, dev, count):
+        """klt_dev_motion_models: the models of the last `count` checked klt_dev_track* calls"""
+        out = (MotionModel * count)()
+        self.dev_check(dev, self.lib.klt_dev_motion_models(dev, count, C.cast(out, C.c_void_p)))
+        return self._models(out)
+
+    def dev_motion_counts(self, dev, hyps):
+        """klt_dev_motion_counts: (m, per-hypothesis inlier counts, -1: no model) of the last checked call"""
+        m, counts = C.c_int(0), np.empty(hyps, np.int32)
+        self.dev_check(dev, self.lib.klt_dev_motion_counts(dev, hyps, C.byref(m), counts.ctypes.data))
+        return m.value, counts
 
     def set_guesses(self, tc, gx, gy, on_device=False):
         """KLTB200SetGuesses for the next tracking call on tc: float32 host arrays, or with on_device
