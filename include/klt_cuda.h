@@ -293,7 +293,8 @@ void klt_dev_force_generic(klt_dev *d, int on);
 void klt_dev_disable_fused(klt_dev *d, int on);
 /* Debug aid (compute-sanitizer's stand-in): guard mode (env KLT_B200_GUARD=1 or klt_dev_set_guard
  * before the next build) puts a 4 KB canary band in front of every plane of the pyramid arena and
- * behind the last one; klt_dev_check_guards synchronises and counts the canary words a kernel has
+ * behind the last one, and on either side of each device buffer the context grows from then on;
+ * klt_dev_check_guards synchronises and counts the canary words a kernel has
  * damaged (0 = no store left its plane) and names the first damaged band. */
 void klt_dev_set_guard(klt_dev *d, int on);
 int klt_dev_check_guards(klt_dev *d, long long *damaged_words, int *first_band);

@@ -1324,6 +1324,7 @@ static constexpr int KLT_SNAP_MAX = 64;
 static constexpr int KLT_HOST_REGS = 32; // pageable frame buffers remembered per context
 static constexpr int KLT_TILE_QUEUES = 16;
 static_assert(KLT_DEV_MAX_LEVELS <= KLT_TILE_QUEUES, "one tile queue per pyramid level");
+static constexpr int KLT_GUARDED_MAX = 48;   // guarded device buffers: a context holds 25 at most
 struct Level {
   int w, h, pitch;           // pitch in floats
   float *img, *gx, *gy;
@@ -1357,7 +1358,7 @@ struct klt_dev {
   float* arena;
   size_t arena_floats;
   int guard;                 // debug: canary bands between the planes of the arena (klt_dev_set_guard)
-  struct Guarded { void* user; size_t bytes; } guarded[24]; int nguarded;   // ... and around the selection / feature buffers
+  struct Guarded { void* user; size_t bytes; } guarded[KLT_GUARDED_MAX]; int nguarded;   // ... and around every grown device buffer
   float* tmp;                // generic path: horizontal-pass result, W*H floats
   unsigned char* frame;      // u8 staging of the frame being built (== frame_buf[frame_idx]), row pitch frame_pitch
   unsigned char* frame_buf[2]; int frame_idx;   // two buffers: frame k+1 goes up while level 0 of frame k is still reading
@@ -1620,21 +1621,21 @@ extern "C" int klt_dev_create(int device, klt_dev** out) {
 
 static constexpr size_t KLT_GUARD_FLOATS = 1024;      // 4 KB: keeps every plane 128-byte aligned
 static constexpr int KLT_GUARD_BYTE = 0xA5;
-// cudaMalloc / cudaFree with a canary band on either side in guard mode (the selection and feature buffers)
-static cudaError_t guarded_malloc(klt_dev* d, void** out, size_t bytes) {
-  if (!d->guard || d->nguarded >= (int)(sizeof(d->guarded) / sizeof(d->guarded[0]))) return cudaMalloc(out, bytes);
+// cudaMalloc / cudaFree with a canary band on either side in guard mode (klt_dev_check_guards)
+static int guarded_malloc(klt_dev* d, void** out, size_t bytes) {
+  if (!d->guard) { CU(cudaMalloc(out, bytes)); return 0; }
+  if (d->nguarded == KLT_GUARDED_MAX) return fail(d, "guard mode: more than %d device buffers", KLT_GUARDED_MAX);
   const size_t gb = KLT_GUARD_FLOATS * sizeof(float), padded = (bytes + 255) / 256 * 256;
   unsigned char* base = nullptr;
-  cudaError_t e = cudaMalloc(&base, padded + 2 * gb);
-  if (e != cudaSuccess) return e;
-  e = cudaMemset(base, KLT_GUARD_BYTE, padded + 2 * gb);
-  if (e != cudaSuccess) { cudaFree(base); return e; }
+  CU(cudaMalloc(&base, padded + 2 * gb));
+  const cudaError_t e = cudaMemset(base, KLT_GUARD_BYTE, padded + 2 * gb);
+  if (e != cudaSuccess) { cudaFree(base); return fail(d, "guard band: %s", cudaGetErrorString(e)); }
   *out = base + gb;
   d->guarded[d->nguarded].user = base + gb; d->guarded[d->nguarded].bytes = bytes; d->nguarded += 1;
-  return cudaSuccess;
+  return 0;
 }
 template <typename T>
-static cudaError_t guarded_malloc(klt_dev* d, T** out, size_t bytes) { return guarded_malloc(d, reinterpret_cast<void**>(out), bytes); }
+static int guarded_malloc(klt_dev* d, T** out, size_t bytes) { return guarded_malloc(d, reinterpret_cast<void**>(out), bytes); }
 static void guarded_free(klt_dev* d, void* p) {
   if (!p) return;
   for (int i = 0; i < d->nguarded; ++i)
@@ -1645,6 +1646,37 @@ static void guarded_free(klt_dev* d, void* p) {
     }
   cudaFree(p);
 }
+template <typename T> static void release(klt_dev* d, T*& p) { guarded_free(d, p); p = nullptr; }
+template <typename T> static void release_pinned(T*& p) { cudaFreeHost(p); p = nullptr; }
+
+// One buffer of a group that grow() re-makes together: where its pointer lives and its size at the
+// new capacity; device memory (guarded in guard mode) or pinned host staging.
+struct GrowBuf { void** p; size_t bytes; bool pinned; };
+template <typename T> static GrowBuf device_buf(T** p, size_t bytes) { return {reinterpret_cast<void**>(p), bytes, false}; }
+template <typename T> static GrowBuf pinned_buf(T** p, size_t bytes) { return {reinterpret_cast<void**>(p), bytes, true}; }
+
+// Makes the buffers that share the capacity *cap hold `need` (in whatever unit the caller counts).
+// Nothing happens when *cap >= need.  Otherwise every stream is drained, since queued kernels and
+// copies may still use the old buffers, these are freed and allocated anew, and *cap = need.  A
+// capacity never shrinks, so calls no larger than an earlier one never drain.  *cap is 0 after a
+// failure, so the next call tries again.
+template <typename C, typename... B>
+static int grow(klt_dev* d, C* cap, size_t need, B... bufs) {
+  if ((size_t)*cap >= need) return 0;
+  if (sync_all(d)) return fail(d, "stream synchronisation failed");
+  const GrowBuf group[] = {bufs...};
+  *cap = 0;
+  for (const GrowBuf& b : group) b.pinned ? release_pinned(*b.p) : release(d, *b.p);
+  for (const GrowBuf& b : group) {
+    if (b.pinned) CU(cudaMallocHost(b.p, b.bytes));
+    else if (guarded_malloc(d, b.p, b.bytes)) return 1;
+  }
+  *cap = (C)need;
+  return 0;
+}
+// the capacity of the per-feature (and per-hypothesis) buffers: n rounded up to a multiple of 1024
+static size_t round_1024(int n) { return (size_t)(n + 1023) / 1024 * 1024; }
+
 static void free_geometry(klt_dev* d) {
   cudaFree(d->arena); d->arena = nullptr;
   cudaFree(d->tmp); d->tmp = nullptr;
@@ -1658,31 +1690,28 @@ extern "C" void klt_dev_destroy(klt_dev* d) {
   sync_all(d);
   klt_dev_forget_host_frames(d);
   free_geometry(d);
-  cudaFree(d->frame_buf[0]); cudaFree(d->frame_buf[1]);
-  guarded_free(d, d->d_x);
-  guarded_free(d, d->d_fb);
-  guarded_free(d, d->d_vel); guarded_free(d, d->d_pred); guarded_free(d, d->d_guess); cudaFreeHost(d->h_guess);
+  release(d, d->frame_buf[0]); release(d, d->frame_buf[1]); release_pinned(d->h_frame);
+  release(d, d->d_x); release_pinned(d->h_x); release(d, d->d_rec); release(d, d->d_x0);
+  release_pinned(d->snap_ring);
+  release(d, d->d_aff_st); release_pinned(d->h_aff_st); release(d, d->d_aff_tmpl);
+  for (int i = 0; i < 2; ++i) { release(d, d->c_val[i]); release(d, d->c_idx[i]); }
+  release(d, d->rank_list); release(d, d->sel_state); release(d, d->cub_tmp);
+  release(d, d->fmap); release(d, d->open_slots);
+  release(d, d->d_fb);
+  release(d, d->d_vel); release(d, d->d_pred); release(d, d->d_guess); release_pinned(d->h_guess);
+  release(d, d->d_mcorr); release(d, d->d_mcidx); release(d, d->d_merr); release(d, d->d_mhyp); release(d, d->d_mring);
   for (int i = 0; i < 2; ++i) if (d->ev_guess[i]) cudaEventDestroy(d->ev_guess[i]);
-  cudaFreeHost(d->h_x);
-  for (int i = 0; i < 2; ++i) { guarded_free(d, d->c_val[i]); guarded_free(d, d->c_idx[i]); }
-  cudaFree(d->cub_tmp); guarded_free(d, d->fmap); guarded_free(d, d->open_slots); guarded_free(d, d->rank_list); guarded_free(d, d->sel_state);
   if (d->ev_made) { cudaEventDestroy(d->ev_a); cudaEventDestroy(d->ev_b); }
   if (d->prof_ev) { for (int i = 0; i < 2 * PROF_POOL; ++i) cudaEventDestroy(d->prof_ev[i]); free(d->prof_ev); free(d->prof_kid);
     cudaEventDestroy(d->ev_origin); free(d->trace_kid); free(d->trace_t0); free(d->trace_t1); }
   cudaFree(d->d_live);
   cudaFree(d->d_tile_ctr);
-  cudaFree(d->d_rec);
   for (int i = 0; i < KLT_DEV_SLOTS; ++i) { cudaEventDestroy(d->ev_built[i]); cudaEventDestroy(d->ev_read[i]); }
   cudaEventDestroy(d->ev_join);
   for (int i = 0; i < KLT_BAND_EVENTS; ++i) cudaEventDestroy(d->ev_band[i]);
   cudaEventDestroy(d->ev_frame_free[0]); cudaEventDestroy(d->ev_frame_free[1]);
   cudaEventDestroy(d->ev_feat);
   cudaEventDestroy(d->ev_stage_free);
-  cudaFreeHost(d->h_frame);
-  cudaFreeHost(d->snap_ring);
-  cudaFree(d->d_aff_st); cudaFreeHost(d->h_aff_st); cudaFree(d->d_aff_tmpl); cudaFree(d->d_x0);
-  guarded_free(d, d->d_mcorr); guarded_free(d, d->d_mcidx); guarded_free(d, d->d_merr);
-  guarded_free(d, d->d_mhyp); guarded_free(d, d->d_mring);
   for (int i = 0; i < d->snap_events; ++i) cudaEventDestroy(d->ev_snap[i]);
   cudaStreamDestroy(d->cstream);
   cudaStreamDestroy(d->stream);
@@ -1741,11 +1770,10 @@ extern "C" void klt_dev_set_guard(klt_dev* d, int on) {
   free_geometry(d);
   // the selection buffers are re-created on demand (the feature arrays keep their state: they are
   // guarded when they are allocated after this call)
-  for (int i = 0; i < 2; ++i) { guarded_free(d, d->c_val[i]); guarded_free(d, d->c_idx[i]); d->c_val[i] = nullptr; d->c_idx[i] = nullptr; }
-  guarded_free(d, d->rank_list); guarded_free(d, d->sel_state); d->rank_list = nullptr; d->sel_state = nullptr;
-  cudaFree(d->cub_tmp); d->cub_tmp = nullptr; d->cand_cap = 0;
-  guarded_free(d, d->fmap); d->fmap = nullptr; d->fmap_cap = 0;
-  guarded_free(d, d->open_slots); d->open_slots = nullptr; d->open_cap = 0;
+  for (int i = 0; i < 2; ++i) { release(d, d->c_val[i]); release(d, d->c_idx[i]); }
+  release(d, d->rank_list); release(d, d->sel_state); release(d, d->cub_tmp); d->cand_cap = 0;
+  release(d, d->fmap); d->fmap_cap = 0;
+  release(d, d->open_slots); d->open_cap = 0;
   d->guard = on ? 1 : 0;
 }
 extern "C" int klt_dev_check_guards(klt_dev* d, long long* damaged_words, int* first_band) {
@@ -1773,7 +1801,7 @@ extern "C" int klt_dev_check_guards(klt_dev* d, long long* damaged_words, int* f
       rc = check(lv.img - KLT_GUARD_FLOATS) || check(lv.gx - KLT_GUARD_FLOATS) || check(lv.gy - KLT_GUARD_FLOATS);
     }
   if (!rc && d->arena) rc = check(d->arena + d->arena_floats - KLT_GUARD_FLOATS);
-  // selection / feature buffers: band in front and band behind (from the first 256-byte boundary after the buffer)
+  // the grown buffers: band in front and band behind (from the first 256-byte boundary after the buffer)
   band = 1000;
   for (int i = 0; i < d->nguarded && !rc; ++i) {
     const unsigned char* u = static_cast<const unsigned char*>(d->guarded[i].user);
@@ -2375,13 +2403,7 @@ static int feed_enqueue_copies(klt_dev* d, BandFeed* f) {
   f->staged = d->stage_threads > 0 && pageable;
   d->last_staged = f->staged ? 1 : 0;
   if (f->staged) {
-    if (d->h_frame_cap < bytes) {
-      if (sync_all(d)) return fail(d, "stream synchronisation failed");
-      cudaFreeHost(d->h_frame); d->h_frame = nullptr; d->h_frame_cap = 0;
-      CU(cudaHostAlloc(&d->h_frame, bytes, cudaHostAllocDefault));
-      d->h_frame_cap = bytes;
-      d->stage_busy = 0;
-    }
+    if (grow(d, &d->h_frame_cap, bytes, pinned_buf(&d->h_frame, bytes))) return 1;
     if (d->stage_busy) { CU(cudaEventSynchronize(d->ev_stage_free)); d->stage_busy = 0; }
     return 0;                   // bands are staged and queued one at a time, each followed by its kernels
   }
@@ -2556,13 +2578,7 @@ extern "C" int klt_dev_build(klt_dev* d, int slot, const unsigned char* img, int
   if (!img_is_device) {
     const int fp = (W + 15) / 16 * 16;          // TMA needs a 16 B multiple row pitch
     const size_t bytes = (size_t)fp * H;
-    if (d->frame_cap < bytes) {
-      if (sync_all(d)) return fail(d, "stream synchronisation failed");
-      for (int i = 0; i < 2; ++i) { cudaFree(d->frame_buf[i]); d->frame_buf[i] = nullptr; d->frame_busy[i] = 0; }
-      d->frame = nullptr; d->frame_cap = 0;
-      for (int i = 0; i < 2; ++i) CU(cudaMalloc(&d->frame_buf[i], bytes));
-      d->frame_cap = bytes;
-    }
+    if (grow(d, &d->frame_cap, bytes, device_buf(&d->frame_buf[0], bytes), device_buf(&d->frame_buf[1], bytes))) return 1;
     d->frame_idx ^= 1;                          // the other buffer may still be read by the previous build
     d->frame = d->frame_buf[d->frame_idx];
     // uploaded inside build_impl: band by band on the copy stream when every level runs fused
@@ -2617,19 +2633,12 @@ extern "C" int klt_dev_read_level(klt_dev* d, int slot, int which, int level, fl
 // ---- features --------------------------------------------------------------------
 // device and pinned-host staging hold x | y | val back to back (one copy each way)
 static int ensure_features(klt_dev* d, int n) {
-  if (n <= d->feat_cap) return 0;
-  if (sync_all(d)) return fail(d, "stream synchronisation failed");
-  guarded_free(d, d->d_x);
-  cudaFreeHost(d->h_x);
-  d->d_x = d->d_y = nullptr; d->d_val = nullptr; d->h_x = d->h_y = nullptr; d->h_val = nullptr;
-  d->feat_cap = 0;
-  const int cap = (n + 1023) / 1024 * 1024;
-  CU(guarded_malloc(d, &d->d_x, (size_t)cap * 12));
-  CU(cudaMallocHost(&d->h_x, (size_t)cap * 12));
+  const size_t want = round_1024(n);
+  const int rc = grow(d, &d->feat_cap, want, device_buf(&d->d_x, want * 12), pinned_buf(&d->h_x, want * 12));
+  const int cap = d->feat_cap;                       // (0 after a failed growth)
   d->d_y = d->d_x + cap; d->d_val = reinterpret_cast<int*>(d->d_y + cap);
   d->h_y = d->h_x + cap; d->h_val = reinterpret_cast<int*>(d->h_y + cap);
-  d->feat_cap = cap;
-  return 0;
+  return rc;
 }
 
 // the pinned staging area is reused by every call: wait for copies that may still read/write it
@@ -2696,12 +2705,7 @@ extern "C" int klt_dev_features_commit_records(klt_dev* d, int n, void* first_re
   CU(cudaSetDevice(d->device));
   if (n < 0 || (stride_bytes & 3) || stride_bytes < 12) return fail(d, "commit_records: bad count / stride");
   const size_t bytes = (size_t)n * stride_bytes;
-  if (d->d_rec_cap < bytes) {
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    cudaFree(d->d_rec); d->d_rec = nullptr; d->d_rec_cap = 0;
-    CU(cudaMalloc(&d->d_rec, bytes ? bytes : 16));
-    d->d_rec_cap = bytes ? bytes : 16;
-  }
+  if (grow(d, &d->d_rec_cap, bytes, device_buf(&d->d_rec, bytes))) return 1;
   d->feat_deferred = 1; d->feat_def_dst = d->d_rec; d->feat_def_src = first_record; d->feat_def_bytes = bytes;
   d->feat_out_host = 2;
   d->h_rec = first_record;
@@ -2742,12 +2746,7 @@ extern "C" int klt_dev_snapshot_ring(klt_dev* d, int depth) {
   if (depth < 1 || depth > KLT_SNAP_MAX) return fail(d, "snapshot ring depth %d (1..%d)", depth, KLT_SNAP_MAX);
   if (d->feat_cap <= 0) return fail(d, "snapshot ring: no device-resident features");
   const size_t bytes = (size_t)depth * d->feat_cap * 12;
-  if (d->snap_bytes < bytes) {
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    cudaFreeHost(d->snap_ring); d->snap_ring = nullptr; d->snap_bytes = 0;
-    CU(cudaHostAlloc(&d->snap_ring, bytes, cudaHostAllocDefault));
-    d->snap_bytes = bytes;
-  }
+  if (grow(d, &d->snap_bytes, bytes, pinned_buf(&d->snap_ring, bytes))) return 1;
   for (int i = d->snap_events; i < depth; ++i) {
     CU(cudaEventCreateWithFlags(&d->ev_snap[i], cudaEventDisableTiming));
     d->snap_events = i + 1;
@@ -2790,12 +2789,7 @@ static void make_view(const PyrSet& S, int L, PyrView* v) {
 
 // the buffer of the positions before the tracker (d_x0), as large as the feature arrays
 static int ensure_x0(klt_dev* d) {
-  if (d->x0_cap >= d->feat_cap) return 0;
-  if (sync_all(d)) return fail(d, "stream synchronisation failed");
-  cudaFree(d->d_x0); d->d_x0 = nullptr; d->x0_cap = 0;
-  CU(cudaMalloc(&d->d_x0, (size_t)d->feat_cap * 12));
-  d->x0_cap = d->feat_cap;
-  return 0;
+  return grow(d, &d->x0_cap, d->feat_cap, device_buf(&d->d_x0, (size_t)d->feat_cap * 12));
 }
 
 // where the tracker records its results: the device arrays (resident pipelines) or, for the
@@ -2890,27 +2884,13 @@ extern "C" void klt_dev_disable_track7w(klt_dev* d, int on) { d->no_track7w = on
 // ---- global motion check (klt_motion.cuh) ----------------------------------------------------
 static int ensure_motion(klt_dev* d, int n, int hyps) {
   if (!d->d_mring) {
-    CU(guarded_malloc(d, &d->d_mring, (size_t)KLT_MOTION_RING * sizeof(MotionModelRec)));
+    if (guarded_malloc(d, &d->d_mring, (size_t)KLT_MOTION_RING * sizeof(MotionModelRec))) return 1;
     d->ring_next = 0; d->ring_n = 0;
   }
-  if (d->motion_cap < n) {
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    guarded_free(d, d->d_mcorr); guarded_free(d, d->d_mcidx); guarded_free(d, d->d_merr);
-    d->d_mcorr = nullptr; d->d_mcidx = nullptr; d->d_merr = nullptr; d->motion_cap = 0;
-    const int cap = (n + 1023) / 1024 * 1024;
-    CU(guarded_malloc(d, &d->d_mcorr, (size_t)cap * sizeof(float4)));
-    CU(guarded_malloc(d, &d->d_mcidx, (size_t)cap * sizeof(int)));
-    CU(guarded_malloc(d, &d->d_merr, (size_t)cap * sizeof(float)));
-    d->motion_cap = cap;
-  }
-  if (d->hyp_cap < hyps) {
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    guarded_free(d, d->d_mhyp); d->d_mhyp = nullptr; d->hyp_cap = 0;
-    const int cap = (hyps + 1023) / 1024 * 1024;
-    CU(guarded_malloc(d, &d->d_mhyp, (size_t)(1 + 10 * (size_t)cap) * sizeof(int)));
-    d->hyp_cap = cap;
-  }
-  return 0;
+  const size_t cap = round_1024(n), hcap = round_1024(hyps);
+  return grow(d, &d->motion_cap, cap, device_buf(&d->d_mcorr, cap * sizeof(float4)), device_buf(&d->d_mcidx, cap * sizeof(int)),
+              device_buf(&d->d_merr, cap * sizeof(float))) ||
+         grow(d, &d->hyp_cap, hcap, device_buf(&d->d_mhyp, (1 + 10 * hcap) * sizeof(int)));
 }
 
 // the three launches of the check behind the tracker of a call on n features; the model record goes
@@ -2939,15 +2919,31 @@ static int motion_launch(klt_dev* d, const klt_dev_track_params* p, int n) {
   return 0;
 }
 
-extern "C" int klt_dev_motion_results(klt_dev* d, int n, float* err) {
+// The per-call results of the last tracking call, for `fn`: `last` is the number of features that
+// call ran `feature` on (< 0: it ran without it) and must equal n.  Copies n records from src on the
+// tracker stream, waits for them and hands them to scatter(host records); `arrays` is false when a
+// caller's output array that must be given is NULL.
+template <typename Rec, typename Scatter>
+static int read_results(klt_dev* d, const char* fn, const char* feature, int last, int n, bool arrays, const Rec* src,
+                        Scatter scatter) {
   CU(cudaSetDevice(d->device));
-  if (d->motion_n < 0) return fail(d, "motion_results: the last tracking call did not run the global motion check");
-  if (n != d->motion_n) return fail(d, "motion_results: %d features requested, the last tracking call had %d", n, d->motion_n);
+  if (last < 0) return fail(d, "%s: the last tracking call ran without %s", fn, feature);
+  if (n != last) return fail(d, "%s: %d features requested, the last tracking call had %d", fn, n, last);
   if (n == 0) return 0;
-  if (!err) return fail(d, "motion_results: NULL array");
-  CU(cudaMemcpyAsync(err, d->d_merr, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, d->tstream));
-  CU(cudaStreamSynchronize(d->tstream));
+  if (!arrays) return fail(d, "%s: NULL array", fn);
+  Rec* h = (Rec*)malloc((size_t)n * sizeof(Rec));
+  if (!h) return fail(d, "out of host memory");
+  cudaError_t e = cudaMemcpyAsync(h, src, (size_t)n * sizeof(Rec), cudaMemcpyDeviceToHost, d->tstream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(d->tstream);
+  if (e == cudaSuccess) scatter(h);
+  free(h);
+  if (e != cudaSuccess) return fail(d, "%s: %s", fn, cudaGetErrorString(e));
   return 0;
+}
+
+extern "C" int klt_dev_motion_results(klt_dev* d, int n, float* err) {
+  return read_results(d, "motion_results", "the global motion check", d->motion_n, n, err != nullptr, d->d_merr,
+                      [&](const float* h) { memcpy(err, h, (size_t)n * sizeof(float)); });
 }
 
 extern "C" int klt_dev_motion_models(klt_dev* d, int count, klt_dev_motion_model* out) {
@@ -2966,14 +2962,11 @@ extern "C" int klt_dev_motion_models(klt_dev* d, int count, klt_dev_motion_model
 }
 
 extern "C" int klt_dev_motion_counts(klt_dev* d, int hyps, int* m, int* counts) {
-  CU(cudaSetDevice(d->device));
-  if (d->motion_n < 0) return fail(d, "motion_counts: the last tracking call did not run the global motion check");
-  if (hyps != d->motion_hyps) return fail(d, "motion_counts: %d hypotheses requested, the last call had %d", hyps, d->motion_hyps);
-  if (!m || !counts) return fail(d, "motion_counts: NULL array");
-  CU(cudaMemcpyAsync(m, d->d_mhyp, sizeof(int), cudaMemcpyDeviceToHost, d->tstream));
-  CU(cudaMemcpyAsync(counts, d->d_mhyp + 1, (size_t)hyps * sizeof(int), cudaMemcpyDeviceToHost, d->tstream));
-  CU(cudaStreamSynchronize(d->tstream));
-  return 0;
+  if (d->motion_n >= 0 && hyps != d->motion_hyps)
+    return fail(d, "motion_counts: %d hypotheses requested, the last call had %d", hyps, d->motion_hyps);
+  // hyps + 1 ints: m, then the inlier count of each hypothesis (MotionHyp)
+  return read_results(d, "motion_counts", "the global motion check", d->motion_n < 0 ? -1 : hyps + 1, hyps + 1,
+                      m && counts, d->d_mhyp, [&](const int* h) { *m = h[0]; memcpy(counts, h + 1, (size_t)hyps * sizeof(int)); });
 }
 
 extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
@@ -3009,21 +3002,12 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
     if (ensure_motion(d, n, hyps)) return 1;
   }
   if (n == 0) return motion ? motion_launch(d, p, 0) : 0;
-  if (fb && d->fb_cap < n) {                         // the check's result records (klt_dev_fb_results)
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    guarded_free(d, d->d_fb); d->d_fb = nullptr; d->fb_cap = 0;
-    const int cap = (n + 1023) / 1024 * 1024;
-    CU(guarded_malloc(d, &d->d_fb, (size_t)cap * sizeof(FbRec)));
-    d->fb_cap = cap;
-  }
+  const size_t cap = round_1024(n);
+  if (fb && grow(d, &d->fb_cap, cap, device_buf(&d->d_fb, cap * sizeof(FbRec)))) return 1;   // (klt_dev_fb_results)
   if (pred && d->pred_cap < n) {                     // the prior's records: new ones hold no velocity
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    guarded_free(d, d->d_vel); guarded_free(d, d->d_pred); d->d_vel = nullptr; d->d_pred = nullptr;
-    d->pred_cap = 0; d->vel_n = 0;
-    const int cap = (n + 1023) / 1024 * 1024;
-    CU(guarded_malloc(d, &d->d_vel, (size_t)cap * sizeof(PredVel)));
-    CU(guarded_malloc(d, &d->d_pred, (size_t)cap * sizeof(PredRec)));
-    d->pred_cap = cap;
+    d->vel_n = 0;
+    if (grow(d, &d->pred_cap, cap, device_buf(&d->d_vel, cap * sizeof(PredVel)), device_buf(&d->d_pred, cap * sizeof(PredRec))))
+      return 1;
   }
   float* const guesses = d->d_guess + (size_t)d->guess_slot * 2 * d->guess_cap;
   d->pred.gx = guess_n >= 0 ? guesses : nullptr;
@@ -3084,23 +3068,14 @@ extern "C" int klt_dev_track_resident(klt_dev* d, int slot_prev, int slot_cur,
 }
 
 extern "C" int klt_dev_fb_results(klt_dev* d, int n, float* xb, float* yb, float* err, int* back_val) {
-  CU(cudaSetDevice(d->device));
-  if (d->fb_n < 0) return fail(d, "fb_results: the last tracking call did not run the forward-backward check");
-  if (n != d->fb_n) return fail(d, "fb_results: %d features requested, the last tracking call had %d", n, d->fb_n);
-  if (n == 0) return 0;
-  FbRec* h = (FbRec*)malloc((size_t)n * sizeof(FbRec));
-  if (!h) return fail(d, "out of host memory");
-  cudaError_t e = cudaMemcpyAsync(h, d->d_fb, (size_t)n * sizeof(FbRec), cudaMemcpyDeviceToHost, d->tstream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(d->tstream);
-  if (e != cudaSuccess) { free(h); return fail(d, "fb_results: %s", cudaGetErrorString(e)); }
-  for (int i = 0; i < n; ++i) {
-    if (xb) xb[i] = h[i].xb;
-    if (yb) yb[i] = h[i].yb;
-    if (err) err[i] = h[i].err;
-    if (back_val) back_val[i] = h[i].back_val;
-  }
-  free(h);
-  return 0;
+  return read_results(d, "fb_results", "the forward-backward check", d->fb_n, n, true, d->d_fb, [&](const FbRec* h) {
+    for (int i = 0; i < n; ++i) {
+      if (xb) xb[i] = h[i].xb;
+      if (yb) yb[i] = h[i].yb;
+      if (err) err[i] = h[i].err;
+      if (back_val) back_val[i] = h[i].back_val;
+    }
+  });
 }
 
 // Pipelined drivers queue the guesses of step k + 1 while step k's tracker may not have run yet: the
@@ -3112,15 +3087,9 @@ extern "C" int klt_dev_set_guesses(klt_dev* d, int n, const float* gx, const flo
   if (n < 0 || (n > 0 && (!gx || !gy))) return fail(d, "set_guesses: bad count or NULL array");
   if (!d->ev_guess[0])
     for (int i = 0; i < 2; ++i) CU(cudaEventCreateWithFlags(&d->ev_guess[i], cudaEventDisableTiming));
-  if (d->guess_cap < n) {
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    guarded_free(d, d->d_guess); cudaFreeHost(d->h_guess);
-    d->d_guess = nullptr; d->h_guess = nullptr; d->guess_cap = 0; d->guess_busy[0] = d->guess_busy[1] = 0;
-    const int cap = (n + 1023) / 1024 * 1024;
-    CU(guarded_malloc(d, &d->d_guess, (size_t)cap * 4 * sizeof(float)));
-    CU(cudaMallocHost(&d->h_guess, (size_t)cap * 4 * sizeof(float)));
-    d->guess_cap = cap;
-  }
+  const size_t cap = round_1024(n);                 // gx | gy of both slots
+  if (grow(d, &d->guess_cap, cap, device_buf(&d->d_guess, cap * 4 * sizeof(float)), pinned_buf(&d->h_guess, cap * 4 * sizeof(float))))
+    return 1;
   const int s = d->guess_slot ^ 1;
   if (d->guess_busy[s]) { CU(cudaEventSynchronize(d->ev_guess[s])); d->guess_busy[s] = 0; }
   float* dst = d->d_guess + (size_t)s * 2 * d->guess_cap;
@@ -3148,22 +3117,13 @@ extern "C" int klt_dev_set_guesses(klt_dev* d, int n, const float* gx, const flo
 extern "C" int klt_dev_guesses_pending(const klt_dev* d) { return d->guess_n; }
 
 extern "C" int klt_dev_prediction_results(klt_dev* d, int n, float* gx, float* gy, int* source) {
-  CU(cudaSetDevice(d->device));
-  if (d->pred_n < 0) return fail(d, "prediction_results: the last tracking call ran without prediction");
-  if (n != d->pred_n) return fail(d, "prediction_results: %d features requested, the last tracking call had %d", n, d->pred_n);
-  if (n == 0) return 0;
-  PredRec* h = (PredRec*)malloc((size_t)n * sizeof(PredRec));
-  if (!h) return fail(d, "out of host memory");
-  cudaError_t e = cudaMemcpyAsync(h, d->d_pred, (size_t)n * sizeof(PredRec), cudaMemcpyDeviceToHost, d->tstream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(d->tstream);
-  if (e != cudaSuccess) { free(h); return fail(d, "prediction_results: %s", cudaGetErrorString(e)); }
-  for (int i = 0; i < n; ++i) {
-    if (gx) gx[i] = h[i].gx;
-    if (gy) gy[i] = h[i].gy;
-    if (source) source[i] = h[i].source;
-  }
-  free(h);
-  return 0;
+  return read_results(d, "prediction_results", "prediction", d->pred_n, n, true, d->d_pred, [&](const PredRec* h) {
+    for (int i = 0; i < n; ++i) {
+      if (gx) gx[i] = h[i].gx;
+      if (gy) gy[i] = h[i].gy;
+      if (source) source[i] = h[i].source;
+    }
+  });
 }
 
 extern "C" int klt_dev_track(klt_dev* d, int slot_prev, int slot_cur, const klt_dev_track_params* p,
@@ -3189,16 +3149,12 @@ extern "C" int klt_dev_affine_begin(klt_dev* d, int n, const klt_dev_affine_para
       ap->window_width * ap->window_height > 2048)
     return fail(d, "affine window %d x %d must be odd, >= 3 and at most 2048 pixels", ap->window_width, ap->window_height);
   const int tsz = (ap->window_width + 2) * (ap->window_height + 2);
-  if (d->aff_cap < n || d->aff_tsz != tsz) {
-    if (sync_all(d)) return fail(d, "stream synchronisation failed");
-    cudaFree(d->d_aff_st); cudaFreeHost(d->h_aff_st); cudaFree(d->d_aff_tmpl);
-    d->d_aff_st = nullptr; d->h_aff_st = nullptr; d->d_aff_tmpl = nullptr; d->aff_cap = 0;
-    const int cap = (n + 1023) / 1024 * 1024;
-    CU(cudaMalloc(&d->d_aff_st, (size_t)cap * sizeof(AffState)));
-    CU(cudaMallocHost(&d->h_aff_st, (size_t)cap * sizeof(AffState)));
-    CU(cudaMalloc(&d->d_aff_tmpl, (size_t)cap * 3 * tsz * sizeof(float)));
-    d->aff_cap = cap; d->aff_tsz = tsz;
-  }
+  const size_t cap = round_1024(n);
+  if (d->aff_tsz != tsz) d->aff_cap = 0;             // templates of another window size: all buffers anew
+  if (grow(d, &d->aff_cap, cap, device_buf(&d->d_aff_st, cap * sizeof(AffState)), pinned_buf(&d->h_aff_st, cap * sizeof(AffState)),
+           device_buf(&d->d_aff_tmpl, cap * 3 * tsz * sizeof(float))))
+    return 1;
+  d->aff_tsz = tsz;
   if (ensure_x0(d)) return 1;
   if (d->feat_out_host == 2) return fail(d, "affine_begin: record-mode features (use the staging area)");
   d->feat_out_host = 0;                              // the check needs the tracker's answers on the device
@@ -3340,26 +3296,21 @@ static CandGeo cand_geometry(const klt_dev* d, const klt_dev_select_params* p) {
 }
 
 static int ensure_candidates(klt_dev* d, size_t n) {
-  if (n <= d->cand_cap) return 0;
-  CU(cudaStreamSynchronize(d->stream));
-  for (int i = 0; i < 2; ++i) { guarded_free(d, d->c_val[i]); guarded_free(d, d->c_idx[i]); d->c_val[i] = nullptr; d->c_idx[i] = nullptr; }
-  cudaFree(d->cub_tmp); d->cub_tmp = nullptr; d->cand_cap = 0;
-  for (int i = 0; i < 2; ++i) {
-    CU(guarded_malloc(d, &d->c_val[i], n * sizeof(int)));
-    CU(guarded_malloc(d, &d->c_idx[i], n * sizeof(unsigned)));
-  }
-  guarded_free(d, d->rank_list); guarded_free(d, d->sel_state); d->rank_list = nullptr; d->sel_state = nullptr;
-  CU(guarded_malloc(d, &d->rank_list, n * sizeof(int)));
-  CU(guarded_malloc(d, &d->sel_state, 8 * sizeof(int)));
+  if (n <= d->cand_cap) return 0;                    // (the size queries below only when growing)
+  int* const no_int = nullptr;                       // a size query reads no buffer
+  unsigned* const no_unsigned = nullptr;
   size_t bytes = 0, bytes2 = 0;
-  CU(cub::DeviceRadixSort::SortPairsDescending(nullptr, bytes, d->c_val[0], d->c_val[1], d->c_idx[0],
-                                               d->c_idx[1], (int)n, 0, 32, d->stream));
-  CU(cub::DeviceSelect::If(nullptr, bytes2, thrust::counting_iterator<int>(0), d->rank_list, d->sel_state + 4,
-                           (int)n, UncoveredOp{}, d->stream));
+  CU(cub::DeviceRadixSort::SortPairsDescending(nullptr, bytes, no_int, no_int, no_unsigned, no_unsigned, (int)n, 0, 32,
+                                               d->stream));
+  CU(cub::DeviceSelect::If(nullptr, bytes2, thrust::counting_iterator<int>(0), no_int, no_int, (int)n, UncoveredOp{},
+                           d->stream));
   if (bytes2 > bytes) bytes = bytes2;
-  CU(cudaMalloc(&d->cub_tmp, bytes ? bytes : 16));
+  if (grow(d, &d->cand_cap, n, device_buf(&d->c_val[0], n * sizeof(int)), device_buf(&d->c_val[1], n * sizeof(int)),
+           device_buf(&d->c_idx[0], n * sizeof(unsigned)), device_buf(&d->c_idx[1], n * sizeof(unsigned)),
+           device_buf(&d->rank_list, n * sizeof(int)), device_buf(&d->sel_state, 8 * sizeof(int)),
+           device_buf(&d->cub_tmp, bytes ? bytes : 16)))
+    return 1;
   d->cub_bytes = bytes;
-  d->cand_cap = n;
   return 0;
 }
 
@@ -3430,18 +3381,8 @@ static int select_core(klt_dev* d, int slot, const klt_dev_select_params* p, int
   if (host && klt_dev_features_upload(d, n, x, y, val)) return 1;
   if (!host && (n != d->feat_n || d->feat_out_host != 0)) return fail(d, "select_resident: %d features are not resident on the device", n);
   const size_t npx = (size_t)d->W * d->H;
-  if (d->fmap_cap < npx) {
-    CU(cudaStreamSynchronize(d->stream));
-    guarded_free(d, d->fmap); d->fmap = nullptr; d->fmap_cap = 0;
-    CU(guarded_malloc(d, &d->fmap, npx + 4));        // (+4: the stamps are written as 32-bit words)
-    d->fmap_cap = npx;
-  }
-  if (d->open_cap < n) {
-    CU(cudaStreamSynchronize(d->stream));
-    guarded_free(d, d->open_slots); d->open_slots = nullptr; d->open_cap = 0;
-    CU(guarded_malloc(d, &d->open_slots, (size_t)n * sizeof(int)));
-    d->open_cap = n;
-  }
+  if (grow(d, &d->fmap_cap, npx, device_buf(&d->fmap, npx + 4))) return 1;   // (+4: the stamps are written as 32-bit words)
+  if (grow(d, &d->open_cap, n, device_buf(&d->open_slots, (size_t)n * sizeof(int)))) return 1;
   CU(cudaMemsetAsync(d->fmap, 0, npx, d->stream));
   const bool prestamp = !p->overwrite_all && !d->no_filter && !d->replace_filter;
   if (!p->overwrite_all && prestamp) {
